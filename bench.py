@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed epoch's outputs as DIR/<name>.npy
 
 A step = one eALS epoch (user half-epoch + item half-epoch, each incl. the S-cache Gram and, with
 N > 1, the exchange of the updated factor rows and the all-reduce of the partial Grams) — what the
@@ -159,6 +160,33 @@ def random_factors(M, N, K, device, seed=1234):
     U = torch.randn(M, K, generator=g, device=f"cuda:{device}", dtype=torch.float64) * 0.01
     V = torch.randn(N, K, generator=g, device=f"cuda:{device}", dtype=torch.float64) * 0.01
     return U, V
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(fals, out_dir, seed=2024):
+    """Write what a caller of the timed path holds after its last epoch, as float64 .npy files: the S caches
+    SU and SV whole, and U and V whole when everything fits in DUMP_BYTES.  Otherwise U_rows / V_rows hold a
+    sample of rows: the same sorted, seeded row ids in every run with the same arguments (the inputs are seeded
+    too), so the files of two builds can be compared one for one.  Reads through the library's host copies,
+    which leave the prediction caches valid: the rest of the run computes what it would without the dump."""
+    from eals_cpp_b200 import _lib
+    os.makedirs(out_dir, exist_ok=True)
+    M, N, K = fals.userCount, fals.itemCount, fals.factors
+    out = {"SU": fals.SU, "SV": fals.SV}
+    rows_each = (DUMP_BYTES - 2 * K * K * 8 - 4 * 4096) // (2 * K * 8)     # 4096: room for the .npy headers
+    rng = np.random.default_rng(seed)
+    for name, which, n in (("U", _lib.BUF_U, M), ("V", _lib.BUF_V, N)):
+        if n <= rows_each:
+            out[name] = fals.U if which == _lib.BUF_U else fals.V
+        else:
+            rows = np.sort(rng.choice(n, size=rows_each, replace=False))
+            out[name + "_rows"] = np.stack([fals._factor_row(which, r) for r in rows])
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, np.float64))
+    log(f"[bench] outputs of the last timed step in {out_dir}: " +
+        ", ".join(f"{k} {tuple(v.shape)}" for k, v in out.items()))
 
 
 # --------------------------------------------------------------------------------------------------
@@ -316,6 +344,20 @@ def cpu_reference_full(sm_host, K, steps, warmup):
     return float(np.mean(times))
 
 
+def cpu_port_full(sm_host, K, steps, warmup):
+    """The same whole epochs through the oracle port (PortModel: the reference's arithmetic and S patches), 1 thread."""
+    from oracle.bindings import PortModel
+    port = PortModel(sm_host.M, sm_host.N, sm_host.row_ptr, sm_host.col_idx, factors=K)
+    times = []
+    for it in range(warmup + steps):
+        t0 = time.perf_counter()
+        port.update_user()
+        port.update_item()
+        if it >= warmup:
+            times.append(time.perf_counter() - t0)
+    return float(np.mean(times))
+
+
 # --------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -329,7 +371,11 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the c1/c2/c3 epochs and the C5 evaluation after the main run")
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--cpu-nnz", type=int, default=0, help="nonzeros per side in the CPU sample (0 = auto)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed epoch computed (U, V rows and the S caches) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         log("[bench] note: fewer than 3 warm-up steps requested")
 
@@ -387,6 +433,8 @@ def main():
         e1.record()
         barrier()
     ms_total = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:     # before anything else trains the factors further
+        dump_outputs(fals, args.dump_outputs)
     if world > 1:
         t = torch.tensor([ms_total], device=f"cuda:{local_rank}", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -624,16 +672,19 @@ def reference_arm(args):
     M, N, K = spec["M"], spec["N"], spec["K"]
     small = spec["nnz"] <= 2_000_000
     threaded = None
-    if not bindings.reference_available(fast=True):
-        print(json.dumps({"impl": "reference", "unavailable": "oracle/_ref was not built (no /root/reference at build time)"}), flush=True)
-        return 0
+    # without the reference's sources oracle/_ref is not built: its C restatement stands in, labelled "port"
+    kind = "reference" if bindings.reference_available(fast=True) else "port"
     if small:
         data = datasets.powerlaw_csr(**spec)
         sm = SparseMat.from_csr(data.M, data.N, data.row_ptr, data.col_idx)
         nnz = sm.nnz
-        epoch_s = cpu_reference_full(sm, K, args.steps, min(args.warmup, 1))
+        if kind == "reference":
+            epoch_s = cpu_reference_full(sm, K, args.steps, min(args.warmup, 1))
+            sample = f"oracle/_ref (reference TUs, g++ -O3), whole epochs incl. S patches, 1 thread, mean of {args.steps}"
+        else:
+            epoch_s = cpu_port_full(sm, K, args.steps, min(args.warmup, 1))
+            sample = f"oracle port (eals_oracle.c, gcc -O2), whole epochs incl. S patches, 1 thread, mean of {args.steps}"
         step_s = epoch_s
-        sample = f"oracle/_ref (reference TUs, g++ -O3), whole epochs incl. S patches, 1 thread, mean of {args.steps}"
     else:
         import torch
         assert torch.cuda.is_available(), "the large synthetic workloads are generated on the GPU (torch: plumbing)"
@@ -641,7 +692,11 @@ def reference_arm(args):
         nnz = sm.nnz
         target = args.cpu_nnz or int(6.4e7 / K)
         t0 = time.perf_counter()
-        epoch_s, sample = cpu_reference_sampled(sm, M, N, K, target, args.steps, min(args.warmup, 1))
+        if kind == "reference":
+            epoch_s, sample = cpu_reference_sampled(sm, M, N, K, target, args.steps, min(args.warmup, 1))
+        else:
+            r = cpu_port_sample(sm, K, 0.01, 10.0, 0.75, target, 1)
+            epoch_s, sample = r["epoch_s_extrapolated"], r["sample"]
         step_s = (time.perf_counter() - t0) / (args.steps + min(args.warmup, 1))
         try:
             r = cpu_port_sample(sm, K, 0.01, 10.0, 0.75, min(nnz // 2, 4_000_000), os.cpu_count() or 1)
@@ -658,7 +713,7 @@ def reference_arm(args):
                    "step": "one eALS epoch = update_user + update_item incl. the S-cache patches" +
                            ("" if small else " — measured on a bounded row sample per step, value = throughput on the sample scaled to the whole matrix")},
         "epoch_ms_whole_matrix": epoch_s * 1e3,
-        "cpu_baseline": {"value": value, "unit": UNIT, "cores": 1, "kind": "reference", "sample": sample},
+        "cpu_baseline": {"value": value, "unit": UNIT, "cores": 1, "kind": kind, "sample": sample},
         "cpu_baseline_threaded_port": threaded,
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }

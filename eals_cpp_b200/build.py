@@ -73,7 +73,8 @@ def build_host_example(force: bool = False) -> str:
             os.path.join(ROOT, "include", "eals_host_types.h")]
     cmd = ["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "include"), src, "-o", out,
            "-L", LIB_DIR, "-leals_b200", "-Wl,-rpath,$ORIGIN"]
-    digest = _digest(deps, cmd)
+    # paths relative to the tree: a built tree that is moved or copied stays fresh
+    digest = _digest(deps, [os.path.relpath(c, ROOT) if os.path.isabs(c) else c for c in cmd])
     if not force and _fresh(out, digest):
         return out
     subprocess.run(cmd, check=True)

@@ -1,21 +1,21 @@
 """Pins the CPU oracle (oracle/eals_oracle.c, a C restatement) to the reference.
 
-Two anchors (SURVEY.md §8c — the reference ships no unit tests or vectors of its own besides
+Anchors (SURVEY.md §8c — the reference ships no unit tests or vectors of its own besides
 Outputs.txt, whose input file yelp.rating is not distributed):
-  1. the committed fixtures in tests/golden/, produced by tests/golden/make_golden.py from the
+  1. the committed fixtures in tests/golden/*.npz, produced by tests/golden/make_golden.py from the
      reference's own unmodified translation units;
-  2. live, when oracle/_ref/libeals_ref.so exists (built from /root/reference here; it travels to
-     the GPU box as a built artefact): function by function on seeded inputs.
+  2. the reference's values on seeded inputs from K = 8 to 200 and at the full c1 size, stored in
+     tests/golden/reference_vectors.json (see tests/reference_vectors.py);
+  3. live, when oracle/_ref/libeals_ref.so was built from the reference's sources: its driver order.
 The restatement follows the reference's operation order and is compiled with -ffp-contract=off, so
 agreement is BIT-EXACT except through libm `pow` in the item weights (same libm here: also exact).
 """
 import os
-import re
-import subprocess
 
 import numpy as np
 import pytest
 
+import reference_vectors
 from conftest import random_csr
 from oracle import bindings
 from oracle.bindings import PortModel, Reference, csr_to_csc
@@ -67,54 +67,22 @@ def test_port_reproduces_golden_run(port, name):
         assert hr.sum() != g["eval_hr"].sum()
 
 
-@have_ref
-@pytest.mark.parametrize("K,M,N,dens,weighted", [(8, 120, 90, 6, False), (20, 200, 310, 15, True), (64, 90, 40, 12, False),
-                                                 (129, 70, 50, 9, False), (200, 60, 45, 8, True)])
+@pytest.mark.parametrize("K,M,N,dens,weighted", reference_vectors.SMALL_CASES)
 def test_port_matches_live_reference(port, K, M, N, dens, weighted):
-    row_ptr, col_idx = random_csr(M, N, dens, seed=K * 7 + M, empty_frac=0.08)
-    val = np.random.default_rng(K).uniform(0.5, 2.5, len(col_idx)) if weighted else None
-    gt = np.random.default_rng(K + 1).integers(0, N, M).astype(np.int32)
-    ref = Reference(M, N, row_ptr, col_idx, val, test_items=gt, factors=K, topK=5)
-    m = PortModel(M, N, row_ptr, col_idx, val, factors=K, port=port)
-    assert np.array_equal(m.U, ref.U) and np.array_equal(m.V, ref.V)
-    assert np.array_equal(m.Wi, ref.Wi)
-    assert np.array_equal(m.SU, ref.SU) and np.array_equal(m.SV, ref.SV)
-    assert m.loss() == ref.loss()
-    for _ in range(2):
-        ref.update_user(); m.update_user()
-        assert np.array_equal(m.U, ref.U) and np.array_equal(m.SU, ref.SU)
-        ref.update_item(); m.update_item()
-        assert np.array_equal(m.V, ref.V) and np.array_equal(m.SV, ref.SV)
-        assert m.loss() == ref.loss()
-    for scale in (1.0, 25.0):
-        if scale != 1.0:
-            rng = np.random.default_rng(3)
-            U = m.U * scale + rng.normal(0, 0.6, m.U.shape)
-            V = m.V * scale + rng.normal(0, 0.6, m.V.shape)
-            m.U[:], m.V[:] = U, V
-            ref.set_UV(U, V)
-        rmean, rhr, rndcg, rprec = ref.evaluate(gt, 5)
-        pmean, phr, pndcg, pprec, _ = m.evaluate(gt, 5, compat=True)
-        assert np.array_equal(phr, rhr) and np.array_equal(pndcg, rndcg) and np.array_equal(pprec, rprec)
-        assert np.array_equal(pmean, rmean)
+    """Against the values the reference's own object computed on these seeded inputs (stored, see
+    tests/reference_vectors.py): factors, S caches, item weights and loss after initialisation and every
+    half-epoch of two epochs, and the top-5 evaluation on trained and on inflated factors — bit for bit."""
+    want = reference_vectors.load()["small"][reference_vectors.case_id(K, M, N, dens, weighted)]
+    reference_vectors.assert_same(reference_vectors.small_case(port, K, M, N, dens, weighted), want)
 
 
-@have_ref
 def test_port_matches_live_reference_at_the_headline_size(port):
     """BASELINE.json configs[0] in full (yelp-shaped: 25677 x 25815, 669k interactions, K = 64, the synthetic
     stand-in bench.py calls c1): one whole epoch of the restatement against the reference's own object — factors,
-    S caches and loss bit for bit.  This is the size the CPU baseline of bench.py is quoted on."""
-    from eals_cpp_b200 import datasets
-    d = datasets.powerlaw_csr(**datasets.WORKLOADS["c1"])
-    K = datasets.WORKLOADS["c1"]["K"]
-    ref = Reference(d.M, d.N, d.row_ptr, d.col_idx, test_items=d.test_items, factors=K, topK=10)
-    m = PortModel(d.M, d.N, d.row_ptr, d.col_idx, factors=K, port=port)
-    assert np.array_equal(m.U, ref.U) and np.array_equal(m.V, ref.V) and np.array_equal(m.Wi, ref.Wi)
-    ref.update_user(); m.update_user()
-    assert np.array_equal(m.U, ref.U) and np.array_equal(m.SU, ref.SU)
-    ref.update_item(); m.update_item()
-    assert np.array_equal(m.V, ref.V) and np.array_equal(m.SV, ref.SV)
-    assert m.loss() == ref.loss()
+    S caches and loss bit for bit (stored, see tests/reference_vectors.py).  This is the size the CPU baseline of
+    bench.py is quoted on."""
+    want = reference_vectors.load()["headline_c1"]
+    reference_vectors.assert_same(reference_vectors.headline_case(port), want)
 
 
 @have_ref
@@ -191,22 +159,18 @@ def _ratings_with_ties(path, M=90, N=60, seed=8):
 
 
 def _reference_transcript(tmp_path):
-    """Run the reference's own driver (oracle/_ref/eals_ref_main = main.cpp unmodified) on tmp_path/yelp.rating."""
-    exe = os.path.join(os.path.dirname(bindings.REF_SO), "eals_ref_main")
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/eals_ref_main not built (no /root/reference at build time)")
-    res = subprocess.run([exe], cwd=str(tmp_path), capture_output=True, text=True, timeout=600)
-    out = res.stdout                                     # exits through its double free AFTER printing (SURVEY.md §3.1)
-    losses = [float(x) for x in re.findall(r"Iter=\d+ \S+ [-+] loss:(\S+)", out)]
-    m = re.search(r"<hr, ndcg, prec>: \t(\S+)\t(\S+)\t(\S+)", out)
-    assert len(losses) == 20 and m, out[-2000:]
-    counts = {k: int(re.search(k + r"\t(\d+)", out).group(1)) for k in ("#Users", "#items", "#Ratings")}
-    return losses, [float(x) for x in m.groups()], counts, out
+    """What the reference's own driver (main.cpp, the run.sh defaults) prints on tmp_path/yelp.rating, stored (see
+    tests/reference_vectors.py): its 20 losses, the final <hr, ndcg, prec>, the counts and its lines with the
+    numbers masked."""
+    want = reference_vectors.load()["transcript_ties"]
+    assert reference_vectors.file_digest(tmp_path / "yelp.rating") == want["ratings_sha256"], "not the stored input"
+    assert len(want["losses"]) == 20
+    return want["losses"], want["metrics"], want["counts"], want["lines"]
 
 
 def test_loader_split_matches_the_reference_binary_with_tied_timestamps(tmp_path):
-    """Our loader (host/eals_main.cpp --dump-split, no GPU) against the reference's own main.cpp on the same
-    file, ties and duplicates included: same counts, and the oracle trained on OUR split reproduces the
+    """Our loader (host/eals_main.cpp --dump-split, no GPU) against what the reference's own main.cpp printed on
+    the same file, ties and duplicates included: same counts, and the oracle trained on OUR split reproduces the
     reference binary's 20 printed losses and its final metrics (which depend on every tie decision)."""
     import subprocess as sp
     from eals_cpp_b200 import build
