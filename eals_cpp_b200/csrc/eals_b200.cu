@@ -26,6 +26,8 @@
 #include <cuda_fp16.h>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_run_length_encode.cuh>
+#include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
 
@@ -36,6 +38,7 @@
 #include "eval_tc.cuh"
 #include "gram.cuh"
 #include "loss.cuh"
+#include "recommend.cuh"
 
 namespace {
 
@@ -204,6 +207,11 @@ struct eals_model {
   long long eval_blk0_users = 0, eval_blk0_items = 0;   // first item block of the tensor-core filter: shape and device time
   double eval_blk0_ms = 0;
   cudaEvent_t ev_blk0_a = nullptr, ev_blk0_b = nullptr;
+  // the last recommend: engine (0 exact fp64, 1 tcgen05 filter), seed items, pairs re-scored, users left after the
+  // first item block, and the first block's users, items and device time
+  int rec_engine = 0;
+  long long rec_seed = 0, rec_pairs = 0, rec_left1 = 0, rec_blk0_users = 0, rec_blk0_items = 0;
+  double rec_blk0_ms = 0;
   double init_stream_s = 0;              // host seconds of the last factor-stream generation
   bool su_fresh = true;          // SU describes the current U (false after single-row user updates without a Gram)
   double* S_tmp = nullptr;       // [LD][LD] scratch Gram for loss() while SU is stale
@@ -1600,7 +1608,12 @@ struct eals_eval_ws {
   WsBuf<unsigned long long> tkey, tkey_out;
   WsBuf<int32_t> tval, tval_out;
   WsBuf<int32_t> active;
+  WsBuf<double> top_s, thr, pscore;               // recommend: per-slot lists and k-th scores, re-scored pairs
+  WsBuf<int32_t> top_i, pval, pval_out, run_cnt, run_off;
+  WsBuf<uint32_t> pkey, pkey_out, run_slot;
   void release() {
+    top_s.release(); thr.release(); pscore.release(); top_i.release(); pval.release(); pval_out.release();
+    run_cnt.release(); run_off.release(); pkey.release(); pkey_out.release(); run_slot.release();
     users.release(); gt.release(); cnt.release(); cnt_exact.release(); list_a.release(); list_b.release(); perm.release();
     ids.release(); exps.release(); scalars.release(); gts.release(); Uh.release(); Vh.release(); W.release();
     un_hat.release(); un_del.release(); un_h.release(); vn_hat.release(); vn_del.release(); vn_h.release();
@@ -1753,7 +1766,7 @@ template <int NKC, int MODE>
 int launch_filter(eals_model* m, const CUtensorMap& mapU, const CUtensorMap& mapV, const eals::tc::TcArgs& a, int max_works) {
   using C = eals::tc::Cfg<NKC>;
   auto kern = eals::tc::eval_filter_kernel<NKC, MODE>;
-  const size_t smem = MODE == 1 ? C::kSmemEmit : C::kSmem;
+  const size_t smem = MODE != 0 ? C::kSmemEmit : C::kSmem;
   CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   (void)max_works;     // the kernel cuts the item range into chunks when there are fewer user tiles than SMs
   kern<<<m->sm_count, eals::tc::kThreads, smem, m->stream>>>(mapU, mapV, a);
@@ -1796,15 +1809,16 @@ __global__ void set_i32_kernel(int32_t* p, int32_t v) { *p = v; }
 
 struct TcStats { long long candidates = 0, pairs = 0, blocks = 0; };
 
-int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, int topk, bool want_triples, ScanResult& out, bool* overflow) {
+// Preparation of the tcgen05 filter for the users d_users[0 .. n) (evaluate and recommend): fp16 copies of V in
+// decreasing-norm order (ws.perm: rank -> item) and of the users' rows, their norms, the per-tile item norms and
+// the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).  Returns the cub scratch
+// sizes of the item sort and of the working-set compaction.
+int tc_prepare(eals_model* m, int n, const int32_t* d_users, const double* d_thr, size_t& tmp_sort, size_t& tmp_sel) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
-  *overflow = false;
-  StageTimer tm;
   const int K = m->K, LD = m->LD, N = m->N;
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
-  const int ut = nkc <= 2 ? 2 : 1;
   cudaStream_t st = m->stream;
   // ---- preparation: fp16 copies, norms, item order, per-slot thresholds ----
   OK(ws.counters.reserve(4));
@@ -1817,7 +1831,7 @@ int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, i
   OK(ws.cnt.reserve((size_t)n)); OK(ws.cnt_exact.reserve((size_t)n));
   OK(ws.list_a.reserve((size_t)n)); OK(ws.list_b.reserve((size_t)n)); OK(ws.flags.reserve((size_t)n));
   OK(ws.scalars.reserve(8));
-  size_t tmp_sort = 0, tmp_sel = 0;
+  tmp_sort = 0; tmp_sel = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, tmp_sort, ws.keys.p, ws.keys_out.p, ws.ids.p, ws.perm.p, N, 0, 32, st);
   {
     size_t t2 = 0;
@@ -1847,9 +1861,24 @@ int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, i
     tc::prep_rows_kernel<true><<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(m->U, K, LD, KP, n, d_users, 0, d_vmax, o);
     OK(check_launch(m));
     const double gamma = (double)KP * (1.0 / 2097152.0);   // KP * 2^-21
-    tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_gts, ws.exps.p, d_vmax, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n, gamma, ws.sp0.p, ws.sp1.p);
+    tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_thr, ws.exps.p, d_vmax, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n, gamma, ws.sp0.p, ws.sp1.p);
     OK(check_launch(m));
   }
+  return EALS_OK;
+}
+
+int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, int topk, bool want_triples, ScanResult& out, bool* overflow) {
+  namespace tc = eals::tc;
+  eals_eval_ws& ws = eval_ws(m);
+  *overflow = false;
+  StageTimer tm;
+  const int K = m->K, LD = m->LD, N = m->N;
+  const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
+  const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
+  const int ut = nkc <= 2 ? 2 : 1;
+  cudaStream_t st = m->stream;
+  size_t tmp_sort = 0, tmp_sel = 0;
+  OK(tc_prepare(m, n, d_users, d_gts, tmp_sort, tmp_sel));
   CU(cudaMemsetAsync(ws.cnt.p, 0, sizeof(int32_t) * n, st));
   CU(cudaMemsetAsync(ws.cnt_exact.p, 0, sizeof(int32_t) * n, st));
   CUtensorMap mapV, mapU0, mapW;
@@ -2062,6 +2091,299 @@ int evaluate_slots(eals_model* m, const std::vector<int32_t>& users_h, const int
     sums[0] += r0; sums[1] += r1; sums[2] += r2;
   }
   tm_host.lap("eval: host ranking replay + metrics");
+  return EALS_OK;
+}
+
+// ---- top-k retrieval (recommend.cuh) --------------------------------------------------------------------
+namespace rec = eals::rec;
+
+rec::MergeArgs rec_args(eals_model* m, const int32_t* d_users, int k, bool exclude) {
+  eals_eval_ws& ws = eval_ws(m);
+  rec::MergeArgs a{};
+  a.U = m->U; a.V = m->V; a.K = m->K; a.LD = m->LD; a.users = d_users; a.k = k;
+  a.top_s = ws.top_s.p; a.top_i = ws.top_i.p; a.thr = ws.thr.p;
+  if (exclude) { a.ptr = m->users.ptr; a.idx = m->users.idx; a.row_base = m->users.row_base; }
+  return a;
+}
+
+int rec_reset(eals_model* m, int n, int k) {
+  eals_eval_ws& ws = eval_ws(m);
+  rec::rec_init_kernel<<<4 * m->sm_count, 256, 0, m->stream>>>(ws.top_s.p, ws.top_i.p, (size_t)n * k, ws.thr.p, n);
+  return check_launch(m);
+}
+
+// the listed slots (list nullable: slots 0 .. n_list-1) against the items order[r0 .. r1), every score exact
+int rec_merge_exact(eals_model* m, rec::MergeArgs a, const int32_t* list, int n_list, const int32_t* order, int r0, int r1) {
+  if (n_list <= 0 || r1 <= r0) return EALS_OK;
+  a.list = list; a.order = order; a.r0 = r0; a.r1 = r1;
+  rec::rec_merge_kernel<rec::SRC_EXACT><<<n_list, rec::kThreads, 0, m->stream>>>(a);
+  return check_launch(m);
+}
+
+// Engine 1: exact fp64 scores of every item.  Short lists, the reference of the tensor-core engine
+// (EALS_EVAL_SCALAR=1) and its fall-back.
+int rec_exact(eals_model* m, int n, const int32_t* d_users, int k, bool exclude) {
+  OK(rec_reset(m, n, k));
+  OK(rec_merge_exact(m, rec_args(m, d_users, k, exclude), nullptr, n, nullptr, 0, m->N));
+  m->rec_engine = 0; m->rec_seed = 0; m->rec_pairs = 0; m->rec_left1 = 0;
+  m->rec_blk0_users = m->rec_blk0_items = 0; m->rec_blk0_ms = 0;
+  return EALS_OK;
+}
+
+// Engine 2: tcgen05 filter.  Seed: the highest-norm items scored exactly (extended tile by tile for users whose
+// list is not full).  Then item blocks in norm order: the filter emits (user, item) only where acc >= t^ - E
+// (t = the user's current k-th score), the pairs are re-scored exactly and merged, t rises, and a user leaves
+// the working set once a Cauchy-Schwarz bound on every remaining item is below t (DESIGN.md §3.5).
+int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, bool* overflow) {
+  namespace tc = eals::tc;
+  eals_eval_ws& ws = eval_ws(m);
+  *overflow = false;
+  StageTimer tm;
+  const int K = m->K, N = m->N;
+  const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
+  const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
+  const int ut = nkc <= 2 ? 2 : 1;
+  cudaStream_t st = m->stream;
+  OK(rec_reset(m, n, k));
+  size_t tmp_sort = 0, tmp_sel = 0;
+  OK(tc_prepare(m, n, d_users, ws.thr.p, tmp_sort, tmp_sel));
+  const double gamma = (double)KP * (1.0 / 2097152.0);
+  auto params = [&]() -> int {   // per-slot filter thresholds from the current k-th scores
+    tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(ws.thr.p, ws.exps.p, ws.counters.p, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n,
+                                                            gamma, ws.sp0.p, ws.sp1.p);
+    return check_launch(m);
+  };
+  // rem[t] >= max |v^| over the items of tiles t.. (|v^| <= |vh| + |dv|), rounded up; rem[n_tiles] = 0
+  std::vector<float2> tn((size_t)n_tiles);
+  CU(cudaMemcpyAsync(tn.data(), ws.tile_norm.p, sizeof(float2) * n_tiles, cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  std::vector<float> rem((size_t)n_tiles + 1, 0.f);
+  for (int t = n_tiles - 1; t >= 0; t--)
+    rem[(size_t)t] = std::max(rem[(size_t)t + 1], std::nextafter(tn[(size_t)t].x + tn[(size_t)t].y, std::numeric_limits<float>::infinity()));
+  int32_t* d_n = ws.scalars.p;          // [0]: working-list size, [1]: scratch, [2]: size of a chunk of the list
+  auto select = [&](const int32_t* in, int n_in, int32_t* out, int* n_out) -> int {   // flagged positions of `in`
+    cudaError_t e;
+    if (in) e = cub::DeviceSelect::Flagged(ws.cub_tmp.p, tmp_sel, in, ws.flags.p, out, d_n, n_in, st);
+    else e = cub::DeviceSelect::Flagged(ws.cub_tmp.p, tmp_sel, thrust::counting_iterator<int32_t>(0), ws.flags.p, out, d_n, n_in, st);
+    if (e != cudaSuccess) return fail(EALS_ERR_CUDA, "working-set compaction");
+    m->launches++;
+    CU(cudaMemcpyAsync(n_out, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    return EALS_OK;
+  };
+  const rec::MergeArgs base = rec_args(m, d_users, k, exclude);
+
+  // ---- seed ----
+  const int seed = (int)std::min<int64_t>(N, ((int64_t)k + tc::kTN - 1) / tc::kTN * tc::kTN);
+  OK(rec_merge_exact(m, base, nullptr, n, ws.perm.p, 0, seed));
+  {
+    const int32_t* lst = nullptr;
+    int nl = n, r_end = seed, step = tc::kTN;
+    int32_t* bufs[2] = {ws.list_a.p, ws.list_b.p};
+    for (int b = 0; nl > 0 && r_end < N; b ^= 1) {
+      rec::rec_unfilled_flags_kernel<<<(nl + 255) / 256, 256, 0, st>>>(lst, nullptr, nl, ws.thr.p, ws.flags.p);
+      OK(check_launch(m));
+      OK(select(lst, nl, bufs[b], &nl));
+      lst = bufs[b];
+      const int r1 = (int)std::min<int64_t>(N, (int64_t)r_end + step);
+      OK(rec_merge_exact(m, base, lst, nl, ws.perm.p, r_end, r1));
+      r_end = r1;
+      step *= 2;
+    }
+  }
+  tm.lap("recommend: prep + exact seed");
+
+  // ---- item blocks ----
+  const int32_t* list = nullptr;
+  int n_act = n;
+  int32_t *list_next = ws.list_a.p, *list_other = ws.list_b.p;
+  auto compact = [&](int it_next) -> int {   // users that may still gain an item from tile it_next on
+    OK(params());
+    rec::rec_keep_flags_kernel<<<(n_act + 255) / 256, 256, 0, st>>>(list, nullptr, n_act, ws.un_hat.p, ws.sp0.p, ws.thr.p,
+                                                                    rem[(size_t)it_next], ws.flags.p);
+    OK(check_launch(m));
+    OK(select(list, n_act, list_next, &n_act));
+    tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, st>>>(ws.Uh.p, KP, list_next, d_n, ws.W.p);
+    OK(check_launch(m));
+    list = list_next;
+    std::swap(list_next, list_other);
+    return EALS_OK;
+  };
+  OK(compact(seed / tc::kTN));
+  CUtensorMap mapV;
+  OK(make_half_map(&mapV, ws.Vh.p, (size_t)N, KP));
+  tc::TcArgs a{};
+  a.sp0 = ws.sp0.p; a.sp1 = ws.sp1.p; a.tile_norm = ws.tile_norm.p; a.n_items = N; a.perm = ws.perm.p; a.n_act = d_n + 2;
+  unsigned long long* d_np = ws.counters.p + 1;
+  unsigned long long cap = 1ull << 24, hard_cap = 1ull << 28;
+  if (const char* e = getenv("EALS_EVAL_PAIR_CAP")) cap = std::max<unsigned long long>(16, strtoull(e, nullptr, 10));
+  if (const char* e = getenv("EALS_EVAL_PAIR_HARD_CAP")) hard_cap = strtoull(e, nullptr, 10);
+  // the sort and run-length encoding of the pairs count in int
+  hard_cap = std::min<unsigned long long>(hard_cap, 0x7fffffffull);
+  cap = std::min(cap, hard_cap);
+  int64_t blk = 32768;
+  if (const char* e = getenv("EALS_EVAL_FIRST_CHUNK")) blk = std::max<int64_t>(tc::kTN, atoll(e));
+  const int quantum = ut * tc::kTM;
+  int chunk = std::max(quantum, (n_act + quantum - 1) / quantum * quantum);
+  m->rec_pairs = 0; m->rec_left1 = n_act; m->rec_blk0_users = 0; m->rec_blk0_items = 0; m->rec_blk0_ms = 0;
+  bool first = true;
+  for (int64_t i0 = seed; i0 < N && n_act > 0;) {
+    const int64_t i1 = std::min<int64_t>(N, i0 + blk);
+    a.it0 = (int)(i0 / tc::kTN); a.it1 = (int)((i1 + tc::kTN - 1) / tc::kTN);
+    for (int p0 = 0; p0 < n_act;) {
+      const int nc = std::min(chunk, n_act - p0);
+      set_i32_kernel<<<1, 1, 0, st>>>(d_n + 2, nc);
+      OK(check_launch(m));
+      CUtensorMap mapW;
+      OK(make_half_map(&mapW, ws.W.p + (size_t)p0 * KP, (size_t)(n + 2 * tc::kTM - p0), KP));
+      OK(ws.pairs.reserve((size_t)cap));
+      a.act = list + p0; a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
+      CU(cudaMemsetAsync(d_np, 0, sizeof(unsigned long long), st));
+      const bool timed = first && p0 == 0 && nc == n_act;
+      if (timed) {
+        if (!m->ev_blk0_a) { CU(cudaEventCreate(&m->ev_blk0_a)); CU(cudaEventCreate(&m->ev_blk0_b)); }
+        CU(cudaEventRecord(m->ev_blk0_a, st));
+      }
+      OK(launch_filter_k<2>(m, nkc, mapW, mapV, a, (nc + quantum - 1) / quantum));
+      if (timed) CU(cudaEventRecord(m->ev_blk0_b, st));
+      unsigned long long got = 0;
+      CU(cudaMemcpyAsync(&got, d_np, sizeof(got), cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
+      if (got > cap) {
+        if (got <= hard_cap) { cap = got; continue; }            // a larger buffer, same chunk
+        if (nc > quantum) {                                       // fewer users per pass
+          chunk = std::max<long long>(quantum, (long long)((double)nc * ((double)hard_cap / (double)got) / 2) / quantum * quantum);
+          continue;
+        }
+        *overflow = true;                                         // the filter is not filtering: exact engine instead
+        return EALS_OK;
+      }
+      if (timed) {
+        float ms = 0;
+        CU(cudaEventElapsedTime(&ms, m->ev_blk0_a, m->ev_blk0_b));
+        m->rec_blk0_ms = ms; m->rec_blk0_users = nc; m->rec_blk0_items = std::min<int64_t>(N, (int64_t)a.it1 * tc::kTN) - i0;
+      }
+      if (got) {
+        OK(ws.pscore.reserve((size_t)got)); OK(ws.pkey.reserve((size_t)got)); OK(ws.pkey_out.reserve((size_t)got));
+        OK(ws.pval.reserve((size_t)got)); OK(ws.pval_out.reserve((size_t)got));
+        OK(ws.run_slot.reserve((size_t)got)); OK(ws.run_cnt.reserve((size_t)got)); OK(ws.run_off.reserve((size_t)got));
+        rec::rec_rescore_kernel<tc::EvalPair><<<16 * m->sm_count, 128, 0, st>>>(m->U, m->V, K, m->LD, d_users, ws.pairs.p, got,
+                                                                               ws.pscore.p, ws.pkey.p, ws.pval.p);
+        OK(check_launch(m));
+        int slot_bits = 1;
+        while ((1ll << slot_bits) < n) slot_bits++;
+        const int ng = (int)got;
+        size_t t1 = 0, t2 = 0, t3 = 0;
+        cub::DeviceRadixSort::SortPairs(nullptr, t1, ws.pkey.p, ws.pkey_out.p, ws.pval.p, ws.pval_out.p, ng, 0, slot_bits, st);
+        cub::DeviceRunLengthEncode::Encode(nullptr, t2, ws.pkey_out.p, ws.run_slot.p, ws.run_cnt.p, d_n + 1, ng, st);
+        cub::DeviceScan::ExclusiveSum(nullptr, t3, ws.run_cnt.p, ws.run_off.p, ng, st);
+        const size_t need = std::max({t1, t2, t3, tmp_sel});
+        if (need > ws.cub_tmp.cap) { OK(ws.cub_tmp.reserve(need + 16)); }
+        size_t tb = ws.cub_tmp.cap;
+        if (cub::DeviceRadixSort::SortPairs(ws.cub_tmp.p, tb, ws.pkey.p, ws.pkey_out.p, ws.pval.p, ws.pval_out.p, ng, 0, slot_bits, st) != cudaSuccess)
+          return fail(EALS_ERR_CUDA, "candidate sort");
+        tb = ws.cub_tmp.cap;
+        if (cub::DeviceRunLengthEncode::Encode(ws.cub_tmp.p, tb, ws.pkey_out.p, ws.run_slot.p, ws.run_cnt.p, d_n + 1, ng, st) != cudaSuccess)
+          return fail(EALS_ERR_CUDA, "candidate runs");
+        int n_runs = 0;
+        CU(cudaMemcpyAsync(&n_runs, d_n + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        tb = ws.cub_tmp.cap;
+        if (cub::DeviceScan::ExclusiveSum(ws.cub_tmp.p, tb, ws.run_cnt.p, ws.run_off.p, n_runs, st) != cudaSuccess)
+          return fail(EALS_ERR_CUDA, "candidate offsets");
+        m->launches += 3;
+        rec::MergeArgs ma = base;
+        ma.run_slot = reinterpret_cast<const int32_t*>(ws.run_slot.p); ma.run_off = ws.run_off.p; ma.run_cnt = ws.run_cnt.p;
+        ma.pos_pair = ws.pval_out.p; ma.pair_item = &ws.pairs.p[0].item; ma.pair_stride = 4; ma.pair_score = ws.pscore.p;
+        rec::rec_merge_kernel<rec::SRC_PAIRS><<<n_runs, rec::kThreads, 0, st>>>(ma);
+        OK(check_launch(m));
+      }
+      m->rec_pairs += (long long)got;
+      p0 += nc;
+    }
+    OK(compact(a.it1));
+    if (first) m->rec_left1 = n_act;
+    first = false;
+    if (tm.on) {
+      char what[96];
+      snprintf(what, sizeof(what), "recommend: items [%lld, %lld) -> %d users left", (long long)i0, (long long)a.it1 * tc::kTN, n_act);
+      tm.lap(what);
+    }
+    i0 = (int64_t)a.it1 * tc::kTN;
+    blk = std::min<int64_t>(blk * 4, 262144);
+  }
+  m->rec_engine = 1; m->rec_seed = seed;
+  return EALS_OK;
+}
+
+int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k, int exclude, int32_t* items, double* scores) {
+  if (!m || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (k < 1 || k > rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", rec::kMaxK, k);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  if (!m->factors_set) return fail(EALS_ERR_STATE, "factors not initialised");
+  if (m->K > rec::kMaxFactors) return fail(EALS_ERR_UNSUPPORTED, "recommend supports up to %d factors", rec::kMaxFactors);
+  CU(cudaSetDevice(m->p.device));
+  if (n == 0) return EALS_OK;
+  if (space == EALS_HOST)
+    for (int s = 0; s < n; s++) {
+      if (users[s] < 0 || users[s] >= m->M) return fail(EALS_ERR_ARG, "user %d (position %d) outside [0, %d)", users[s], s, m->M);
+      if (users[s] < m->ub || users[s] >= m->ue)
+        return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", users[s], s, m->ub, m->ue);
+    }
+  eals_eval_ws& ws = eval_ws(m);
+  // Per-slot lists for at most `per` users at a time (12 bytes per entry; EALS_REC_LIST_BYTES, default 4 GiB): the
+  // users are answered in balanced chunks, each a complete call of an engine.
+  size_t list_bytes = (size_t)4 << 30;
+  if (const char* e = getenv("EALS_REC_LIST_BYTES")) list_bytes = std::max<size_t>(12 * (size_t)k, strtoull(e, nullptr, 10));
+  const int max_per = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, list_bytes / (12 * (size_t)k)));
+  const int n_chunks = (n + max_per - 1) / max_per, per = (n + n_chunks - 1) / n_chunks;
+  const size_t pk = (size_t)per * k;
+  OK(ws.users.reserve((size_t)n)); OK(ws.top_s.reserve(pk)); OK(ws.top_i.reserve(pk)); OK(ws.thr.reserve((size_t)per));
+  OK(copy_in(ws.users.p, users, (size_t)n, space, m->stream));
+  if (space == EALS_DEVICE) {
+    const int none = 0x7fffffff;
+    int bad = none;
+    CU(cudaMemcpyAsync(m->flags, &none, sizeof(int), cudaMemcpyHostToDevice, m->stream));
+    rec::rec_check_users_kernel<<<(n + 255) / 256, 256, 0, m->stream>>>(ws.users.p, n, m->ub, m->ue, m->flags);
+    OK(check_launch(m));
+    CU(cudaMemcpyAsync(&bad, m->flags, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+    CU(cudaStreamSynchronize(m->stream));
+    if (bad != none) {
+      int u = 0;
+      CU(cudaMemcpy(&u, ws.users.p + (bad - 1), sizeof(int), cudaMemcpyDeviceToHost));
+      if (u < 0 || u >= m->M) return fail(EALS_ERR_ARG, "user %d (position %d) outside [0, %d)", u, bad - 1, m->M);
+      return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", u, bad - 1, m->ub, m->ue);
+    }
+  }
+  const bool scalar_only = getenv("EALS_EVAL_SCALAR") && getenv("EALS_EVAL_SCALAR")[0] == '1';
+  const cudaMemcpyKind kind = space == EALS_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+  bool all_tc = true;
+  long long pairs = 0, left1 = 0, blk0_users = 0, blk0_items = 0;
+  double blk0_ms = 0;
+  for (int s0 = 0; s0 < n; s0 += per) {
+    const int nc = std::min(per, n - s0);
+    const size_t nck = (size_t)nc * k;
+    bool done = false;
+    if (nc >= kTcMinUsers && m->K <= 256 && !scalar_only) {
+      bool overflow = false;
+      OK(rec_tc(m, nc, ws.users.p + s0, k, exclude != 0, &overflow));
+      done = !overflow;
+    }
+    if (!done) OK(rec_exact(m, nc, ws.users.p + s0, k, exclude != 0));
+    all_tc &= done;
+    pairs += m->rec_pairs; left1 += m->rec_left1;
+    if (s0 == 0) { blk0_users = m->rec_blk0_users; blk0_items = m->rec_blk0_items; blk0_ms = m->rec_blk0_ms; }
+    rec::rec_finish_kernel<<<4 * m->sm_count, 256, 0, m->stream>>>(ws.top_i.p, nck);
+    OK(check_launch(m));
+    CU(cudaMemcpyAsync(items + (size_t)s0 * k, ws.top_i.p, sizeof(int32_t) * nck, kind, m->stream));
+    if (scores) CU(cudaMemcpyAsync(scores + (size_t)s0 * k, ws.top_s.p, sizeof(double) * nck, kind, m->stream));
+    CU(cudaStreamSynchronize(m->stream));   // the lists are reused by the next chunk
+  }
+  m->rec_engine = all_tc ? 1 : 0; m->rec_pairs = pairs; m->rec_left1 = left1;
+  m->rec_blk0_users = blk0_users; m->rec_blk0_items = blk0_items; m->rec_blk0_ms = blk0_ms;
+  if (!all_tc) m->rec_seed = 0;
+  CU(cudaStreamSynchronize(m->stream));
   return EALS_OK;
 }
 
@@ -2577,6 +2899,18 @@ int eals_eval_stats(eals_model* m, int64_t out[6]) {
   out[3] = m->eval_engine == 1 ? m->eval_blk0_users : 0;
   out[4] = m->eval_engine == 1 ? m->eval_blk0_items : 0;
   out[5] = m->eval_engine == 1 ? (int64_t)(m->eval_blk0_ms * 1000.0) : 0;
+  return EALS_OK;
+}
+
+int eals_recommend(eals_model* m, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
+                   int32_t* items, double* scores) {
+  return recommend_impl(m, space, n, users, k, exclude_seen, items, scores);
+}
+
+int eals_recommend_stats(eals_model* m, int64_t out[7]) {
+  if (!m || !out) return fail(EALS_ERR_ARG, "null argument");
+  out[0] = m->rec_engine; out[1] = m->rec_seed; out[2] = m->rec_pairs; out[3] = m->rec_left1;
+  out[4] = m->rec_blk0_users; out[5] = m->rec_blk0_items; out[6] = (int64_t)(m->rec_blk0_ms * 1000.0);
   return EALS_OK;
 }
 

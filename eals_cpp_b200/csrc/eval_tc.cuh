@@ -33,7 +33,8 @@
 //   warp 1      tcgen05.mma issuer (one lane): per stage UT x (KP/16) MMAs of 128 x 128 x 16 into one of
 //               two TMEM accumulator buffers; tcgen05.commit releases the stage and publishes the buffer
 //   warps 2-9   epilogue: tcgen05.ld of the warp's 32 TMEM lanes (= 32 users) x 64 columns, compare against
-//               the per-(user, tile) thresholds, count in registers (MODE 0) or emit candidates (MODE 1)
+//               the per-(user, tile) thresholds, count in registers (MODE 0) or emit candidates (MODE 1; MODE 2
+//               for recommend.cuh: acc >= t^ - E only, t^ = the user's k-th score in place of the gt score)
 // Two user tiles share every staged item tile (UT = 2 for K <= 128): 32 bytes of L2 traffic per SM and
 // clock instead of 64, which is what keeps 148 SMs under the L2 fabric's ~6300 B/clk.  The host walks
 // the catalogue in L2-sized item blocks and compacts the working set between them on the device.
@@ -347,8 +348,10 @@ eval_filter_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_consta
             // candidate masks: bit i of m1 = "may exceed the gt score", of m2 = "|score| may reach 1".  Almost every
             // lane has no candidate in a given tile (0.04 per lane and tile at 10M x 2M), so a two-compare screen
             // per score comes first and the masks are only built by the lanes that need them.
+            // MODE 2 (recommend): only "may reach the user's k-th score" (thr_lo); no |score| >= 1 clause.
             uint32_t m1[2] = {0u, 0u}, m2[2] = {0u, 0u};
-            const float t_pos = fminf(thr_lo, thr_one), t_neg = -thr_one;
+            const float t_pos = MODE == 2 ? thr_lo : fminf(thr_lo, thr_one);
+            const float t_neg = MODE == 2 ? -__int_as_float(0x7f800000) : -thr_one;
             bool hit = false;
 #pragma unroll
             for (int i = 0; i < kCols; i++) hit |= (v[i] >= t_pos) | (v[i] <= t_neg);
@@ -359,7 +362,7 @@ eval_filter_kernel(const __grid_constant__ CUtensorMap mapU, const __grid_consta
 #pragma unroll
                 for (int i = 0; i < 32; i++) {
                   b1 |= (v[c * 32 + i] >= thr_lo ? 1u : 0u) << i;
-                  b2 |= (fabsf(v[c * 32 + i]) >= thr_one ? 1u : 0u) << i;
+                  if (MODE == 1) b2 |= (fabsf(v[c * 32 + i]) >= thr_one ? 1u : 0u) << i;
                 }
                 const int lim = nvalid - c * 32;
                 const uint32_t live = lim <= 0 ? 0u : (lim >= 32 ? 0xffffffffu : ((1u << lim) - 1u));

@@ -433,6 +433,53 @@ int eals_group_evaluate(eals_group* g, const int32_t* gt_items, int32_t topk, in
   return EALS_OK;
 }
 
+// Every user goes to the rank that owns its row of the train matrix (U and V are replicated, the seen items are
+// the owner's); the ranks run at once, each on its own stream, and the results land in input order.
+int eals_group_recommend(eals_group* g, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
+                         int32_t* items, double* scores) {
+  if (!g || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(group_barrier(g));
+  if (n == 0) return EALS_OK;
+  std::vector<int32_t> hu((size_t)n);
+  if (space == EALS_DEVICE) CU(cudaMemcpy(hu.data(), users, sizeof(int32_t) * n, cudaMemcpyDeviceToHost));
+  else std::memcpy(hu.data(), users, sizeof(int32_t) * n);
+  std::vector<std::vector<int32_t>> pos((size_t)g->n), who((size_t)g->n);
+  for (int s = 0; s < n; s++) {
+    if (hu[(size_t)s] < 0 || hu[(size_t)s] >= g->base.n_users)
+      return fail(EALS_ERR_ARG, "user %d (position %d) outside [0, %d)", hu[(size_t)s], s, g->base.n_users);
+    const int q = group_owner(g->ub, hu[(size_t)s]);
+    pos[(size_t)q].push_back(s);
+    who[(size_t)q].push_back(hu[(size_t)s]);
+  }
+  const size_t nk = (size_t)n * k;
+  std::vector<int32_t> out_i(nk);
+  std::vector<double> out_s(nk);
+  OK(parallel_ranks(g, [&](int q) -> int {
+    const size_t nq = pos[(size_t)q].size();
+    if (nq == 0) return EALS_OK;
+    std::vector<int32_t> ri(nq * k);
+    std::vector<double> rs(nq * k);
+    OK(eals_recommend(g->r[q], EALS_HOST, (int32_t)nq, who[(size_t)q].data(), k, exclude_seen, ri.data(), rs.data()));
+    for (size_t t = 0; t < nq; t++) {
+      const size_t s = (size_t)pos[(size_t)q][t];
+      std::memcpy(&out_i[s * k], &ri[t * k], sizeof(int32_t) * k);
+      std::memcpy(&out_s[s * k], &rs[t * k], sizeof(double) * k);
+    }
+    return EALS_OK;
+  }));
+  if (space == EALS_DEVICE) {
+    CU(cudaMemcpy(items, out_i.data(), sizeof(int32_t) * nk, cudaMemcpyHostToDevice));
+    if (scores) CU(cudaMemcpy(scores, out_s.data(), sizeof(double) * nk, cudaMemcpyHostToDevice));
+  } else {
+    std::memcpy(items, out_i.data(), sizeof(int32_t) * nk);
+    if (scores) std::memcpy(scores, out_s.data(), sizeof(double) * nk);
+  }
+  return EALS_OK;
+}
+
 int eals_group_evaluate_user(eals_group* g, int32_t u, int32_t gt_item, int32_t topk, int32_t mode, double out[3]) {
   if (!g) return fail(EALS_ERR_ARG, "null group");
   OK(group_barrier(g));

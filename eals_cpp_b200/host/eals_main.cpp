@@ -12,12 +12,14 @@
 // Unlike the reference it takes real arguments:
 //   eals_main [--data yelp.rating] [--factors 64] [--iters 20] [--w0 10] [--alpha 0.75] [--reg 0.01]
 //             [--topk 10] [--no-loss] [--exact-eval] [--device 0] [--gpus N | --devices 0,1,..] [--online U,I]
-//             [--save FILE] [--load FILE]
+//             [--save FILE] [--load FILE] [--recommend K [--recommend-out FILE]]
 // --gpus N: shard users and items over GPUs device .. device+N-1 (eals_group: the exchange runs inside the
 // library); --devices lists them explicitly — a repeated id puts several ranks on one GPU.
 // --save / --load: factor checkpoint after training / instead of the random initialisation.
 // --dump-split FILE: write the hold-one-out split (per user: test item, then the train items) and stop before
 // the model is built — needs no GPU; the loader is checked against the reference's own binary this way.
+// --recommend K: after training and evaluation, every user's top-K unseen items, one line "user item score" per
+// recommended item (score with %.17g), to --recommend-out FILE (default: stdout).
 // --online U,I: after training and evaluation, add the interaction (U, I) with the online update
 // (updateModel, MF_fastALS.cpp:223-242) and print the prediction before and after.
 #include <algorithm>
@@ -47,7 +49,8 @@ int main(int argc, char** argv) {
   bool showProgress = false, showLoss = true, exact = false;
   int online_u = -1, online_i = -1, n_gpus = 1;
   std::vector<int> devices;
-  std::string save_path, load_path, dump_split;
+  std::string save_path, load_path, dump_split, recommend_out;
+  int recommend_k = 0;
   for (int a = 1; a < argc; a++) {
     auto is = [&](const char* f) { return std::strcmp(argv[a], f) == 0; };
     auto next = [&]() -> const char* { if (a + 1 >= argc) { std::fprintf(stderr, "missing value after %s\n", argv[a]); std::exit(2); } return argv[++a]; };
@@ -64,6 +67,8 @@ int main(int argc, char** argv) {
     else if (is("--save")) save_path = next();
     else if (is("--load")) load_path = next();
     else if (is("--dump-split")) dump_split = next();
+    else if (is("--recommend")) recommend_k = std::atoi(next());
+    else if (is("--recommend-out")) recommend_out = next();
     else if (is("--no-loss")) showLoss = false;
     else if (is("--exact-eval")) exact = true;
     else if (is("--online")) { if (std::sscanf(next(), "%d,%d", &online_u, &online_i) != 2) { std::fprintf(stderr, "--online wants U,I\n"); return 2; } }
@@ -138,6 +143,19 @@ int main(int argc, char** argv) {
     if (n_gpus > 1) std::cerr << "replicas consistent: " << (fals.replicas_consistent() ? "yes" : "NO") << std::endl;
     std::vector<double> res = fals.evaluate(exact);
     std::cout << "<hr, ndcg, prec>: \t" << res[0] << "\t" << res[1] << "\t" << res[2] << std::endl;
+    if (recommend_k > 0) {
+      std::vector<int> all((size_t)userCount);
+      for (int u = 0; u < userCount; u++) all[(size_t)u] = u;
+      const auto rec = fals.recommend(all, recommend_k, true);
+      FILE* f = recommend_out.empty() ? stdout : std::fopen(recommend_out.c_str(), "w");
+      if (!f) { std::fprintf(stderr, "Error: cannot write %s\n", recommend_out.c_str()); return EXIT_FAILURE; }
+      for (int u = 0; u < userCount; u++)
+        for (int j = 0; j < recommend_k; j++) {
+          const size_t q = (size_t)u * recommend_k + j;
+          if (rec.items[q] >= 0) std::fprintf(f, "%d %d %.17g\n", u, rec.items[q], rec.scores[q]);
+        }
+      if (f != stdout && std::fclose(f) != 0) { std::fprintf(stderr, "Error: writing %s failed\n", recommend_out.c_str()); return EXIT_FAILURE; }
+    }
     if (online_u >= 0) {
       const double before = fals.predict(online_u, online_i);
       fals.updateModel(online_u, online_i);

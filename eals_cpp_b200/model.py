@@ -176,6 +176,39 @@ def insert_interaction(sm: "SparseMat", u: int, i: int):
     return SparseMat(sm.M, sm.N, rp, ci, cp, ri, rv, cv)
 
 
+def _recommend_call(fn, handle, users, k, exclude_seen):
+    """One eals_recommend / eals_group_recommend call.  ``users``: a sequence, a numpy array or a torch tensor
+    (a CUDA tensor stays on the device: inputs and outputs then live there).  Returns torch tensors for a CUDA
+    input, numpy arrays otherwise."""
+    k = int(k)
+    if not isinstance(users, np.ndarray) and hasattr(users, "is_cuda") and users.is_cuda:
+        import torch
+        u = users.to(torch.int32).contiguous()
+        n = u.numel()
+        items = torch.empty((n, k), dtype=torch.int32, device=u.device)
+        scores = torch.empty((n, k), dtype=torch.float64, device=u.device)
+        torch.cuda.current_stream(u.device).synchronize()
+        check(fn(handle, _lib.EALS_DEVICE, n, _ptr(u), k, int(bool(exclude_seen)), _ptr(items), _ptr(scores)))
+        return items, scores
+    u = np.ascontiguousarray(users.cpu().numpy() if hasattr(users, "cpu") else users, np.int32).reshape(-1)
+    items = np.empty((u.size, k), np.int32)
+    scores = np.empty((u.size, k), np.float64)
+    check(fn(handle, _lib.EALS_HOST, u.size, _ptr(u), k, int(bool(exclude_seen)), _ptr(items), _ptr(scores)))
+    return items, scores
+
+
+def _recommend_stats(lib, h, factors):
+    out = np.zeros(7, np.int64)
+    check(lib.eals_recommend_stats(h, _ptr(out)))
+    st = {"engine": "tcgen05" if out[0] == 1 else "fp64", "seed_items": int(out[1]), "pairs_rescored": int(out[2]),
+          "users_left_after_first_block": int(out[3])}
+    if out[6] > 0:
+        kp = -(-factors // 64) * 64
+        st["first_block"] = {"users": int(out[4]), "items": int(out[5]), "ms": out[6] / 1e3,
+                             "tflops": 2.0 * out[4] * out[5] * kp / (out[6] * 1e-6) / 1e12}
+    return st
+
+
 class _DevArray:
     """Expose a raw device pointer to torch through __cuda_array_interface__."""
 
@@ -732,6 +765,68 @@ class MF_fastALS:
                                  "tflops": 2.0 * out[3] * out[4] * kp / (out[5] * 1e-6) / 1e12}
         return st
 
+    # ---- top-k retrieval -------------------------------------------------------------------------------------
+    def recommend(self, users, k, exclude_seen=True):
+        """The k items of highest score for each user: ``(items int32[n, k], scores float64[n, k])`` in the order
+        of ``users``, score = ``predict(u, i)`` bit for bit, ties by item id ascending.  ``exclude_seen`` leaves out
+        the user's items in the current train matrix; slots that cannot be filled hold item -1, score -inf.
+        ``users`` may be a torch CUDA tensor (no host round trip of the inputs).  With several ranks the call is
+        collective: every rank answers the users it owns and an all-gather gives every rank the whole result."""
+        if self.world == 1:
+            items, scores = _recommend_call(self.lib.eals_recommend, self.h, users, k, exclude_seen)
+            return (items.cpu().numpy(), scores.cpu().numpy()) if not isinstance(items, np.ndarray) else (items, scores)
+        import torch
+        import torch.distributed as dist
+        dev = f"cuda:{self.device}"
+        u = (users if hasattr(users, "to") else torch.from_numpy(np.ascontiguousarray(users, np.int32).reshape(-1)))
+        u = u.to(device=dev, dtype=torch.int32).reshape(-1)
+        n, k = u.numel(), int(k)
+        bad = u[(u < 0) | (u >= self.userCount)][:1].contiguous()
+        if bad.numel():                   # the library's own argument error (EALS_ERR_ARG)
+            out = torch.empty((1, max(k, 1)), dtype=torch.int32, device=dev)
+            check(self.lib.eals_recommend(self.h, _lib.EALS_DEVICE, 1, _ptr(bad), k, int(bool(exclude_seen)), _ptr(out), None))
+        bounds = torch.tensor(self.user_bounds, dtype=torch.int32, device=dev)
+        owner = torch.bucketize(u, bounds[1:-1], right=True)            # rank owning each position
+        counts = torch.bincount(owner, minlength=self.world).tolist()
+        mine = torch.nonzero(owner == self.rank).reshape(-1)
+        width = max(1, max(counts))
+        items = torch.full((width, k), -1, dtype=torch.int32, device=dev)
+        scores = torch.full((width, k), float("-inf"), dtype=torch.float64, device=dev)
+        # An error on one rank (arguments, out of memory, ...) must not leave the others waiting in the all-gather:
+        # every rank reports success or failure first, and all of them raise together.
+        err = None
+        try:
+            if mine.numel():
+                it, sc = _recommend_call(self.lib.eals_recommend, self.h, u[mine].contiguous(), k, exclude_seen)
+                items[:mine.numel()] = it
+                scores[:mine.numel()] = sc
+            else:
+                check(self.lib.eals_recommend(self.h, _lib.EALS_DEVICE, 0, None, k, int(bool(exclude_seen)), None, None))
+        except Exception as e:
+            err = e
+        failed = torch.tensor([0 if err is None else self.rank + 1], dtype=torch.int32, device=dev)
+        dist.all_reduce(failed, op=dist.ReduceOp.MAX, group=self.group)
+        if err is not None:
+            raise err
+        if int(failed.item()):
+            raise RuntimeError(f"recommend failed on rank {int(failed.item()) - 1}")
+        all_items = torch.empty((self.world * width, k), dtype=torch.int32, device=dev)
+        all_scores = torch.empty((self.world * width, k), dtype=torch.float64, device=dev)
+        dist.all_gather_into_tensor(all_items, items, group=self.group)
+        dist.all_gather_into_tensor(all_scores, scores, group=self.group)
+        out_i = torch.empty((n, k), dtype=torch.int32, device=dev)
+        out_s = torch.empty((n, k), dtype=torch.float64, device=dev)
+        for q in range(self.world):
+            pos = torch.nonzero(owner == q).reshape(-1)
+            out_i[pos] = all_items[q * width:q * width + counts[q]]
+            out_s[pos] = all_scores[q * width:q * width + counts[q]]
+        return out_i.cpu().numpy(), out_s.cpu().numpy()
+
+    def recommend_stats(self):
+        """How the last recommend ran on this rank: engine ('tcgen05' or 'fp64'), exact seed size, pairs re-scored,
+        users left after the first item block and that block's shape, time and tensor rate."""
+        return _recommend_stats(self.lib, self.h, self.factors)
+
     # ---- instrumentation -----------------------------------------------------------------------------------
     def timings(self):
         ms = np.zeros(6)
@@ -929,6 +1024,11 @@ class GroupMF_fastALS:
         check(self.lib.eals_group_evaluate(self.g, _ptr(items), topK, _lib.EVAL_EXACT if exact else _lib.EVAL_REFERENCE,
                                            _ptr(means), _ptr(hr), _ptr(ndcg), _ptr(prec), _ptr(cnt)))
         return (means, hr, ndcg, prec, cnt) if per_user else means
+
+    def recommend(self, users, k, exclude_seen=True):
+        """``MF_fastALS.recommend`` over all ranks: each user is answered by the rank that owns it."""
+        items, scores = _recommend_call(self.lib.eals_group_recommend, self.g, users, k, exclude_seen)
+        return (items.cpu().numpy(), scores.cpu().numpy()) if not isinstance(items, np.ndarray) else (items, scores)
 
     def replicas_consistent(self) -> bool:
         ok = C.c_int32()

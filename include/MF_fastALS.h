@@ -181,6 +181,19 @@ class MF_fastALS_T {
     }
   }
 
+  // Top-k retrieval: for each user the k items of highest score (= predict(u, i) bit for bit), ties by item id,
+  // the user's train items left out with exclude_seen.  Row-major [users.size()][k]; slots that cannot be filled
+  // hold item -1 and score -inf.  1 <= k <= 1024.
+  struct Recommendations { std::vector<int32_t> items; std::vector<double> scores; };
+  Recommendations recommend(const std::vector<int>& users, int k, bool exclude_seen = true) {
+    Recommendations r;
+    std::vector<int32_t> u(users.begin(), users.end());
+    r.items.resize(u.size() * (size_t)std::max(k, 0));
+    r.scores.resize(r.items.size());
+    check(eals_group_recommend(g_, EALS_HOST, (int32_t)u.size(), u.data(), k, exclude_seen ? 1 : 0, r.items.data(),
+                               r.scores.data()), "eals_group_recommend");
+    return r;
+  }
   void update_user_thread(int u) { check(eals_group_update_user_row(g_, u), "eals_group_update_user_row"); }
   void update_item_thread(int i) { check(eals_group_update_item_row(g_, i), "eals_group_update_item_row"); }
   void update_user_SU(double* oldVector, double* uget) { check(eals_group_patch_SU(g_, oldVector, uget), "eals_group_patch_SU"); }

@@ -216,6 +216,21 @@ int eals_evaluate_user(eals_model* m, int32_t u, int32_t gt_item, int32_t topk, 
  * items: the one launch of known shape, 2 * users * items * roundup(factors, 64) flop — the tensor roofline). */
 int eals_eval_stats(eals_model* m, int64_t out[6]);
 
+/* Top-k retrieval: for each of the n users (global ids, owned by this model), the k items of highest score,
+ * score = predict(u, i) bit for bit, ordered by score descending and item id ascending.  With exclude_seen != 0
+ * the items of the user's row of the current train matrix (after eals_set_train) are left out.  Slots a user
+ * cannot fill (fewer than k eligible items) hold item -1 and score -inf.  items: [n][k] int32, scores: [n][k]
+ * double or NULL; users, items and scores are host or device memory as `space` says (EALS_HOST / EALS_DEVICE).
+ * 1 <= k <= 1024.  Lists of >= 128 users with factors <= 256 go through the tcgen05 filter (every output decided
+ * by exact fp64 comparisons; the same result as the exact engine); EALS_EVAL_SCALAR=1 forces the exact engine. */
+int eals_recommend(eals_model* m, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
+                   int32_t* items, double* scores);
+/* How the last eals_recommend ran (7 values): out[0] = engine (1 tcgen05 filter, 0 exact fp64), out[1] = items of
+ * the exact seed, out[2] = candidate pairs re-scored exactly, out[3] = users still in the working set after the
+ * first item block, out[4], out[5], out[6] = users, items and device microseconds of the filter's first item
+ * block (2 * users * items * roundup(factors, 64) flop). */
+int eals_recommend_stats(eals_model* m, int64_t out[7]);
+
 /* Plumbing for the host layer. */
 int eals_leading_dim(const eals_model* m);                 /* ld of U/V/SU/SV rows, in doubles   */
 int eals_device_buffer(eals_model* m, int32_t which, void** dev_ptr, int64_t* bytes);
@@ -304,6 +319,9 @@ int eals_group_predict(eals_group* g, int32_t u, int32_t i, double* score);
 int eals_group_evaluate(eals_group* g, const int32_t* gt_items, int32_t topk, int32_t mode, double means[3],
                         double* hr, double* ndcg, double* prec, int32_t* count_larger);
 int eals_group_evaluate_user(eals_group* g, int32_t u, int32_t gt_item, int32_t topk, int32_t mode, double out[3]);
+/* eals_recommend over the whole user range: each user is answered by the rank that owns it, results in input order. */
+int eals_group_recommend(eals_group* g, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
+                         int32_t* items, double* scores);
 int eals_group_sync(eals_group* g);
 int eals_group_replicas_consistent(eals_group* g, int32_t* ok);             /* all U / V replicas bit-identical */
 int eals_group_save_factors(eals_group* g, const char* path);
