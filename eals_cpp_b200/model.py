@@ -197,15 +197,20 @@ def _recommend_call(fn, handle, users, k, exclude_seen):
     return items, scores
 
 
+def _first_block(users, items, us, factors):
+    """The first filtered item block's shape, device time and tensor rate (factors padded to 64 in fp16)."""
+    kp = -(-factors // 64) * 64
+    return {"users": int(users), "items": int(items), "ms": us / 1e3,
+            "tflops": 2.0 * users * items * kp / (us * 1e-6) / 1e12}
+
+
 def _recommend_stats(lib, h, factors):
     out = np.zeros(7, np.int64)
     check(lib.eals_recommend_stats(h, _ptr(out)))
     st = {"engine": "tcgen05" if out[0] == 1 else "fp64", "seed_items": int(out[1]), "pairs_rescored": int(out[2]),
           "users_left_after_first_block": int(out[3])}
     if out[6] > 0:
-        kp = -(-factors // 64) * 64
-        st["first_block"] = {"users": int(out[4]), "items": int(out[5]), "ms": out[6] / 1e3,
-                             "tflops": 2.0 * out[4] * out[5] * kp / (out[6] * 1e-6) / 1e12}
+        st["first_block"] = _first_block(out[4], out[5], out[6], factors)
     return st
 
 
@@ -760,9 +765,7 @@ class MF_fastALS:
         check(self.lib.eals_eval_stats(self.h, _ptr(out)))
         st = {"engine": "tcgen05" if out[0] == 1 else "fp64", "candidates": int(out[1]), "pairs_rescored": int(out[2])}
         if out[5] > 0:
-            kp = -(-self.factors // 64) * 64
-            st["first_block"] = {"users": int(out[3]), "items": int(out[4]), "ms": out[5] / 1e3,
-                                 "tflops": 2.0 * out[3] * out[4] * kp / (out[5] * 1e-6) / 1e12}
+            st["first_block"] = _first_block(out[3], out[4], out[5], self.factors)
         return st
 
     # ---- top-k retrieval -------------------------------------------------------------------------------------
