@@ -78,6 +78,8 @@ SIGNATURES = {
     "eals_eval_stats": (C.c_int, [_P, _P]),
     "eals_recommend": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
     "eals_recommend_stats": (C.c_int, [_P, _P]),
+    "eals_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
+    "eals_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     "eals_leading_dim": (C.c_int, [_P]),
     "eals_device_buffer": (C.c_int, [_P, C.c_int32, C.POINTER(_P), C.POINTER(C.c_int64)]),
     "eals_stream": (C.c_int, [_P, C.POINTER(_P)]),
@@ -119,6 +121,8 @@ SIGNATURES = {
     "eals_group_evaluate": (C.c_int, [_P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P, _P]),
     "eals_group_evaluate_user": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, C.c_int32, _P]),
     "eals_group_recommend": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
+    "eals_group_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
+    "eals_group_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     "eals_group_sync": (C.c_int, [_P]),
     "eals_group_replicas_consistent": (C.c_int, [_P, C.POINTER(C.c_int32)]),
     "eals_group_save_factors": (C.c_int, [_P, C.c_char_p]),

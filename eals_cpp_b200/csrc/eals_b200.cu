@@ -680,9 +680,10 @@ int build_launch_order(eals_model* m, Side& s) {
   return done(EALS_OK);
 }
 
-// Upload the owned slice [begin, end) of one orientation of the matrix and bucket its rows.
+// Upload the owned slice [begin, end) of one orientation of the matrix and bucket its rows.  `check` is 6 ints of
+// device scratch that belong to this side alone (the validation's read-back overlaps the host bucketing).
 int build_side(eals_model* m, Side& s, int begin, int end, int other_dim, int space,
-               const int64_t* ptr_full, const int32_t* idx_full, const double* val_full) {
+               const int64_t* ptr_full, const int32_t* idx_full, const double* val_full, int* check) {
   StageTimer tm;
   s.rows = end - begin;
   s.row_base = begin;
@@ -733,7 +734,7 @@ int build_side(eals_model* m, Side& s, int begin, int end, int other_dim, int sp
   // indices must ascend strictly inside a row and stay in range (main.cpp:198-205 order)
   int* sorted_flag = nullptr;
   if (s.rows > 0) {
-    int* bad = m->flags + (&s == &m->users ? 0 : 8);          // 6 ints: bad, pad, descents (u64), row-start descents (u64)
+    int* bad = check;                                          // 6 ints: bad, pad, descents (u64), row-start descents (u64)
     unsigned long long* counts = reinterpret_cast<unsigned long long*>(bad + 2);
     CU(cudaMemsetAsync(bad, 0, 6 * sizeof(int), m->stream));
     if (s.nnz > 0) {
@@ -1126,8 +1127,10 @@ int run_heavy_batch(eals_model* m, Side& s, const CdSide& a, const HeavyBatch& b
   return EALS_OK;
 }
 
+// timed: the whole-side launches go to the sweep sub-phase timers (eals_timings_detail); fold-in runs the same
+// kernels untimed, so the timers keep reporting training sweeps only.
 template <int LD, bool USER>
-int launch_cd(eals_model* m, Side& s, const CdSide& a, int only_row) {
+int launch_cd(eals_model* m, Side& s, const CdSide& a, int only_row, bool timed) {
   if (only_row >= 0) {  // single-row API: a one-entry order list in scratch
     const int64_t n = s.h_ptr[only_row + 1] - s.h_ptr[only_row];
     if (n == 0) return EALS_OK;
@@ -1148,21 +1151,19 @@ int launch_cd(eals_model* m, Side& s, const CdSide& a, int only_row) {
   }
   // heavy rows first: their launch chain is the longest
   const int t0 = USER ? T_U_HEAVY : T_I_HEAVY;
-  tic(m, t0);
+  if (timed) tic(m, t0);
   for (const HeavyBatch& b : s.batches) OK((run_heavy_batch<LD, USER>(m, s, a, b, true)));
-  toc(m, t0);
-  tic(m, t0 + 1);
+  if (timed) { toc(m, t0); tic(m, t0 + 1); }
   OK((launch_cd_row_block<LD, 8, 2, USER>(m, a, s.order, s.first[7], s.first[8] - s.first[7])));   // 385..512
   OK((launch_cd_row_block<LD, 4, 3, USER>(m, a, s.order, s.first[6], s.first[7] - s.first[6])));   // 257..384
   OK((launch_cd_row_block<LD, 4, 2, USER>(m, a, s.order, s.first[5], s.first[6] - s.first[5])));   // 129..256
-  toc(m, t0 + 1);
-  tic(m, t0 + 2);
+  if (timed) { toc(m, t0 + 1); tic(m, t0 + 2); }
   // one warp per row up to 128 nonzeros: no CTA barrier anywhere in the row loop
   OK((launch_cd_warp_block<LD, 4, USER>(m, a, s.order, s.first[4], s.first[5] - s.first[4])));
   OK((launch_cd_warp_block<LD, 3, USER>(m, a, s.order, s.first[3], s.first[4] - s.first[3])));
   OK((launch_cd_warp_block<LD, 2, USER>(m, a, s.order, s.first[2], s.first[3] - s.first[2])));
   OK((launch_cd_warp_block<LD, 1, USER>(m, a, s.order, s.first[1], s.first[2] - s.first[1])));
-  toc(m, t0 + 2);
+  if (timed) toc(m, t0 + 2);
   return EALS_OK;
 }
 
@@ -1307,8 +1308,8 @@ int sweep(eals_model* m, bool user, int only_row) {
     in_valid = false;    // this side's cache describes the factors BEFORE this sweep
     out_valid = true;    // every nonzero's final prediction is stored on the other side by this sweep
   }
-  if (user) { DISPATCH_LD(m->LD, OK((launch_cd<LD, true>(m, s, a, only_row)))); }
-  else      { DISPATCH_LD(m->LD, OK((launch_cd<LD, false>(m, s, a, only_row)))); }
+  if (user) { DISPATCH_LD(m->LD, OK((launch_cd<LD, true>(m, s, a, only_row, true)))); }
+  else      { DISPATCH_LD(m->LD, OK((launch_cd<LD, false>(m, s, a, only_row, true)))); }
   if (a.pc_stage && s.nnz > 0) {
     // Second phase: staged predictions to their owners, in destination order.  Nobody needs them before the
     // NEXT half-epoch's sweep, so the copy is launched by gram() on a side stream right behind the Gram's main
@@ -1618,8 +1619,8 @@ int eals_create(const eals_params* params, const int64_t* row_ptr, const int32_t
   TRYCU(cudaMemsetAsync(m->SU, 0, sizeof(double) * (size_t)m->LD * m->LD, m->stream));
   TRYCU(cudaMemsetAsync(m->SV, 0, sizeof(double) * (size_t)m->LD * m->LD, m->stream));
   TRYCU(cudaMemsetAsync(m->terms, 0, sizeof(double) * 4, m->stream));
-  TRY(build_side(m, m->users, m->ub, m->ue, m->N, params->input_space, row_ptr, col_idx, row_val));
-  TRY(build_side(m, m->items, m->ib, m->ie, m->M, params->input_space, col_ptr, row_idx, col_val));
+  TRY(build_side(m, m->users, m->ub, m->ue, m->N, params->input_space, row_ptr, col_idx, row_val, m->flags));
+  TRY(build_side(m, m->items, m->ib, m->ie, m->M, params->input_space, col_ptr, row_idx, col_val, m->flags + 8));
   TRY(compute_item_weights(m, params->input_space, col_ptr));
   TRY(build_pred_cache(m, params->input_space, row_ptr, col_idx, col_ptr, row_idx));
   TRYCU(cudaStreamSynchronize(m->stream));
@@ -1636,8 +1637,8 @@ int eals_set_train(eals_model* m, int32_t input_space, const int64_t* row_ptr, c
   if ((row_val == nullptr) != (col_val == nullptr)) return fail(EALS_ERR_ARG, "row_val and col_val must both be given or both be null");
   CU(cudaSetDevice(m->p.device));
   m->config_gen++;
-  OK(build_side(m, m->users, m->ub, m->ue, m->N, input_space, row_ptr, col_idx, row_val));
-  OK(build_side(m, m->items, m->ib, m->ie, m->M, input_space, col_ptr, row_idx, col_val));
+  OK(build_side(m, m->users, m->ub, m->ue, m->N, input_space, row_ptr, col_idx, row_val, m->flags));
+  OK(build_side(m, m->items, m->ib, m->ie, m->M, input_space, col_ptr, row_idx, col_val, m->flags + 8));
   return build_pred_cache(m, input_space, row_ptr, col_idx, col_ptr, row_idx);
 }
 
@@ -2024,6 +2025,16 @@ int eals_eval_stats(eals_model* m, int64_t out[6]) {
 int eals_recommend(eals_model* m, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
                    int32_t* items, double* scores) {
   return recommend_impl(m, space, n, users, k, exclude_seen, items, scores);
+}
+
+int eals_fold_in(eals_model* m, int32_t space, int32_t n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
+                 const double* init, int32_t n_iter, double* out) {
+  return fold_in_impl(m, space, n, row_ptr, col_idx, val, init, n_iter, out);
+}
+
+int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
+                           int32_t k, int32_t* items, double* scores) {
+  return recommend_vectors_impl(m, space, n, Q, ex_ptr, ex_idx, k, items, scores);
 }
 
 int eals_recommend_stats(eals_model* m, int64_t out[7]) {

@@ -480,6 +480,115 @@ int eals_group_recommend(eals_group* g, int32_t space, int32_t n, const int32_t*
   return EALS_OK;
 }
 
+}  // extern "C"
+
+namespace {
+
+// The n queries of fold_in / recommend_vectors in balanced contiguous slices over the ranks (V, SV and Wi are
+// replicated: any rank can answer any query), the ranks at once.  Device inputs are staged through the host like
+// eals_group_recommend's, so each rank reads them whatever device it is on; fn(rank, lo, hi) runs a host-space call.
+template <typename F>
+int group_slices(eals_group* g, int n, F fn) {
+  return parallel_ranks(g, [&](int q) -> int {
+    const int lo = (int)((int64_t)n * q / g->n), hi = (int)((int64_t)n * (q + 1) / g->n);
+    return hi > lo ? fn(q, lo, hi) : EALS_OK;
+  });
+}
+
+// A host copy of a CSR of n rows (host or device), offsets rebased to 0; val stays empty for NULL.
+struct HostCsr {
+  std::vector<int64_t> ptr;
+  std::vector<int32_t> idx;
+  std::vector<double> val;
+  int load(int space, int n, const int64_t* p, const int32_t* i, const double* v) {
+    ptr.resize((size_t)n + 1);
+    if (space == EALS_DEVICE) CU(cudaMemcpy(ptr.data(), p, sizeof(int64_t) * (n + 1), cudaMemcpyDeviceToHost));
+    else std::memcpy(ptr.data(), p, sizeof(int64_t) * (n + 1));
+    const int64_t base = ptr[0], nnz = ptr[(size_t)n] - base;
+    if (nnz < 0) return fail(EALS_ERR_ARG, "offsets not monotone");
+    for (auto& x : ptr) x -= base;
+    idx.resize((size_t)std::max<int64_t>(nnz, 1));   // a non-null index array even when every row is empty
+    if (v) val.resize((size_t)nnz);
+    if (space == EALS_DEVICE) {
+      if (nnz) CU(cudaMemcpy(idx.data(), i + base, sizeof(int32_t) * nnz, cudaMemcpyDeviceToHost));
+      if (v && nnz) CU(cudaMemcpy(val.data(), v + base, sizeof(double) * nnz, cudaMemcpyDeviceToHost));
+    } else {
+      if (nnz) std::memcpy(idx.data(), i + base, sizeof(int32_t) * nnz);
+      if (v && nnz) std::memcpy(val.data(), v + base, sizeof(double) * nnz);
+    }
+    return EALS_OK;
+  }
+  const double* vals(const double* given) const { return given ? val.data() : nullptr; }
+};
+
+// Host staging of `count` elements of a host or device array (device: copied; host: the caller's memory).
+template <typename T>
+int host_view(int space, const T* src, size_t count, std::vector<T>& buf, const T** out) {
+  if (!src || space == EALS_HOST) { *out = src; return EALS_OK; }
+  buf.resize(count);
+  if (count) CU(cudaMemcpy(buf.data(), src, sizeof(T) * count, cudaMemcpyDeviceToHost));
+  *out = buf.data();
+  return EALS_OK;
+}
+
+// Results staged in host memory -> the caller's host or device array.
+template <typename T>
+int host_result(int space, T* dst, const std::vector<T>& buf) {
+  if (space == EALS_DEVICE) CU(cudaMemcpy(dst, buf.data(), sizeof(T) * buf.size(), cudaMemcpyHostToDevice));
+  else std::memcpy(dst, buf.data(), sizeof(T) * buf.size());
+  return EALS_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int eals_group_fold_in(eals_group* g, int32_t space, int32_t n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
+                       const double* init, int32_t n_iter, double* out) {
+  if (!g || (n > 0 && (!row_ptr || !col_idx || !out))) return fail(EALS_ERR_ARG, "null argument");
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (n_iter < 1) return fail(EALS_ERR_ARG, "n_iter must be >= 1, got %d", n_iter);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(group_barrier(g));
+  if (n == 0) return EALS_OK;
+  const size_t K = (size_t)g->base.factors;
+  HostCsr h;
+  OK(h.load(space, n, row_ptr, col_idx, val));
+  std::vector<double> init_buf, res((size_t)n * K);
+  const double* hinit = nullptr;
+  OK(host_view(space, init, (size_t)n * K, init_buf, &hinit));
+  OK(group_slices(g, n, [&](int q, int lo, int hi) {
+    return eals_fold_in(g->r[q], EALS_HOST, hi - lo, h.ptr.data() + lo, h.idx.data(), h.vals(val), hinit ? hinit + lo * K : nullptr,
+                        n_iter, res.data() + lo * K);
+  }));
+  return host_result(space, out, res);
+}
+
+int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr,
+                                 const int32_t* ex_idx, int32_t k, int32_t* items, double* scores) {
+  if (!g || (n > 0 && (!Q || !items))) return fail(EALS_ERR_ARG, "null argument");
+  if ((ex_ptr == nullptr) != (ex_idx == nullptr)) return fail(EALS_ERR_ARG, "ex_ptr and ex_idx must both be given or both be null");
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(group_barrier(g));
+  if (n == 0) return EALS_OK;
+  const size_t K = (size_t)g->base.factors;
+  HostCsr ex;
+  if (ex_ptr) OK(ex.load(space, n, ex_ptr, ex_idx, nullptr));
+  std::vector<double> q_buf, out_s((size_t)n * k);
+  std::vector<int32_t> out_i((size_t)n * k);
+  const double* hq = nullptr;
+  OK(host_view(space, Q, (size_t)n * K, q_buf, &hq));
+  OK(group_slices(g, n, [&](int q, int lo, int hi) {
+    return eals_recommend_vectors(g->r[q], EALS_HOST, hi - lo, hq + lo * K, ex_ptr ? ex.ptr.data() + lo : nullptr,
+                                  ex_ptr ? ex.idx.data() : nullptr, k, out_i.data() + (size_t)lo * k, out_s.data() + (size_t)lo * k);
+  }));
+  OK(host_result(space, items, out_i));
+  if (scores) OK(host_result(space, scores, out_s));
+  return EALS_OK;
+}
+
 int eals_group_evaluate_user(eals_group* g, int32_t u, int32_t gt_item, int32_t topk, int32_t mode, double out[3]) {
   if (!g) return fail(EALS_ERR_ARG, "null group");
   OK(group_barrier(g));

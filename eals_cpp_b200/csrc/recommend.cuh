@@ -44,12 +44,12 @@ __device__ __forceinline__ bool row_has(const int32_t* __restrict__ idx, int64_t
 }
 
 struct MergeArgs {
-  const double* U; const double* V; int K, LD;
-  const int32_t* users;                 // slot -> global user id
+  const double* U; const double* V; int K, LD;   // U: the query rows (the model's U, or query vectors)
+  const int32_t* users;                 // slot -> row of U (nullable: the slot itself)
   int k;
   double* top_s; int32_t* top_i;        // [n][k] per slot
   double* thr;                          // [n] per slot: score of the k-th entry (-inf while the list is not full)
-  // seen items: CSR of the owned user rows (row = user - row_base); ptr == nullptr: no exclusion
+  // excluded items: CSR with a row per row of U (row = U row - row_base); ptr == nullptr: no exclusion
   const int64_t* ptr; const int32_t* idx; int row_base;
   // SRC_EXACT: list of slots (nullable: block b = slot b) and the items order[r0 .. r1) (order nullable: identity)
   const int32_t* list; const int32_t* order; int r0, r1;
@@ -84,7 +84,7 @@ rec_merge_kernel(MergeArgs a) {
     c0 = a.run_off[blockIdx.x];
     c_n = a.run_cnt[blockIdx.x];
   }
-  const int u = a.users[slot];
+  const int u = a.users ? a.users[slot] : slot;
   double* ts = a.top_s + (size_t)slot * k;
   int32_t* ti = a.top_i + (size_t)slot * k;
   for (int t = tid; t < P; t += kThreads) {
@@ -184,6 +184,16 @@ __global__ void rec_init_kernel(double* __restrict__ top_s, int32_t* __restrict_
   }
 }
 
+// Every factor of the query rows X[0 .. n) finite (the filter's error bound assumes it); bad[0] = 1 + first
+// offending row otherwise.
+__global__ void rec_check_finite_kernel(const double* __restrict__ X, int n, int K, int LD, int* __restrict__ bad) {
+  const size_t total = (size_t)n * K;
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+    const size_t r = t / K;
+    if (!isfinite(X[r * LD + t % K])) atomicMin(bad, (int)r + 1);
+  }
+}
+
 // users[s] in [lo, hi) for every s; bad[0] = 1 + first offending position otherwise
 __global__ void rec_check_users_kernel(const int32_t* __restrict__ users, int n, int lo, int hi, int* __restrict__ bad) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -196,7 +206,8 @@ __global__ void rec_finish_kernel(int32_t* __restrict__ top_i, size_t n) {
     if (top_i[t] == kNoItem) top_i[t] = -1;
 }
 
-// Exact scores of the filter's candidate pairs (seq_dot, bit-identical to predict) and the slot sort keys.
+// Exact scores of the filter's candidate pairs (seq_dot, bit-identical to predict) and the slot sort keys.  users:
+// slot -> row of U (nullable: the slot itself).
 template <typename Pair>
 __global__ void __launch_bounds__(128)
 rec_rescore_kernel(const double* __restrict__ U, const double* __restrict__ V, int K, int LD, const int32_t* __restrict__ users,
@@ -211,7 +222,7 @@ rec_rescore_kernel(const double* __restrict__ U, const double* __restrict__ V, i
     if (live) {
       const Pair pr = pairs[t];
       slot = pr.slot;
-      pa = U + (size_t)users[pr.slot] * LD;
+      pa = U + (size_t)(users ? users[pr.slot] : pr.slot) * LD;
       pb = V + (size_t)pr.item * LD;
     }
     const double acc = seq_dot_warp32(pa, pb, K, sm[threadIdx.x >> 5]);

@@ -136,6 +136,13 @@ struct eals_eval_ws {
   WsBuf<int32_t> top_i, pval, pval_out, run_cnt, run_off;
   WsBuf<uint32_t> pkey, pkey_out, run_slot;
   BlockTimer blk0;
+  // fold-in and recommend_vectors: the histories / exclusion lists (validated and bucketed by build_side, row_base
+  // 0), their validation scratch (6 ints each), and the query rows [n][LD] (fold-in's X, padding columns zero)
+  Side hist, excl;
+  WsBuf<int> hist_check, excl_check;
+  WsBuf<double> qx;
+  eals_eval_ws() = default;
+  ~eals_eval_ws() { free_side(hist); free_side(excl); }
 };
 
 namespace {
@@ -378,10 +385,10 @@ int select_flagged(eals_model* m, const int32_t* in, int n, int32_t* out, int32_
   return in ? run(in) : run(thrust::counting_iterator<int32_t>(0));
 }
 
-// Preparation of the tcgen05 filter for the users d_users[0 .. n) (evaluate and recommend): fp16 copies of V in
-// decreasing-norm order (ws.perm: rank -> item) and of the users' rows, their norms, the per-tile item norms and
-// the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).
-int tc_prepare(eals_model* m, int n, const int32_t* d_users, const double* d_thr) {
+// Preparation of the tcgen05 filter for the rows X[d_rows[0 .. n)] (d_rows nullable: X[0 .. n); evaluate and
+// recommend): fp16 copies of V in decreasing-norm order (ws.perm: rank -> item) and of the query rows, their norms,
+// the per-tile item norms and the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).
+int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
   const int K = m->K, LD = m->LD, N = m->N;
@@ -416,7 +423,7 @@ int tc_prepare(eals_model* m, int n, const int32_t* d_users, const double* d_thr
   }
   {
     tc::PrepOut o{ws.Uh.p, ws.un_hat.p, ws.un_del.p, ws.un_h.p, ws.exps.p};
-    tc::prep_rows_kernel<true><<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(m->U, K, LD, KP, n, d_users, 0, d_vmax, o);
+    tc::prep_rows_kernel<true><<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(X, K, LD, KP, n, d_rows, 0, d_vmax, o);
     OK(check_launch(m));
     const double gamma = (double)KP * (1.0 / 2097152.0);   // KP * 2^-21
     tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_thr, ws.exps.p, d_vmax, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n, gamma, ws.sp0.p, ws.sp1.p);
@@ -434,7 +441,7 @@ int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, i
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
   cudaStream_t st = m->stream;
-  OK(tc_prepare(m, n, d_users, d_gts));
+  OK(tc_prepare(m, n, m->U, d_users, d_gts));
   CU(cudaMemsetAsync(ws.cnt.p, 0, sizeof(int32_t) * n, st));
   CU(cudaMemsetAsync(ws.cnt_exact.p, 0, sizeof(int32_t) * n, st));
   CUtensorMap mapV, mapU0, mapW;
@@ -619,12 +626,30 @@ int evaluate_slots(eals_model* m, const std::vector<int32_t>& users_h, const int
 // ---- top-k retrieval (recommend.cuh) --------------------------------------------------------------------
 namespace rec = eals::rec;
 
-rec::MergeArgs rec_args(eals_model* m, const int32_t* d_users, int k, bool exclude) {
+// What the engines answer: slot s asks for the top-k of row rows[s] of X (rows nullable: row s), its excluded items
+// being row (that row - ex_base) of the CSR ex_ptr / ex_idx (ex_ptr nullable: none).  recommend: the model's U, the
+// users, the owned train rows; recommend_vectors: the query vectors copied to [n][LD], the identity, the caller's
+// exclusion lists.
+struct RecQuery {
+  const double* X;
+  const int32_t* rows;
+  const int64_t* ex_ptr;
+  const int32_t* ex_idx;
+  int ex_base;
+  RecQuery from(int s0, int LD) const {   // the same query for the slots s0 ..
+    RecQuery q = *this;
+    if (rows) q.rows += s0;
+    else { q.X += (size_t)s0 * LD; if (q.ex_ptr) q.ex_ptr += s0; }
+    return q;
+  }
+};
+
+rec::MergeArgs rec_args(eals_model* m, const RecQuery& q, int k) {
   eals_eval_ws& ws = eval_ws(m);
   rec::MergeArgs a{};
-  a.U = m->U; a.V = m->V; a.K = m->K; a.LD = m->LD; a.users = d_users; a.k = k;
+  a.U = q.X; a.V = m->V; a.K = m->K; a.LD = m->LD; a.users = q.rows; a.k = k;
   a.top_s = ws.top_s.p; a.top_i = ws.top_i.p; a.thr = ws.thr.p;
-  if (exclude) { a.ptr = m->users.ptr; a.idx = m->users.idx; a.row_base = m->users.row_base; }
+  a.ptr = q.ex_ptr; a.idx = q.ex_idx; a.row_base = q.ex_base;
   return a;
 }
 
@@ -644,9 +669,9 @@ int rec_merge_exact(eals_model* m, rec::MergeArgs a, const int32_t* list, int n_
 
 // Engine 1: exact fp64 scores of every item.  Short lists, the reference of the tensor-core engine
 // (EALS_EVAL_SCALAR=1) and its fall-back.
-int rec_exact(eals_model* m, int n, const int32_t* d_users, int k, bool exclude) {
+int rec_exact(eals_model* m, int n, const RecQuery& q, int k) {
   OK(rec_reset(m, n, k));
-  return rec_merge_exact(m, rec_args(m, d_users, k, exclude), nullptr, n, nullptr, 0, m->N);
+  return rec_merge_exact(m, rec_args(m, q, k), nullptr, n, nullptr, 0, m->N);
 }
 
 // Engine 2: tcgen05 filter.  Seed: the highest-norm items scored exactly (extended tile by tile for users whose
@@ -654,7 +679,7 @@ int rec_exact(eals_model* m, int n, const int32_t* d_users, int k, bool exclude)
 // (t = the user's current k-th score), the pairs are re-scored exactly and merged, t rises, and a user leaves
 // the working set once a Cauchy-Schwarz bound on every remaining item is below t (DESIGN.md §3.5).  Fills `stats`
 // (engine 1) when it answers; leaves them as they are when the filter stops filtering.
-int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, RecStats& stats) {
+int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
   StageTimer tm;
@@ -664,7 +689,7 @@ int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, Re
   const int ut = nkc <= 2 ? 2 : 1;
   cudaStream_t st = m->stream;
   OK(rec_reset(m, n, k));
-  OK(tc_prepare(m, n, d_users, ws.thr.p));
+  OK(tc_prepare(m, n, q.X, q.rows, ws.thr.p));
   const double gamma = (double)KP * (1.0 / 2097152.0);
   auto params = [&]() -> int {   // per-slot filter thresholds from the current k-th scores
     tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(ws.thr.p, ws.exps.p, ws.counters.p, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n,
@@ -685,7 +710,7 @@ int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, Re
     CU(cudaStreamSynchronize(st));
     return EALS_OK;
   };
-  const rec::MergeArgs base = rec_args(m, d_users, k, exclude);
+  const rec::MergeArgs base = rec_args(m, q, k);
 
   // ---- seed ----
   const int seed = (int)std::min<int64_t>(N, ((int64_t)k + tc::kTN - 1) / tc::kTN * tc::kTN);
@@ -768,7 +793,7 @@ int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, Re
         OK(ws.pscore.reserve((size_t)got)); OK(ws.pkey.reserve((size_t)got)); OK(ws.pkey_out.reserve((size_t)got));
         OK(ws.pval.reserve((size_t)got)); OK(ws.pval_out.reserve((size_t)got));
         OK(ws.run_slot.reserve((size_t)got)); OK(ws.run_cnt.reserve((size_t)got)); OK(ws.run_off.reserve((size_t)got));
-        rec::rec_rescore_kernel<tc::EvalPair><<<16 * m->sm_count, 128, 0, st>>>(m->U, m->V, K, m->LD, d_users, ws.pairs.p, got,
+        rec::rec_rescore_kernel<tc::EvalPair><<<16 * m->sm_count, 128, 0, st>>>(q.X, m->V, K, m->LD, q.rows, ws.pairs.p, got,
                                                                                ws.pscore.p, ws.pkey.p, ws.pval.p);
         OK(check_launch(m));
         const int ng = (int)got, end_bit = slot_bits(n);
@@ -804,13 +829,53 @@ int rec_tc(eals_model* m, int n, const int32_t* d_users, int k, bool exclude, Re
   return EALS_OK;
 }
 
-int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k, int exclude, int32_t* items, double* scores) {
-  if (!m || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
+// Answers the slots 0 .. n-1 of q into items / scores (host or device memory as `space` says) and m->rec_stats.
+int rec_answer(eals_model* m, int space, int n, const RecQuery& q, int k, int32_t* items, double* scores) {
+  eals_eval_ws& ws = eval_ws(m);
+  // Per-slot lists for at most `per` slots at a time (12 bytes per entry; EALS_REC_LIST_BYTES, default 4 GiB): the
+  // slots are answered in balanced chunks, each a complete call of an engine.
+  size_t list_bytes = (size_t)4 << 30;
+  if (const char* e = getenv("EALS_REC_LIST_BYTES")) list_bytes = std::max<size_t>(12 * (size_t)k, strtoull(e, nullptr, 10));
+  const int max_per = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, list_bytes / (12 * (size_t)k)));
+  const int n_chunks = (n + max_per - 1) / max_per, per = (n + n_chunks - 1) / n_chunks;
+  const size_t pk = (size_t)per * k;
+  OK(ws.top_s.reserve(pk)); OK(ws.top_i.reserve(pk)); OK(ws.thr.reserve((size_t)per));
+  const cudaMemcpyKind kind = space == EALS_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+  RecStats total;
+  for (int s0 = 0; s0 < n; s0 += per) {
+    const int nc = std::min(per, n - s0);
+    const size_t nck = (size_t)nc * k;
+    const RecQuery qc = q.from(s0, m->LD);
+    RecStats c;   // stays zero for a chunk of the exact engine
+    if (use_tc_engine(m, nc)) OK(rec_tc(m, nc, qc, k, c));
+    if (c.engine == 0) OK(rec_exact(m, nc, qc, k));
+    if (s0 == 0) total = c;                              // engine, seed and the first block from chunk 0
+    else { total.pairs += c.pairs; total.left1 += c.left1; }
+    if (c.engine == 0) { total.engine = 0; total.seed = 0; }   // tcgen05 and its seed only if every chunk ran there
+    rec::rec_finish_kernel<<<4 * m->sm_count, 256, 0, m->stream>>>(ws.top_i.p, nck);
+    OK(check_launch(m));
+    CU(cudaMemcpyAsync(items + (size_t)s0 * k, ws.top_i.p, sizeof(int32_t) * nck, kind, m->stream));
+    if (scores) CU(cudaMemcpyAsync(scores + (size_t)s0 * k, ws.top_s.p, sizeof(double) * nck, kind, m->stream));
+    CU(cudaStreamSynchronize(m->stream));   // the lists are reused by the next chunk
+  }
+  m->rec_stats = total;
+  CU(cudaStreamSynchronize(m->stream));
+  return EALS_OK;
+}
+
+// The argument checks every top-k call shares.
+int rec_check_args(eals_model* m, int space, int n, int k) {
   if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
   if (k < 1 || k > rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", rec::kMaxK, k);
   if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
   if (!m->factors_set) return fail(EALS_ERR_STATE, "factors not initialised");
   if (m->K > rec::kMaxFactors) return fail(EALS_ERR_UNSUPPORTED, "recommend supports up to %d factors", rec::kMaxFactors);
+  return EALS_OK;
+}
+
+int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k, int exclude, int32_t* items, double* scores) {
+  if (!m || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
+  OK(rec_check_args(m, space, n, k));
   CU(cudaSetDevice(m->p.device));
   if (n == 0) return EALS_OK;
   if (space == EALS_HOST)
@@ -820,14 +885,7 @@ int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k,
         return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", users[s], s, m->ub, m->ue);
     }
   eals_eval_ws& ws = eval_ws(m);
-  // Per-slot lists for at most `per` users at a time (12 bytes per entry; EALS_REC_LIST_BYTES, default 4 GiB): the
-  // users are answered in balanced chunks, each a complete call of an engine.
-  size_t list_bytes = (size_t)4 << 30;
-  if (const char* e = getenv("EALS_REC_LIST_BYTES")) list_bytes = std::max<size_t>(12 * (size_t)k, strtoull(e, nullptr, 10));
-  const int max_per = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, list_bytes / (12 * (size_t)k)));
-  const int n_chunks = (n + max_per - 1) / max_per, per = (n + n_chunks - 1) / n_chunks;
-  const size_t pk = (size_t)per * k;
-  OK(ws.users.reserve((size_t)n)); OK(ws.top_s.reserve(pk)); OK(ws.top_i.reserve(pk)); OK(ws.thr.reserve((size_t)per));
+  OK(ws.users.reserve((size_t)n));
   OK(copy_in(ws.users.p, users, (size_t)n, space, m->stream));
   if (space == EALS_DEVICE) {
     const int none = 0x7fffffff;
@@ -844,26 +902,75 @@ int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k,
       return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", u, bad - 1, m->ub, m->ue);
     }
   }
-  const cudaMemcpyKind kind = space == EALS_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
-  RecStats total;
-  for (int s0 = 0; s0 < n; s0 += per) {
-    const int nc = std::min(per, n - s0);
-    const size_t nck = (size_t)nc * k;
-    RecStats c;   // stays zero for a chunk of the exact engine
-    if (use_tc_engine(m, nc)) OK(rec_tc(m, nc, ws.users.p + s0, k, exclude != 0, c));
-    if (c.engine == 0) OK(rec_exact(m, nc, ws.users.p + s0, k, exclude != 0));
-    if (s0 == 0) total = c;                              // engine, seed and the first block from chunk 0
-    else { total.pairs += c.pairs; total.left1 += c.left1; }
-    if (c.engine == 0) { total.engine = 0; total.seed = 0; }   // tcgen05 and its seed only if every chunk ran there
-    rec::rec_finish_kernel<<<4 * m->sm_count, 256, 0, m->stream>>>(ws.top_i.p, nck);
-    OK(check_launch(m));
-    CU(cudaMemcpyAsync(items + (size_t)s0 * k, ws.top_i.p, sizeof(int32_t) * nck, kind, m->stream));
-    if (scores) CU(cudaMemcpyAsync(scores + (size_t)s0 * k, ws.top_s.p, sizeof(double) * nck, kind, m->stream));
-    CU(cudaStreamSynchronize(m->stream));   // the lists are reused by the next chunk
-  }
-  m->rec_stats = total;
+  RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0};
+  if (exclude) { q.ex_ptr = m->users.ptr; q.ex_idx = m->users.idx; q.ex_base = m->users.row_base; }
+  return rec_answer(m, space, n, q, k, items, scores);
+}
+
+// ---- fold-in and top-k for arbitrary query vectors (DESIGN.md §3.6) ---------------------------------------------
+
+// A CSR of n caller rows over the items (histories, exclusion lists), validated like the train matrix and bucketed
+// into `s`.  Heavy rows may grow the shared scratch m->partials; a captured epoch graph refers to the old buffer, so
+// it is captured again at the next eals_run_epochs.
+int build_query_side(eals_model* m, Side& s, WsBuf<int>& check, int n, int space, const int64_t* ptr, const int32_t* idx,
+                     const double* val) {
+  OK(check.reserve(8));
+  const double* partials = m->partials;
+  const int rc = build_side(m, s, 0, n, m->N, space, ptr, idx, val, check.p);
+  if (m->partials != partials) m->config_gen++;
+  return rc;
+}
+
+// n_iter passes of update_user_thread (MF_fastALS.cpp:243-322) over each history row, from `init` (NULL: zeros),
+// with the model's V, SV, Wi and reg: the user CD kernels on a CdSide whose X is the workspace, no peers, no
+// prediction cache (every pass recomputes the predictions), untimed.  Nothing of the model changes.
+int fold_in_impl(eals_model* m, int space, int n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
+                 const double* init, int n_iter, double* out) {
+  if (!m || (n > 0 && (!row_ptr || !col_idx || !out))) return fail(EALS_ERR_ARG, "null argument");
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (n_iter < 1) return fail(EALS_ERR_ARG, "n_iter must be >= 1, got %d", n_iter);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  if (!m->factors_set) return fail(EALS_ERR_STATE, "factors not initialised");
+  CU(cudaSetDevice(m->p.device));
+  if (n == 0) return EALS_OK;
+  eals_eval_ws& ws = eval_ws(m);
+  OK(build_query_side(m, ws.hist, ws.hist_check, n, space, row_ptr, col_idx, val));
+  OK(ws.qx.reserve((size_t)n * m->LD));
+  if (init) OK(upload_dense(m, ws.qx.p, init, (size_t)n, space));   // padding columns written as zeros
+  else CU(cudaMemsetAsync(ws.qx.p, 0, sizeof(double) * (size_t)n * m->LD, m->stream));
+  CdSide a{};
+  a.ptr = ws.hist.ptr; a.idx = ws.hist.idx; a.val = ws.hist.val;
+  a.X = ws.qx.p; a.Y = m->V; a.S = m->SV; a.Wi = m->Wi;
+  a.row_base = 0; a.K = m->K; a.reg = m->p.reg;
+  for (int it = 0; it < n_iter; it++) DISPATCH_LD(m->LD, OK((launch_cd<LD, true>(m, ws.hist, a, -1, false))));
+  return download_dense(m, out, ws.qx.p, (size_t)n, space);
+}
+
+// Top-k of the query vectors Q[0 .. n) ([n][K]) with the same engines and contract as recommend (Q[s] stands in for
+// U[u]), the items of row s of the optional CSR ex_ptr / ex_idx left out.
+int recommend_vectors_impl(eals_model* m, int space, int n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
+                           int k, int32_t* items, double* scores) {
+  if (!m || (n > 0 && (!Q || !items))) return fail(EALS_ERR_ARG, "null argument");
+  if ((ex_ptr == nullptr) != (ex_idx == nullptr)) return fail(EALS_ERR_ARG, "ex_ptr and ex_idx must both be given or both be null");
+  OK(rec_check_args(m, space, n, k));
+  CU(cudaSetDevice(m->p.device));
+  if (n == 0) return EALS_OK;
+  eals_eval_ws& ws = eval_ws(m);
+  if (ex_ptr) OK(build_query_side(m, ws.excl, ws.excl_check, n, space, ex_ptr, ex_idx, nullptr));
+  OK(ws.qx.reserve((size_t)n * m->LD));
+  OK(upload_dense(m, ws.qx.p, Q, (size_t)n, space));
+  const int none = 0x7fffffff;
+  int bad = none;
+  CU(cudaMemcpyAsync(m->flags, &none, sizeof(int), cudaMemcpyHostToDevice, m->stream));
+  rec::rec_check_finite_kernel<<<std::min((unsigned)(((size_t)n * m->K + 255) / 256), 8u * m->sm_count), 256, 0, m->stream>>>(
+      ws.qx.p, n, m->K, m->LD, m->flags);
+  OK(check_launch(m));
+  CU(cudaMemcpyAsync(&bad, m->flags, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
   CU(cudaStreamSynchronize(m->stream));
-  return EALS_OK;
+  if (bad != none) return fail(EALS_ERR_ARG, "query row %d has a non-finite entry", bad - 1);
+  RecQuery q{ws.qx.p, nullptr, nullptr, nullptr, 0};
+  if (ex_ptr) { q.ex_ptr = ws.excl.ptr; q.ex_idx = ws.excl.idx; }
+  return rec_answer(m, space, n, q, k, items, scores);
 }
 
 }  // namespace

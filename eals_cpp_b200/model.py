@@ -214,6 +214,79 @@ def _recommend_stats(lib, h, factors):
     return st
 
 
+def _is_cuda(a) -> bool:
+    return a is not None and not isinstance(a, np.ndarray) and getattr(a, "is_cuda", False)
+
+
+def _same_space(arrays, device):
+    """The arrays of one fold_in / recommend_vectors call in ONE memory space: torch tensors on ``device`` when any of
+    them is a CUDA tensor, numpy arrays otherwise (None stays None).  ``arrays``: (array, numpy dtype) pairs.  An empty
+    array becomes a one-element one, so that the library never sees a null pointer for a present argument."""
+    on_dev = any(_is_cuda(a) for a, _ in arrays)
+    out = []
+    for a, dt in arrays:
+        if a is None:
+            out.append(None)
+            continue
+        if on_dev:
+            import torch
+            t = torch.as_tensor(a, device=device).to(torch.from_numpy(np.empty(0, dt)).dtype).contiguous()
+            out.append(t if t.numel() else torch.zeros(1, dtype=t.dtype, device=device))
+        else:
+            h = a.cpu().numpy() if hasattr(a, "cpu") else a
+            h = np.ascontiguousarray(h, dt)
+            out.append(h if h.size else np.zeros(1, dt))
+    if on_dev:
+        import torch
+        torch.cuda.current_stream(torch.device(device)).synchronize()
+    return (_lib.EALS_DEVICE if on_dev else _lib.EALS_HOST), out
+
+
+def _rows(a) -> int:
+    return int(a.shape[0])
+
+
+def _fold_in_call(fn, handle, factors, device, histories, init, n_iter):
+    """One eals_fold_in / eals_group_fold_in call; returns float64 [n, factors] on the host."""
+    n = _rows(histories.row_ptr) - 1
+    if init is not None and tuple(init.shape) != (n, factors):
+        raise ValueError(f"init must be [{n}, {factors}], got {tuple(init.shape)}")
+    space, (rp, ci, rv, ini) = _same_space([(histories.row_ptr, np.int64), (histories.col_idx, np.int32),
+                                            (histories.row_val, np.float64), (init, np.float64)], device)
+    if space == _lib.EALS_DEVICE:
+        import torch
+        out = torch.empty((max(n, 1), factors), dtype=torch.float64, device=device)
+    else:
+        out = np.empty((max(n, 1), factors), np.float64)
+    check(fn(handle, space, n, _ptr(rp), _ptr(ci), _ptr(rv), _ptr(ini), int(n_iter), _ptr(out)))
+    out = out[:n]
+    return out if isinstance(out, np.ndarray) else out.cpu().numpy()
+
+
+def _recommend_vectors_call(fn, handle, factors, device, Q, k, exclude):
+    """One eals_recommend_vectors / eals_group_recommend_vectors call; returns (items, scores) on the host."""
+    k = int(k)
+    if not hasattr(Q, "shape"):
+        Q = np.asarray(Q, np.float64)
+    n = _rows(Q)
+    if len(Q.shape) != 2 or Q.shape[1] != factors:
+        raise ValueError(f"Q must be [n, {factors}], got {tuple(Q.shape)}")
+    if exclude is not None and _rows(exclude.row_ptr) - 1 != n:
+        raise ValueError(f"exclude must have one row per query ({n}), got {_rows(exclude.row_ptr) - 1}")
+    ex = (None, None) if exclude is None else (exclude.row_ptr, exclude.col_idx)
+    space, (q, ep, ei) = _same_space([(Q, np.float64), (ex[0], np.int64), (ex[1], np.int32)], device)
+    shape = (max(n, 1), max(k, 1))
+    if space == _lib.EALS_DEVICE:
+        import torch
+        items = torch.empty(shape, dtype=torch.int32, device=device)
+        scores = torch.empty(shape, dtype=torch.float64, device=device)
+    else:
+        items, scores = np.empty(shape, np.int32), np.empty(shape, np.float64)
+    check(fn(handle, space, n, _ptr(q), _ptr(ep), _ptr(ei), k, _ptr(items), _ptr(scores)))
+    items, scores = items[:n], scores[:n]
+    return (items, scores) if isinstance(items, np.ndarray) else (items.cpu().numpy(), scores.cpu().numpy())
+
+
 class _DevArray:
     """Expose a raw device pointer to torch through __cuda_array_interface__."""
 
@@ -825,6 +898,80 @@ class MF_fastALS:
             out_s[pos] = all_scores[q * width:q * width + counts[q]]
         return out_i.cpu().numpy(), out_s.cpu().numpy()
 
+    def fold_in(self, histories: SparseMat, init=None, n_iter=10):
+        """User vectors for interaction histories, the model left as it is: ``n_iter`` passes (default 10, the
+        reference's ``maxIterOnline``) of ``update_user_thread`` over each row of ``histories`` (a SparseMat whose
+        rows are histories over this model's items; ratings are the confidence weights, None = 1), starting from
+        ``init`` ([n, factors], None = zeros), against the current V, SV, Wi and reg.  Returns float64 [n, factors].
+        Covers new users, users whose history changed since training and "what if" queries; together with
+        ``recommend_vectors(Q, k, exclude=histories)`` it recommends for a history.  Inputs may be torch CUDA
+        tensors.  With several ranks the call is collective: every rank folds in a slice of the histories and an
+        all-gather gives every rank the whole result."""
+        if self.world == 1:
+            return _fold_in_call(self.lib.eals_fold_in, self.h, self.factors, f"cuda:{self.device}", histories, init, n_iter)
+        host = lambda a: None if a is None else (a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a))
+        rp, ci, rv, ini = host(histories.row_ptr), host(histories.col_idx), host(histories.row_val), host(init)
+
+        def run(lo, hi):
+            part = SparseMat(hi - lo, histories.N, rp[lo:hi + 1], ci, None, None, rv)
+            return (_fold_in_call(self.lib.eals_fold_in, self.h, self.factors, f"cuda:{self.device}", part,
+                                  None if ini is None else ini[lo:hi], n_iter),)
+        return self._collective_slices(len(rp) - 1, run, [((self.factors,), np.float64, 0.0)])[0]
+
+    def recommend_vectors(self, Q, k, exclude: SparseMat = None):
+        """``recommend`` for arbitrary query vectors: the k items of highest score ``seq_dot(Q[s], V[i])`` for each
+        row of ``Q`` ([n, factors]; ``Q[s] == U[u]`` gives exactly ``recommend([u])``), the items of row s of
+        ``exclude`` (a SparseMat with one row per query, or None) left out.  Returns ``(items int32[n, k], scores
+        float64[n, k])``.  Inputs may be torch CUDA tensors.  With several ranks the call is collective, like
+        ``recommend``."""
+        if self.world == 1:
+            return _recommend_vectors_call(self.lib.eals_recommend_vectors, self.h, self.factors, f"cuda:{self.device}",
+                                           Q, k, exclude)
+        host = lambda a: None if a is None else (a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a))
+        q = host(Q)
+        ep, ei = (None, None) if exclude is None else (host(exclude.row_ptr), host(exclude.col_idx))
+        k = int(k)
+
+        def run(lo, hi):
+            part = None if ep is None else SparseMat(hi - lo, exclude.N, ep[lo:hi + 1], ei, None, None)
+            return _recommend_vectors_call(self.lib.eals_recommend_vectors, self.h, self.factors, f"cuda:{self.device}",
+                                           q[lo:hi], k, part)
+        return tuple(self._collective_slices(len(q), run, [((max(k, 1),), np.int32, -1),
+                                                           ((max(k, 1),), np.float64, float("-inf"))]))
+
+    def _collective_slices(self, n, run, outs):
+        """Several processes: rank r answers the queries [n*r/world, n*(r+1)/world) with run(lo, hi), one host array
+        per entry (trailing shape, dtype, pad) of ``outs``.  Every rank reports success or failure before an NCCL
+        all-gather gives every rank the whole result, so an error on one rank raises on all of them instead of
+        leaving the others in the all-gather, and no rank starts its next sweep (which stores into the other ranks'
+        V replicas) while another still reads its own."""
+        import torch
+        import torch.distributed as dist
+        dev = f"cuda:{self.device}"
+        bounds = [n * q // self.world for q in range(self.world + 1)]
+        width = max(1, max(bounds[q + 1] - bounds[q] for q in range(self.world)))
+        tdt = lambda dt: torch.from_numpy(np.empty(0, dt)).dtype
+        bufs = [torch.full((width, *shape), pad, dtype=tdt(dt), device=dev) for shape, dt, pad in outs]
+        lo, hi = bounds[self.rank], bounds[self.rank + 1]
+        err = None
+        try:
+            for b, a in zip(bufs, run(lo, hi)):
+                b[:hi - lo] = torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+        except Exception as e:
+            err = e
+        failed = torch.tensor([0 if err is None else self.rank + 1], dtype=torch.int32, device=dev)
+        dist.all_reduce(failed, op=dist.ReduceOp.MAX, group=self.group)
+        if err is not None:
+            raise err
+        if int(failed.item()):
+            raise RuntimeError(f"call failed on rank {int(failed.item()) - 1}")
+        res = []
+        for b in bufs:
+            full = torch.empty((self.world * width, *b.shape[1:]), dtype=b.dtype, device=dev)
+            dist.all_gather_into_tensor(full, b, group=self.group)
+            res.append(torch.cat([full[q * width:q * width + bounds[q + 1] - bounds[q]] for q in range(self.world)]).cpu().numpy())
+        return res
+
     def recommend_stats(self):
         """How the last recommend ran on this rank: engine ('tcgen05' or 'fp64'), exact seed size, pairs re-scored,
         users left after the first item block and that block's shape, time and tensor rate."""
@@ -1032,6 +1179,16 @@ class GroupMF_fastALS:
         """``MF_fastALS.recommend`` over all ranks: each user is answered by the rank that owns it."""
         items, scores = _recommend_call(self.lib.eals_group_recommend, self.g, users, k, exclude_seen)
         return (items.cpu().numpy(), scores.cpu().numpy()) if not isinstance(items, np.ndarray) else (items, scores)
+
+    def fold_in(self, histories: SparseMat, init=None, n_iter=10):
+        """``MF_fastALS.fold_in`` over all ranks: balanced contiguous slices of the histories, one per rank."""
+        return _fold_in_call(self.lib.eals_group_fold_in, self.g, self.factors, f"cuda:{self.devices[0]}", histories,
+                             init, n_iter)
+
+    def recommend_vectors(self, Q, k, exclude: SparseMat = None):
+        """``MF_fastALS.recommend_vectors`` over all ranks: balanced contiguous slices of the queries, one per rank."""
+        return _recommend_vectors_call(self.lib.eals_group_recommend_vectors, self.g, self.factors, f"cuda:{self.devices[0]}",
+                                       Q, k, exclude)
 
     def replicas_consistent(self) -> bool:
         ok = C.c_int32()

@@ -194,6 +194,33 @@ class MF_fastALS_T {
                                r.scores.data()), "eals_group_recommend");
     return r;
   }
+  // Fold-in: user vectors for n histories (CSR over the items: row_ptr of n + 1 offsets, ascending col_idx, ratings
+  // in val or all 1 when it is empty), n_iter passes of update_user_thread from init ([n][factors], empty: zeros)
+  // against the current model, which stays as it is.  Row-major [n][factors].
+  std::vector<double> fold_in(const std::vector<int64_t>& row_ptr, const std::vector<int32_t>& col_idx,
+                              const std::vector<double>& val = {}, const std::vector<double>& init = {}, int n_iter = 10) {
+    const int n = row_ptr.empty() ? 0 : (int)row_ptr.size() - 1;
+    std::vector<double> out((size_t)n * factors);
+    const int32_t none = 0;
+    check(eals_group_fold_in(g_, EALS_HOST, n, row_ptr.data(), col_idx.empty() ? &none : col_idx.data(),
+                             val.empty() ? nullptr : val.data(), init.empty() ? nullptr : init.data(), n_iter, out.data()),
+          "eals_group_fold_in");
+    return out;
+  }
+  // recommend() for query vectors Q ([n][factors] row-major, e.g. from fold_in), the items of row s of the CSR
+  // ex_ptr / ex_idx left out of row s's list (ex_ptr empty: no exclusion).
+  Recommendations recommend_vectors(const std::vector<double>& Q, int k, const std::vector<int64_t>& ex_ptr = {},
+                                    const std::vector<int32_t>& ex_idx = {}) {
+    const int n = (int)(Q.size() / (size_t)factors);
+    Recommendations r;
+    r.items.resize((size_t)n * (size_t)std::max(k, 0));
+    r.scores.resize(r.items.size());
+    const int32_t none = 0;
+    check(eals_group_recommend_vectors(g_, EALS_HOST, n, Q.data(), ex_ptr.empty() ? nullptr : ex_ptr.data(),
+                                       ex_ptr.empty() ? nullptr : (ex_idx.empty() ? &none : ex_idx.data()), k, r.items.data(),
+                                       r.scores.data()), "eals_group_recommend_vectors");
+    return r;
+  }
   void update_user_thread(int u) { check(eals_group_update_user_row(g_, u), "eals_group_update_user_row"); }
   void update_item_thread(int i) { check(eals_group_update_item_row(g_, i), "eals_group_update_item_row"); }
   void update_user_SU(double* oldVector, double* uget) { check(eals_group_patch_SU(g_, oldVector, uget), "eals_group_patch_SU"); }

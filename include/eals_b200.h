@@ -231,6 +231,24 @@ int eals_recommend(eals_model* m, int32_t space, int32_t n, const int32_t* users
  * block (2 * users * items * roundup(factors, 64) flop). */
 int eals_recommend_stats(eals_model* m, int64_t out[7]);
 
+/* Fold-in: the user vectors the eALS online step computes for n histories without touching the model.  row_ptr,
+ * col_idx and val are a CSR of n rows over the model's items with the rules of eals_set_train (indices in
+ * [0, n_items), strictly ascending inside a row; val NULL = every rating 1; row_ptr[0] may be non-zero).  Each row
+ * starts from init ([n][factors], NULL: zeros) and gets n_iter >= 1 passes of update_user_thread
+ * (MF_fastALS.cpp:243-322) against the model's current V, SV, Wi and reg, every pass recomputing the row's
+ * predictions; an empty row keeps its init.  out: [n][factors], dense rows.  All arrays are host or device memory
+ * as `space` says.  U, V, the S caches, Wi, the prediction-cache state and the timers stay exactly as they were.
+ * With init = U[u], n_iter = 1 and u's train row the result is U[u] after eals_update_user_row(u), bit for bit. */
+int eals_fold_in(eals_model* m, int32_t space, int32_t n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
+                 const double* init, int32_t n_iter, double* out);
+/* eals_recommend for arbitrary query vectors: Q is [n][factors] (finite, checked on the device) and row s stands in
+ * for U[u], so score = predict's seq_dot(Q[s], V[i]) — bit-identical to eals_recommend when Q[s] == U[u] — with the
+ * same order, padding, 1 <= k <= 1024, factors <= 256 and engines.  ex_ptr / ex_idx: an optional CSR of n rows of
+ * items to leave out of row s's list (both or neither; validated like a history), e.g. the history a vector was
+ * folded in from.  eals_recommend_stats reports the last eals_recommend or eals_recommend_vectors call. */
+int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
+                           int32_t k, int32_t* items, double* scores);
+
 /* Plumbing for the host layer. */
 int eals_leading_dim(const eals_model* m);                 /* ld of U/V/SU/SV rows, in doubles   */
 int eals_device_buffer(eals_model* m, int32_t which, void** dev_ptr, int64_t* bytes);
@@ -322,6 +340,12 @@ int eals_group_evaluate_user(eals_group* g, int32_t u, int32_t gt_item, int32_t 
 /* eals_recommend over the whole user range: each user is answered by the rank that owns it, results in input order. */
 int eals_group_recommend(eals_group* g, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
                          int32_t* items, double* scores);
+/* eals_fold_in / eals_recommend_vectors over the group: the queries go to the ranks in balanced contiguous slices
+ * (V, SV and Wi are replicated), results in input order. */
+int eals_group_fold_in(eals_group* g, int32_t space, int32_t n, const int64_t* row_ptr, const int32_t* col_idx,
+                       const double* val, const double* init, int32_t n_iter, double* out);
+int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr,
+                                 const int32_t* ex_idx, int32_t k, int32_t* items, double* scores);
 int eals_group_sync(eals_group* g);
 int eals_group_replicas_consistent(eals_group* g, int32_t* ok);             /* all U / V replicas bit-identical */
 int eals_group_save_factors(eals_group* g, const char* path);
