@@ -14,6 +14,7 @@ LIB_PATH = os.path.join(HERE, "lib", "libeals_b200.so")
 EALS_HOST, EALS_DEVICE = 0, 1
 BUF_U, BUF_V, BUF_SU, BUF_SV, BUF_WI, BUF_LOSS_TERMS, BUF_PC_USER, BUF_PC_ITEM = range(8)
 EVAL_REFERENCE, EVAL_EXACT = 0, 1
+ERR_ARG = -1
 FLAG_SYNC_EACH_CALL = 1
 
 
@@ -80,6 +81,7 @@ SIGNATURES = {
     "eals_recommend_stats": (C.c_int, [_P, _P]),
     "eals_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "eals_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    "eals_ranking_metrics": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "eals_leading_dim": (C.c_int, [_P]),
     "eals_device_buffer": (C.c_int, [_P, C.c_int32, C.POINTER(_P), C.POINTER(C.c_int64)]),
     "eals_stream": (C.c_int, [_P, C.POINTER(_P)]),
@@ -123,6 +125,7 @@ SIGNATURES = {
     "eals_group_recommend": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
     "eals_group_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "eals_group_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    "eals_group_ranking_metrics": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "eals_group_sync": (C.c_int, [_P]),
     "eals_group_replicas_consistent": (C.c_int, [_P, C.POINTER(C.c_int32)]),
     "eals_group_save_factors": (C.c_int, [_P, C.c_char_p]),

@@ -38,6 +38,7 @@
 #include "eval_tc.cuh"
 #include "gram.cuh"
 #include "loss.cuh"
+#include "ranking.cuh"
 #include "recommend.cuh"
 
 namespace {
@@ -2035,6 +2036,11 @@ int eals_fold_in(eals_model* m, int32_t space, int32_t n, const int64_t* row_ptr
 int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
                            int32_t k, int32_t* items, double* scores) {
   return recommend_vectors_impl(m, space, n, Q, ex_ptr, ex_idx, k, items, scores);
+}
+
+int eals_ranking_metrics(eals_model* m, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
+                         int32_t exclude_seen, double sums[6], int64_t* n_users, double* per_user, int32_t* ranks) {
+  return ranking_metrics_impl(m, space, test_ptr, test_idx, k, exclude_seen, sums, n_users, per_user, ranks);
 }
 
 int eals_recommend_stats(eals_model* m, int64_t out[7]) {

@@ -589,6 +589,38 @@ int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const 
   return EALS_OK;
 }
 
+// Every rank ranks the test entries of the rows it owns (its train rows are the ones to exclude), the ranks at once;
+// the sums are added in rank order.
+int eals_group_ranking_metrics(eals_group* g, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
+                               int32_t exclude_seen, double means[6], int64_t* n_users, double* per_user, int32_t* ranks) {
+  if (!g || !test_ptr || !test_idx || !means || !n_users) return fail(EALS_ERR_ARG, "null argument");
+  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(group_barrier(g));
+  const int M = g->base.n_users;
+  HostCsr t;
+  OK(t.load(space, M, test_ptr, test_idx, nullptr));
+  std::vector<double> sums((size_t)6 * g->n, 0.0), pu(per_user ? (size_t)M * 6 : 0);
+  std::vector<int64_t> cnt((size_t)g->n, 0);
+  std::vector<int32_t> rk(ranks ? (size_t)t.ptr[(size_t)M] : 0);
+  OK(parallel_ranks(g, [&](int q) {
+    const int b = g->ub[q];
+    return eals_ranking_metrics(g->r[q], EALS_HOST, t.ptr.data(), t.idx.data(), k, exclude_seen, &sums[(size_t)6 * q], &cnt[(size_t)q],
+                                per_user ? pu.data() + (size_t)b * 6 : nullptr, ranks ? rk.data() + t.ptr[(size_t)b] : nullptr);
+  }));
+  int64_t users = 0;
+  for (int q = 0; q < g->n; q++) users += cnt[(size_t)q];
+  for (int j = 0; j < 6; j++) {
+    double s = 0;
+    for (int q = 0; q < g->n; q++) s += sums[(size_t)6 * q + j];
+    means[j] = users > 0 ? s / (double)users : 0.0;
+  }
+  *n_users = users;
+  if (per_user) OK(host_result(space, per_user, pu));
+  if (ranks && !rk.empty()) OK(host_result(space, ranks, rk));
+  return EALS_OK;
+}
+
 int eals_group_evaluate_user(eals_group* g, int32_t u, int32_t gt_item, int32_t topk, int32_t mode, double out[3]) {
   if (!g) return fail(EALS_ERR_ARG, "null group");
   OK(group_barrier(g));

@@ -141,8 +141,15 @@ struct eals_eval_ws {
   Side hist, excl;
   WsBuf<int> hist_check, excl_check;
   WsBuf<double> qx;
+  // ranking metrics: the owned rows of the test matrix (validated by build_side, row_base = the first owned user),
+  // per entry its rank, per slot c_R and the certain-count limit, the chunk's train scores, the per-user metrics
+  // and the gain / ideal-DCG tables
+  Side test;
+  WsBuf<int> test_check;
+  WsBuf<int32_t> ranks, c_r, lim;
+  WsBuf<double> tscore, rm_out, rm_tab;
   eals_eval_ws() = default;
-  ~eals_eval_ws() { free_side(hist); free_side(excl); }
+  ~eals_eval_ws() { free_side(hist); free_side(excl); free_side(test); }
 };
 
 namespace {
@@ -388,24 +395,19 @@ int select_flagged(eals_model* m, const int32_t* in, int n, int32_t* out, int32_
 // Preparation of the tcgen05 filter for the rows X[d_rows[0 .. n)] (d_rows nullable: X[0 .. n); evaluate and
 // recommend): fp16 copies of V in decreasing-norm order (ws.perm: rank -> item) and of the query rows, their norms,
 // the per-tile item norms and the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).
-int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
+// The item half (once per call of ranking_metrics, which prepares several chunks of rows against it) ...
+int tc_prepare_items(eals_model* m) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
   const int K = m->K, LD = m->LD, N = m->N;
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
   cudaStream_t st = m->stream;
-  // ---- preparation: fp16 copies, norms, item order, per-slot thresholds ----
+  // ---- preparation: fp16 copies, norms, item order ----
   OK(ws.counters.reserve(4));
   OK(ws.keys.reserve((size_t)N)); OK(ws.keys_out.reserve((size_t)N)); OK(ws.ids.reserve((size_t)N)); OK(ws.perm.reserve((size_t)N));
   OK(ws.Vh.reserve((size_t)N * KP)); OK(ws.vn_hat.reserve((size_t)N)); OK(ws.vn_del.reserve((size_t)N)); OK(ws.vn_h.reserve((size_t)N));
   OK(ws.tile_norm.reserve((size_t)n_tiles));
-  OK(ws.Uh.reserve((size_t)n * KP)); OK(ws.W.reserve(((size_t)n + 2 * tc::kTM) * KP));
-  OK(ws.un_hat.reserve((size_t)n)); OK(ws.un_del.reserve((size_t)n)); OK(ws.un_h.reserve((size_t)n)); OK(ws.exps.reserve((size_t)n));
-  OK(ws.sp0.reserve((size_t)n)); OK(ws.sp1.reserve((size_t)n));
-  OK(ws.cnt.reserve((size_t)n)); OK(ws.cnt_exact.reserve((size_t)n));
-  OK(ws.list_a.reserve((size_t)n)); OK(ws.list_b.reserve((size_t)n)); OK(ws.flags.reserve((size_t)n));
-  OK(ws.scalars.reserve(8));
   unsigned long long* d_vmax = ws.counters.p;
   CU(cudaMemsetAsync(ws.counters.p, 0, 4 * sizeof(unsigned long long), st));
   tc::absmax_kernel<<<4 * m->sm_count, 256, 0, st>>>(m->V, (size_t)N, K, LD, d_vmax);
@@ -421,6 +423,23 @@ int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, con
     tc::tile_norm_kernel<<<n_tiles, 32, 0, st>>>(ws.vn_h.p, ws.vn_del.p, N, n_tiles, ws.tile_norm.p);
     OK(check_launch(m));
   }
+  return EALS_OK;
+}
+
+// ... and the row half: fp16 copies of X[d_rows[0 .. n)], their norms and the per-slot thresholds.
+int tc_prepare_rows(eals_model* m, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
+  namespace tc = eals::tc;
+  eals_eval_ws& ws = eval_ws(m);
+  const int K = m->K, LD = m->LD;
+  const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
+  cudaStream_t st = m->stream;
+  OK(ws.Uh.reserve((size_t)n * KP)); OK(ws.W.reserve(((size_t)n + 2 * tc::kTM) * KP));
+  OK(ws.un_hat.reserve((size_t)n)); OK(ws.un_del.reserve((size_t)n)); OK(ws.un_h.reserve((size_t)n)); OK(ws.exps.reserve((size_t)n));
+  OK(ws.sp0.reserve((size_t)n)); OK(ws.sp1.reserve((size_t)n));
+  OK(ws.cnt.reserve((size_t)n)); OK(ws.cnt_exact.reserve((size_t)n));
+  OK(ws.list_a.reserve((size_t)n)); OK(ws.list_b.reserve((size_t)n)); OK(ws.flags.reserve((size_t)n));
+  OK(ws.scalars.reserve(8));
+  const unsigned long long* d_vmax = ws.counters.p;   // max |V|, from tc_prepare_items
   {
     tc::PrepOut o{ws.Uh.p, ws.un_hat.p, ws.un_del.p, ws.un_h.p, ws.exps.p};
     tc::prep_rows_kernel<true><<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st>>>(X, K, LD, KP, n, d_rows, 0, d_vmax, o);
@@ -430,6 +449,11 @@ int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, con
     OK(check_launch(m));
   }
   return EALS_OK;
+}
+
+int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
+  OK(tc_prepare_items(m));
+  return tc_prepare_rows(m, n, X, d_rows, d_thr);
 }
 
 // Fills `out` and m->eval_stats (engine 1), or returns with neither touched when the pair list overflows.
@@ -913,10 +937,10 @@ int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k,
 // into `s`.  Heavy rows may grow the shared scratch m->partials; a captured epoch graph refers to the old buffer, so
 // it is captured again at the next eals_run_epochs.
 int build_query_side(eals_model* m, Side& s, WsBuf<int>& check, int n, int space, const int64_t* ptr, const int32_t* idx,
-                     const double* val) {
+                     const double* val, int begin = 0) {   // rows begin .. begin + n of ptr
   OK(check.reserve(8));
   const double* partials = m->partials;
-  const int rc = build_side(m, s, 0, n, m->N, space, ptr, idx, val, check.p);
+  const int rc = build_side(m, s, begin, begin + n, m->N, space, ptr, idx, val, check.p);
   if (m->partials != partials) m->config_gen++;
   return rc;
 }
@@ -971,6 +995,236 @@ int recommend_vectors_impl(eals_model* m, int space, int n, const double* Q, con
   RecQuery q{ws.qx.p, nullptr, nullptr, nullptr, 0};
   if (ex_ptr) { q.ex_ptr = ws.excl.ptr; q.ex_idx = ws.excl.idx; }
   return rec_answer(m, space, n, q, k, items, scores);
+}
+
+
+// ---- ranking metrics on a held-out test matrix (ranking.cuh, DESIGN.md §3.7) ------------------------------------
+namespace rk = eals::rk;
+
+// The device bytes a chunk of test entries may use (the entries' fp16 rows and working lists, the train scores):
+// recommend's list budget, EALS_REC_LIST_BYTES (default 4 GiB).
+size_t rm_chunk_bytes() {
+  size_t bytes = (size_t)4 << 30;
+  if (const char* e = getenv("EALS_REC_LIST_BYTES")) bytes = std::max<size_t>(1, strtoull(e, nullptr, 10));
+  return bytes;
+}
+
+// Engine 2 for the test entries of the owned rows [r0, r1) (n entries from e0 on, slot s = entry e0 + s): ranks of the
+// slots into d_ranks[0 .. n).  Fills `st` and sets `done` when it answers; leaves both as they are when the
+// candidate list overflows (the filter is not filtering: the exact engine answers instead).
+int rm_chunk_tc(eals_model* m, int r0, int r1, int k, bool exclude, bool timed, int32_t* d_ranks, EvalStats& st, bool& done) {
+  namespace tc = eals::tc;
+  eals_eval_ws& ws = eval_ws(m);
+  const Side &T = ws.test, &R = m->users;
+  const int K = m->K, LD = m->LD, N = m->N;
+  const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
+  const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
+  const int64_t e0 = T.h_ptr[(size_t)r0];
+  const int n = (int)(T.h_ptr[(size_t)r1] - e0);
+  cudaStream_t st_ = m->stream;
+  StageTimer tm;
+  // ---- slots: user, item, exact score of (u, g); train correction c_R and the certain-count limit ----
+  OK(ws.users.reserve((size_t)n)); OK(ws.gt.reserve((size_t)n)); OK(ws.gts.reserve((size_t)n));
+  OK(ws.c_r.reserve((size_t)n)); OK(ws.lim.reserve((size_t)n));
+  rk::rm_entry_kernel<<<(n + 255) / 256, 256, 0, st_>>>(T.ptr, T.idx, r0, r1, m->ub, e0, n, ws.users.p, ws.gt.p);
+  OK(check_launch(m));
+  eals::eval_gt_score_kernel<<<(n + 127) / 128, 128, 0, st_>>>(m->U, m->V, ws.gt.p, ws.users.p, 0, n, K, LD, ws.gts.p);
+  OK(check_launch(m));
+  const int64_t z0 = R.h_ptr[(size_t)r0], nz = R.h_ptr[(size_t)r1] - z0;
+  if (exclude && nz > 0) {   // every train nonzero of these users scored once; the entries then only compare
+    OK(ws.tscore.reserve((size_t)nz));
+    rk::rm_train_score_kernel<<<16 * m->sm_count, 128, 0, st_>>>(m->U, m->V, K, LD, R.ptr, R.idx, T.ptr, r0, r1, m->ub, z0, nz, ws.tscore.p);
+    OK(check_launch(m));
+  }
+  rk::rm_train_count_kernel<<<(unsigned)(((size_t)n * 32 + 255) / 256), 256, 0, st_>>>(exclude ? R.ptr : nullptr, R.idx, ws.tscore.p, z0,
+                                                                                       m->ub, ws.users.p, ws.gt.p, ws.gts.p, n, k,
+                                                                                       ws.c_r.p, ws.lim.p);
+  OK(check_launch(m));
+  OK(tc_prepare_rows(m, n, m->U, ws.users.p, ws.gts.p));
+  CU(cudaMemsetAsync(ws.cnt.p, 0, sizeof(int32_t) * n, st_));
+  CU(cudaMemsetAsync(ws.cnt_exact.p, 0, sizeof(int32_t) * n, st_));
+  CUtensorMap mapV, mapU0, mapW;
+  OK(make_half_map(&mapV, ws.Vh.p, (size_t)N, KP));
+  OK(make_half_map(&mapU0, ws.Uh.p, (size_t)n, KP));
+  OK(make_half_map(&mapW, ws.W.p, (size_t)n + 2 * tc::kTM, KP));
+  int32_t* d_n = ws.scalars.p;          // [0]: size of the current working list, [1]: next
+  set_i32_kernel<<<1, 1, 0, st_>>>(d_n, n);
+  OK(check_launch(m));
+  tm.lap("ranking: slots, train correction, fp16 rows");
+
+  // ---- MODE 0 over the item blocks; a slot leaves once its certain count reaches k + c_R ----
+  tc::TcArgs a{};
+  a.sp0 = ws.sp0.p; a.sp1 = ws.sp1.p; a.tile_norm = ws.tile_norm.p; a.n_items = N; a.cnt_hi = ws.cnt.p; a.perm = ws.perm.p;
+  const int32_t* list = nullptr;        // identity
+  int32_t *list_next = ws.list_a.p, *list_other = ws.list_b.p;
+  auto compact = [&](void) -> int {     // slots of the current list still below their limit -> list_next, rows -> W
+    rk::rm_keep_flags_kernel<<<(n + 255) / 256, 256, 0, st_>>>(list, d_n, n, ws.cnt.p, ws.lim.p, ws.flags.p);
+    OK(check_launch(m));
+    OK(select_flagged(m, list, n, list_next, d_n + 1));
+    CU(cudaMemcpyAsync(d_n, d_n + 1, sizeof(int32_t), cudaMemcpyDeviceToDevice, st_));
+    tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, st_>>>(ws.Uh.p, KP, list_next, d_n, ws.W.p);
+    OK(check_launch(m));
+    list = list_next;
+    std::swap(list_next, list_other);
+    return EALS_OK;
+  };
+  if (exclude) OK(compact());           // test items that are in the train row (limit 0) never enter the filter
+  for (ItemBlocks blk(N, 0); blk.i0 < N; blk.next()) {
+    a.act = list; a.n_act = d_n; a.it0 = blk.it0; a.it1 = blk.it1;
+    const bool first_block = timed && blk.i0 == 0;
+    if (first_block) OK(ws.blk0.start(st_));
+    OK(launch_filter_k<0>(m, nkc, list ? mapW : mapU0, mapV, a));
+    if (first_block) OK(ws.blk0.stop(st_, n, std::min<int64_t>(N, (int64_t)a.it1 * tc::kTN)));
+    OK(compact());
+  }
+  tm.lap("ranking: certain count (MODE 0)");
+  // ---- MODE 2 for the survivors (every item not certainly below s_g), exact tie-aware count ----
+  int n_cand = 0;
+  CU(cudaMemcpyAsync(&n_cand, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st_));
+  CU(cudaStreamSynchronize(st_));
+  unsigned long long got = 0;
+  unsigned long long* d_np = ws.counters.p + 1;
+  if (n_cand > 0) {
+    unsigned long long cap = std::min<unsigned long long>(1ull << 27, std::max<unsigned long long>(1ull << 20, 2048ull * (unsigned long long)n_cand));
+    unsigned long long hard_cap = 1ull << 30;
+    read_pair_caps(cap, hard_cap, ~0ull);
+    cap = std::min(cap, hard_cap);
+    for (int attempt = 0; attempt < 2; attempt++) {
+      OK(ws.pairs.reserve((size_t)cap));
+      CU(cudaMemsetAsync(d_np, 0, sizeof(unsigned long long), st_));
+      a.act = list; a.n_act = d_n; a.it0 = 0; a.it1 = n_tiles;
+      a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
+      OK(launch_filter_k<2>(m, nkc, mapW, mapV, a));
+      CU(cudaMemcpyAsync(&got, d_np, sizeof(got), cudaMemcpyDeviceToHost, st_));
+      CU(cudaStreamSynchronize(st_));
+      if (got <= cap) break;
+      if (attempt == 1 || got > hard_cap) return EALS_OK;   // degenerate scores: exact engine instead
+      cap = got;
+    }
+    if (got) {
+      rk::rm_rescore_kernel<<<16 * m->sm_count, 128, 0, st_>>>(m->U, m->V, K, LD, ws.users.p, ws.gt.p, ws.gts.p, ws.pairs.p, got, ws.cnt_exact.p);
+      OK(check_launch(m));
+    }
+  }
+  rk::rm_rank_kernel<<<(n + 255) / 256, 256, 0, st_>>>(n, ws.cnt.p, ws.lim.p, ws.cnt_exact.p, ws.c_r.p, k, d_ranks);
+  OK(check_launch(m));
+  CU(cudaStreamSynchronize(st_));
+  tm.lap("ranking: candidates (MODE 2) + exact re-score");
+  if (timed) OK(ws.blk0.read(st.blk0));
+  st.engine = 1; st.candidates += n_cand; st.pairs += (long long)got;
+  done = true;
+  return EALS_OK;
+}
+
+// Engine 1 for the owned rows [r0, r1): recommend's exact engine (rec_exact) for the users with test entries, a
+// list budget's worth at a time, and each test item looked up in its user's list.  d_ranks: every owned entry, -1
+// where no list reaches.
+int rm_chunk_exact(eals_model* m, int r0, int r1, int k, bool exclude, int32_t* d_ranks) {
+  eals_eval_ws& ws = eval_ws(m);
+  const Side& T = ws.test;
+  std::vector<int32_t> users;
+  for (int r = r0; r < r1; r++)
+    if (T.h_ptr[(size_t)r + 1] > T.h_ptr[(size_t)r]) users.push_back(m->ub + r);
+  const int n = (int)users.size();
+  const int per = (int)std::min<size_t>((size_t)std::max(n, 1), std::max<size_t>(1, rm_chunk_bytes() / (12 * (size_t)k)));
+  for (int d0 = 0; d0 < n; d0 += per) {
+    const int nd = std::min(per, n - d0);
+    OK(ws.users.reserve((size_t)nd));
+    OK(ws.top_s.reserve((size_t)nd * k)); OK(ws.top_i.reserve((size_t)nd * k)); OK(ws.thr.reserve((size_t)nd));
+    CU(cudaMemcpyAsync(ws.users.p, users.data() + d0, sizeof(int32_t) * nd, cudaMemcpyHostToDevice, m->stream));
+    RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0};
+    if (exclude) { q.ex_ptr = m->users.ptr; q.ex_idx = m->users.idx; q.ex_base = m->users.row_base; }
+    OK(rec_exact(m, nd, q, k));
+    rk::rm_lookup_kernel<<<(unsigned)(((size_t)nd * k + 255) / 256), 256, 0, m->stream>>>(ws.top_i.p, k, nd, ws.users.p, m->ub, T.ptr,
+                                                                                          T.idx, d_ranks);
+    OK(check_launch(m));
+    CU(cudaStreamSynchronize(m->stream));   // the users' host slice and the lists are reused by the next piece
+  }
+  return EALS_OK;
+}
+
+// Ranks and metrics at k of the owned rows of the test CSR (M rows, train-matrix rules), DESIGN.md §3.7.
+int ranking_metrics_impl(eals_model* m, int space, const int64_t* test_ptr, const int32_t* test_idx, int k, int exclude_seen,
+                         double sums[6], int64_t* n_users, double* per_user, int32_t* ranks) {
+  if (!m || !test_ptr || !test_idx || !sums || !n_users) return fail(EALS_ERR_ARG, "null argument");
+  OK(rec_check_args(m, space, 0, k));
+  CU(cudaSetDevice(m->p.device));
+  eals_eval_ws& ws = eval_ws(m);
+  const int n_rows = m->ue - m->ub;
+  const bool exclude = exclude_seen != 0;
+  OK(build_query_side(m, ws.test, ws.test_check, n_rows, space, test_ptr, test_idx, nullptr, m->ub));
+  const Side &T = ws.test, &R = m->users;
+  const int64_t n_ent = T.nnz;
+  OK(ws.ranks.reserve((size_t)std::max<int64_t>(n_ent, 1)));
+  CU(cudaMemsetAsync(ws.ranks.p, 0xff, sizeof(int32_t) * (size_t)std::max<int64_t>(n_ent, 1), m->stream));   // -1
+  m->eval_stats = EvalStats{};
+  // ---- ranks, chunk by chunk of whole rows within the device budget ----
+  const int KP = (m->K + eals::tc::kKC - 1) / eals::tc::kKC * eals::tc::kKC;
+  const size_t budget = rm_chunk_bytes();
+  const size_t per_entry = 4 * (size_t)KP + 128, per_nz = exclude ? 8 : 0;
+  EvalStats total;
+  bool any = false, all_tc = true, items_ready = false;
+  for (int r0 = 0; r0 < n_rows;) {
+    int r1 = r0;
+    size_t cost = 0;
+    while (r1 < n_rows) {
+      const int64_t ne = T.h_ptr[(size_t)r1 + 1] - T.h_ptr[(size_t)r1], nz = R.h_ptr[(size_t)r1 + 1] - R.h_ptr[(size_t)r1];
+      const size_t c = (size_t)ne * per_entry + (size_t)nz * per_nz;
+      if (r1 > r0 && (cost + c > budget || T.h_ptr[(size_t)r1 + 1] - T.h_ptr[(size_t)r0] > (1 << 28))) break;
+      cost += c;
+      r1++;
+    }
+    const int64_t e0 = T.h_ptr[(size_t)r0];
+    const int64_t n = T.h_ptr[(size_t)r1] - e0;
+    if (n > 0) {
+      EvalStats c;
+      bool done = false;
+      if (use_tc_engine(m, (int)n)) {   // n <= max(2^28, one row of at most N items)
+        if (!items_ready) OK(tc_prepare_items(m));
+        items_ready = true;
+        OK(rm_chunk_tc(m, r0, r1, k, exclude, !any, ws.ranks.p + e0, c, done));
+      }
+      if (!done) { OK(rm_chunk_exact(m, r0, r1, k, exclude, ws.ranks.p)); all_tc = false; }
+      if (!any) total.blk0 = c.blk0;   // the first block of the first chunk
+      total.candidates += c.candidates; total.pairs += c.pairs;
+      any = true;
+    }
+    r0 = r1;
+  }
+  total.engine = any && all_tc ? 1 : 0;
+  m->eval_stats = total;
+  // ---- per-user metrics on the device, sums on the host in user order ----
+  std::vector<double> pu((size_t)n_rows * rk::kMetrics);
+  if (n_rows > 0) {
+    std::vector<double> tab(2 * (size_t)k + 1);   // gain[0 .. k), idcg[0 .. k]
+    double acc = 0.0;
+    tab[(size_t)k] = 0.0;
+    for (int j = 0; j < k; j++) {
+      tab[(size_t)j] = metric_ndcg(j);
+      acc += tab[(size_t)j];
+      tab[(size_t)k + 1 + j] = acc;
+    }
+    OK(ws.rm_tab.reserve(tab.size())); OK(ws.rm_out.reserve(pu.size()));
+    CU(cudaMemcpyAsync(ws.rm_tab.p, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, m->stream));
+    rk::rm_metrics_kernel<<<(unsigned)(((size_t)n_rows * 32 + 127) / 128), 128, 0, m->stream>>>(T.ptr, n_rows, ws.ranks.p, k, ws.rm_tab.p,
+                                                                                                 ws.rm_tab.p + k, ws.rm_out.p);
+    OK(check_launch(m));
+    CU(cudaMemcpyAsync(pu.data(), ws.rm_out.p, sizeof(double) * pu.size(), cudaMemcpyDeviceToHost, m->stream));
+    CU(cudaStreamSynchronize(m->stream));
+  }
+  for (int j = 0; j < rk::kMetrics; j++) sums[j] = 0.0;
+  int64_t users = 0;
+  for (int r = 0; r < n_rows; r++) {
+    if (T.h_ptr[(size_t)r + 1] == T.h_ptr[(size_t)r]) continue;
+    users++;
+    for (int j = 0; j < rk::kMetrics; j++) sums[j] += pu[(size_t)r * rk::kMetrics + j];
+  }
+  *n_users = users;
+  const cudaMemcpyKind kind = space == EALS_DEVICE ? cudaMemcpyHostToDevice : cudaMemcpyHostToHost;
+  if (per_user && n_rows > 0) CU(cudaMemcpy(per_user, pu.data(), sizeof(double) * pu.size(), kind));
+  if (ranks && n_ent > 0)
+    CU(cudaMemcpy(ranks, ws.ranks.p, sizeof(int32_t) * (size_t)n_ent, space == EALS_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost));
+  return EALS_OK;
 }
 
 }  // namespace

@@ -287,6 +287,43 @@ def _recommend_vectors_call(fn, handle, factors, device, Q, k, exclude):
     return (items, scores) if isinstance(items, np.ndarray) else (items.cpu().numpy(), scores.cpu().numpy())
 
 
+RANKING_METRICS = ("hit_rate", "precision", "recall", "ndcg", "map", "mrr")
+
+
+def _ranking_metrics_call(fn, handle, device, test, n_users, k, exclude_seen, rows, per_user, ranks):
+    """One eals_ranking_metrics / eals_group_ranking_metrics call over ``rows`` = (first, end) user rows of ``test``
+    (the rows the call reads).  Returns (sums or means [6], users with test items, per-user [end - first, 6] or None,
+    ranks of the rows' test entries or None), the arrays on the host."""
+    if _rows(test.row_ptr) - 1 != n_users:
+        raise _lib.EalsError(_lib.ERR_ARG, f"the test matrix must have one row per user ({n_users}), got "
+                                           f"{_rows(test.row_ptr) - 1}")
+    space, (rp, ci) = _same_space([(test.row_ptr, np.int64), (test.col_idx, np.int32)], device)
+    first, end = rows
+    n_rows, n_ent = end - first, int(rp[end]) - int(rp[first])
+    if space == _lib.EALS_DEVICE:
+        import torch
+        pu = torch.zeros((max(n_rows, 1), 6), dtype=torch.float64, device=device) if per_user else None
+        rk = torch.full((max(n_ent, 1),), -1, dtype=torch.int32, device=device) if ranks else None
+    else:
+        pu = np.zeros((max(n_rows, 1), 6)) if per_user else None
+        rk = np.full(max(n_ent, 1), -1, np.int32) if ranks else None
+    sums, users = np.zeros(6), C.c_int64()
+    check(fn(handle, space, _ptr(rp), _ptr(ci), int(k), int(bool(exclude_seen)), _ptr(sums), C.byref(users), _ptr(pu), _ptr(rk)))
+    host = lambda a: None if a is None else (a if isinstance(a, np.ndarray) else a.cpu().numpy())
+    pu, rk = host(pu), host(rk)
+    return sums, int(users.value), None if pu is None else pu[:n_rows], None if rk is None else rk[:n_ent]
+
+
+def _ranking_result(means, users, per_user, ranks):
+    out = dict(zip(RANKING_METRICS, (float(x) for x in means)))
+    out["users"] = int(users)
+    if per_user is not None:
+        out["per_user"] = per_user
+    if ranks is not None:
+        out["ranks"] = ranks
+    return out
+
+
 class _DevArray:
     """Expose a raw device pointer to torch through __cuda_array_interface__."""
 
@@ -832,8 +869,9 @@ class MF_fastALS:
         return v.value
 
     def eval_stats(self):
-        """Engine of the last evaluate(): 'tcgen05' (fp16 tensor-core filter + exact fp64 re-score of the close
-        calls) or 'fp64' (exact tile scan), the number of candidate users and of re-scored pairs."""
+        """Engine of the last evaluate() or ranking_metrics(): 'tcgen05' (fp16 tensor-core filter + exact fp64 re-score
+        of the close calls) or 'fp64' (exact engine), the number of candidates (users, or test entries) and of
+        re-scored pairs, and the first filtered item block's shape, time and tensor rate."""
         out = np.zeros(6, np.int64)
         check(self.lib.eals_eval_stats(self.h, _ptr(out)))
         st = {"engine": "tcgen05" if out[0] == 1 else "fp64", "candidates": int(out[1]), "pairs_rescored": int(out[2])}
@@ -938,6 +976,64 @@ class MF_fastALS:
                                            q[lo:hi], k, part)
         return tuple(self._collective_slices(len(q), run, [((max(k, 1),), np.int32, -1),
                                                            ((max(k, 1),), np.float64, float("-inf"))]))
+
+    def ranking_metrics(self, test: SparseMat, k, exclude_seen=True, per_user=False, ranks=False):
+        """Ranking metrics at k on a held-out test matrix ``test`` (a SparseMat with one row per user over this model's
+        items; only its CSR is read).  For a test entry (u, g) the rank is g's 0-based position in
+        ``recommend([u], k, exclude_seen)[0]``, or -1 (with ``exclude_seen`` a test item in u's train row is always
+        -1 and still counts in u's test items).  Returns a dict of the means over the users with test items of
+        ``hit_rate``, ``precision`` (hits / k), ``recall`` (hits / n_u), ``ndcg``, ``map`` and ``mrr``, plus ``users``
+        (their number); ``per_user=True`` adds ``per_user`` (float64 [userCount, 6] in that order, 0 for users without
+        test items), ``ranks=True`` adds ``ranks`` (int32, one per test entry in CSR order).  The model is not touched.
+        Inputs may be torch CUDA tensors.  With several ranks the call is collective: every rank ranks the rows it
+        owns, every rank reports success or failure, then the sums are added in rank order and the arrays gathered."""
+        dev = f"cuda:{self.device}"
+        if self.world == 1:
+            sums, users, pu, rk = _ranking_metrics_call(self.lib.eals_ranking_metrics, self.h, dev, test, self.userCount, k,
+                                                        exclude_seen, (0, self.userCount), per_user, ranks)
+            return _ranking_result(sums / users if users else sums * 0.0, users, pu, rk)
+        import torch
+        import torch.distributed as dist
+        ub, ue = self.user_bounds[self.rank], self.user_bounds[self.rank + 1]
+        err, sums, users, pu, rk = None, np.zeros(6), 0, None, None
+        try:
+            sums, users, pu, rk = _ranking_metrics_call(self.lib.eals_ranking_metrics, self.h, dev, test, self.userCount, k,
+                                                        exclude_seen, (ub, ue), per_user, ranks)
+        except Exception as e:
+            err = e
+        failed = torch.tensor([0 if err is None else self.rank + 1], dtype=torch.int32, device=dev)
+        dist.all_reduce(failed, op=dist.ReduceOp.MAX, group=self.group)
+        if err is not None:
+            raise err
+        if int(failed.item()):
+            raise RuntimeError(f"ranking_metrics failed on rank {int(failed.item()) - 1}")
+        part = torch.tensor([*sums.tolist(), float(users)], dtype=torch.float64, device=dev)
+        every = torch.empty(self.world * 7, dtype=torch.float64, device=dev)
+        dist.all_gather_into_tensor(every, part, group=self.group)
+        every = every.cpu().numpy().reshape(self.world, 7)
+        tot, n = np.zeros(6), 0
+        for q in range(self.world):          # rank order: the same sums on every rank
+            tot += every[q, :6]
+            n += int(every[q, 6])
+        rp = test.row_ptr.cpu().numpy() if hasattr(test.row_ptr, "cpu") else np.asarray(test.row_ptr)
+        if per_user:
+            pu = self._gather_parts(pu, [self.user_bounds[q + 1] - self.user_bounds[q] for q in range(self.world)])
+        if ranks:
+            b = self.user_bounds
+            rk = self._gather_parts(rk, [int(rp[b[q + 1]]) - int(rp[b[q]]) for q in range(self.world)])
+        return _ranking_result(tot / n if n else tot, n, pu, rk)
+
+    def _gather_parts(self, a, counts):
+        """Every rank's host array ``a`` (counts[rank] leading rows) concatenated in rank order, on every rank."""
+        import torch
+        import torch.distributed as dist
+        dev = f"cuda:{self.device}"
+        width = max(1, max(counts))
+        buf = torch.zeros((width, *a.shape[1:]), dtype=torch.from_numpy(a[:0]).dtype, device=dev)
+        buf[:len(a)] = torch.from_numpy(np.ascontiguousarray(a)).to(dev)
+        full = torch.empty((self.world * width, *a.shape[1:]), dtype=buf.dtype, device=dev)
+        dist.all_gather_into_tensor(full, buf, group=self.group)
+        return torch.cat([full[q * width:q * width + counts[q]] for q in range(self.world)]).cpu().numpy()
 
     def _collective_slices(self, n, run, outs):
         """Several processes: rank r answers the queries [n*r/world, n*(r+1)/world) with run(lo, hi), one host array
@@ -1189,6 +1285,12 @@ class GroupMF_fastALS:
         """``MF_fastALS.recommend_vectors`` over all ranks: balanced contiguous slices of the queries, one per rank."""
         return _recommend_vectors_call(self.lib.eals_group_recommend_vectors, self.g, self.factors, f"cuda:{self.devices[0]}",
                                        Q, k, exclude)
+
+    def ranking_metrics(self, test: SparseMat, k, exclude_seen=True, per_user=False, ranks=False):
+        """``MF_fastALS.ranking_metrics`` over all ranks: each rank ranks the test rows it owns, sums in rank order."""
+        means, users, pu, rk = _ranking_metrics_call(self.lib.eals_group_ranking_metrics, self.g, f"cuda:{self.devices[0]}", test,
+                                                     self.userCount, k, exclude_seen, (0, self.userCount), per_user, ranks)
+        return _ranking_result(means, users, pu, rk)
 
     def replicas_consistent(self) -> bool:
         ok = C.c_int32()

@@ -221,6 +221,31 @@ class MF_fastALS_T {
                                        r.scores.data()), "eals_group_recommend_vectors");
     return r;
   }
+  // Ranking metrics at k on a held-out test matrix (CSR over all users: row_ptr of userCount + 1 offsets, ascending
+  // col_idx).  A test item's rank is its position in recommend({u}, k, exclude_seen), or -1; the means are over the
+  // users with test items.  per_user: [userCount][6] (hit rate, precision, recall, NDCG, MAP, MRR), ranks: one per
+  // test entry, both filled only when asked for.  1 <= k <= 1024.  The model is not touched.
+  struct RankingMetrics {
+    double hit_rate = 0, precision = 0, recall = 0, ndcg = 0, map = 0, mrr = 0;
+    int64_t users = 0;
+    std::vector<double> per_user;
+    std::vector<int32_t> ranks;
+  };
+  RankingMetrics ranking_metrics(const std::vector<int64_t>& row_ptr, const std::vector<int32_t>& col_idx, int k,
+                                 bool exclude_seen = true, bool want_per_user = false, bool want_ranks = false) {
+    if ((int64_t)row_ptr.size() != (int64_t)userCount + 1) throw std::invalid_argument("ranking_metrics: row_ptr must have userCount + 1 offsets");
+    RankingMetrics r;
+    if (want_per_user) r.per_user.resize((size_t)userCount * 6);
+    if (want_ranks) r.ranks.resize((size_t)(row_ptr.back() - row_ptr.front()));
+    double means[6];
+    const int32_t none = 0;
+    check(eals_group_ranking_metrics(g_, EALS_HOST, row_ptr.data(), col_idx.empty() ? &none : col_idx.data(), k, exclude_seen ? 1 : 0,
+                                     means, &r.users, want_per_user ? r.per_user.data() : nullptr,
+                                     want_ranks && !r.ranks.empty() ? r.ranks.data() : nullptr),
+          "eals_group_ranking_metrics");
+    r.hit_rate = means[0]; r.precision = means[1]; r.recall = means[2]; r.ndcg = means[3]; r.map = means[4]; r.mrr = means[5];
+    return r;
+  }
   void update_user_thread(int u) { check(eals_group_update_user_row(g_, u), "eals_group_update_user_row"); }
   void update_item_thread(int i) { check(eals_group_update_item_row(g_, i), "eals_group_update_item_row"); }
   void update_user_SU(double* oldVector, double* uget) { check(eals_group_patch_SU(g_, oldVector, uget), "eals_group_patch_SU"); }

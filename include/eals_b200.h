@@ -208,9 +208,10 @@ int eals_evaluate(eals_model* m, const int32_t* gt_items, int32_t topk, int32_t 
                   double sums[3], double* hr, double* ndcg, double* prec, int32_t* count_larger);
 int eals_evaluate_user(eals_model* m, int32_t u, int32_t gt_item, int32_t topk, int32_t mode,
                        double out[3]);
-/* How the last eals_evaluate ran: out[0] = 1 when the scores went through the tcgen05 fp16 filter (lists of
- * >= 128 users; every close call re-scored in fp64 with the reference's operation order, so the results are
- * identical to the all-fp64 scan), 0 for the exact fp64 tile scan; out[1] = users whose certain count stayed
+/* How the last eals_evaluate or eals_ranking_metrics ran (for ranking metrics "users" are test entries, and out[0] is
+ * 1 only when every chunk of entries went through the filter): out[0] = 1 when the scores went through the tcgen05
+ * fp16 filter (lists of >= 128 users; every close call re-scored in fp64 with the reference's operation order, so
+ * the results are identical to the all-fp64 scan), 0 for the exact fp64 tile scan; out[1] = users whose certain count stayed
  * <= topK after the filter (candidates), out[2] = (user, item) pairs re-scored exactly; out[3], out[4], out[5] =
  * users, items and device microseconds of the filter's FIRST item block (every user against the highest-norm
  * items: the one launch of known shape, 2 * users * items * roundup(factors, 64) flop — the tensor roofline). */
@@ -248,6 +249,21 @@ int eals_fold_in(eals_model* m, int32_t space, int32_t n, const int64_t* row_ptr
  * folded in from.  eals_recommend_stats reports the last eals_recommend or eals_recommend_vectors call. */
 int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
                            int32_t k, int32_t* items, double* scores);
+
+/* Ranking metrics at k on a held-out test matrix.  test_ptr / test_idx: a CSR with one row per user (n_users + 1
+ * offsets, the rules of eals_set_train; this model reads the rows of its own users).  For a test entry (u, g) the
+ * rank is g's 0-based position in the list eals_recommend(u, k, exclude_seen) returns, or -1 when g is not in it (a
+ * test item in u's train row is always -1 with exclude_seen).  Per user with n_u > 0 test items and H the hit ranks:
+ * [0] hit rate (H non-empty), [1] precision |H| / k, [2] recall |H| / n_u, [3] NDCG sum_{h in H} ln 2 / ln(h + 2)
+ * over the same sum for 0 .. min(k, n_u) - 1, [4] MAP (1 / min(k, n_u)) sum_{h in H} #{h' in H : h' <= h} / (h + 1),
+ * [5] MRR 1 / (min H + 1).  sums[6]: the sums over this model's users with test items, in user order, *n_users their
+ * number; per_user ([user_end - user_begin][6], 0 for users without test items) and ranks (one per test entry of
+ * the owned rows, in CSR order) are optional.  1 <= k <= 1024; every rank is decided by exact fp64 comparisons
+ * (tcgen05 filter for lists of >= 128 entries, the exact engine otherwise or with EALS_EVAL_SCALAR=1, both giving
+ * the same result).  Arrays are host or device memory as `space` says.  The model stays exactly as it was;
+ * eals_eval_stats reports this call like an evaluate. */
+int eals_ranking_metrics(eals_model* m, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
+                         int32_t exclude_seen, double sums[6], int64_t* n_users, double* per_user, int32_t* ranks);
 
 /* Plumbing for the host layer. */
 int eals_leading_dim(const eals_model* m);                 /* ld of U/V/SU/SV rows, in doubles   */
@@ -346,6 +362,10 @@ int eals_group_fold_in(eals_group* g, int32_t space, int32_t n, const int64_t* r
                        const double* val, const double* init, int32_t n_iter, double* out);
 int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr,
                                  const int32_t* ex_idx, int32_t k, int32_t* items, double* scores);
+/* eals_ranking_metrics over the whole matrix: each rank on the rows it owns, sums added in rank order.  means[6] are
+ * divided by *n_users (0 when no user has test items); per_user is [n_users][6], ranks in test-entry order. */
+int eals_group_ranking_metrics(eals_group* g, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
+                               int32_t exclude_seen, double means[6], int64_t* n_users, double* per_user, int32_t* ranks);
 int eals_group_sync(eals_group* g);
 int eals_group_replicas_consistent(eals_group* g, int32_t* ok);             /* all U / V replicas bit-identical */
 int eals_group_save_factors(eals_group* g, const char* path);
