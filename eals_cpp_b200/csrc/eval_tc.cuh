@@ -554,16 +554,18 @@ __global__ void item_sort_keys_kernel(const double* __restrict__ V, int K, int L
   }
 }
 
-// flags[s] = 1 when slot s is still undecided (certain count <= topK)
-__global__ void undecided_flags_kernel(const int32_t* __restrict__ list, const int32_t* __restrict__ n_list, int n_max,
-                                       const int32_t* __restrict__ cnt_hi, int topk, uint8_t* __restrict__ flags) {
+// flags[p] = 1 while the slot s at list position p stays in the working set: its certain count is below its limit,
+// lim[s] (lim nullable: lim_all for every slot).  evaluate: topK + 1; ranking metrics: k + c_R per slot.
+__global__ void below_limit_flags_kernel(const int32_t* __restrict__ list, const int32_t* __restrict__ n_list, int n_max,
+                                         const int32_t* __restrict__ cnt_hi, const int32_t* __restrict__ lim, int lim_all,
+                                         uint8_t* __restrict__ flags) {
   const int p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= n_max) return;
   const int n = n_list ? *n_list : n_max;
   uint8_t f = 0;
   if (p < n) {
     const int s = list ? list[p] : p;
-    f = cnt_hi[s] <= topk;
+    f = cnt_hi[s] < (lim ? lim[s] : lim_all);
   }
   flags[p] = f;
 }

@@ -438,9 +438,7 @@ int eals_group_evaluate(eals_group* g, const int32_t* gt_items, int32_t topk, in
 int eals_group_recommend(eals_group* g, int32_t space, int32_t n, const int32_t* users, int32_t k, int32_t exclude_seen,
                          int32_t* items, double* scores) {
   if (!g || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
-  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
-  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
-  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(check_topk_args(space, n, k));
   OK(group_barrier(g));
   if (n == 0) return EALS_OK;
   std::vector<int32_t> hu((size_t)n);
@@ -546,9 +544,7 @@ extern "C" {
 int eals_group_fold_in(eals_group* g, int32_t space, int32_t n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
                        const double* init, int32_t n_iter, double* out) {
   if (!g || (n > 0 && (!row_ptr || !col_idx || !out))) return fail(EALS_ERR_ARG, "null argument");
-  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
-  if (n_iter < 1) return fail(EALS_ERR_ARG, "n_iter must be >= 1, got %d", n_iter);
-  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(check_fold_in_args(space, n, n_iter));
   OK(group_barrier(g));
   if (n == 0) return EALS_OK;
   const size_t K = (size_t)g->base.factors;
@@ -568,9 +564,7 @@ int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const 
                                  const int32_t* ex_idx, int32_t k, int32_t* items, double* scores) {
   if (!g || (n > 0 && (!Q || !items))) return fail(EALS_ERR_ARG, "null argument");
   if ((ex_ptr == nullptr) != (ex_idx == nullptr)) return fail(EALS_ERR_ARG, "ex_ptr and ex_idx must both be given or both be null");
-  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
-  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
-  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(check_topk_args(space, n, k));
   OK(group_barrier(g));
   if (n == 0) return EALS_OK;
   const size_t K = (size_t)g->base.factors;
@@ -594,8 +588,7 @@ int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const 
 int eals_group_ranking_metrics(eals_group* g, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
                                int32_t exclude_seen, double means[6], int64_t* n_users, double* per_user, int32_t* ranks) {
   if (!g || !test_ptr || !test_idx || !means || !n_users) return fail(EALS_ERR_ARG, "null argument");
-  if (k < 1 || k > eals::rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", eals::rec::kMaxK, k);
-  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(check_topk_args(space, 0, k));
   OK(group_barrier(g));
   const int M = g->base.n_users;
   HostCsr t;

@@ -11,7 +11,7 @@
 //   rm_train_score_kernel  the exact score of every train nonzero of the users that have test entries, once
 //   rm_train_count_kernel  c_R = train items ahead of g (they are ahead in the full order but not in the list), the
 //                          "g is in the train row" verdict, and the per-slot limit k + c_R of the certain count
-//   rm_keep_flags_kernel   working set: certain count < limit
+//                          (the working set keeps a slot while its certain count is below it: below_limit_flags_kernel)
 //   rm_rescore_kernel      exact tie-aware count over the MODE 2 candidates of the survivors
 //   rm_rank_kernel         rank = exact count - c_R, or -1
 //   rm_lookup_kernel       exact engine: positions of the test items in recommend's exact lists
@@ -74,7 +74,8 @@ rm_train_score_kernel(const double* __restrict__ U, const double* __restrict__ V
 // One warp per slot s (test entry of user[s], item[s], exact score gts[s]).  rptr == nullptr (no exclusion): c_r = 0,
 // lim = k.  Otherwise the walk over the user's train row (scores from rm_train_score_kernel, score[z - z0]):
 // c_r[s] = train items ahead of g under the list's order, and lim[s] = k + c_r[s], or 0 when g itself is in the
-// train row (rank -1, the slot never enters the filter).
+// train row (rank -1, the slot never enters the filter).  A slot whose certain count reaches k + c_R has at least k
+// eligible items ahead of it (at most c_R of the certainly larger ones are train items).
 __global__ void rm_train_count_kernel(const int64_t* __restrict__ rptr, const int32_t* __restrict__ ridx, const double* __restrict__ score,
                                       int64_t z0, int ub, const int32_t* __restrict__ user, const int32_t* __restrict__ item,
                                       const double* __restrict__ gts, int n, int k, int32_t* __restrict__ c_r, int32_t* __restrict__ lim) {
@@ -99,22 +100,6 @@ __global__ void rm_train_count_kernel(const int64_t* __restrict__ rptr, const in
     c_r[s] = cnt;
     lim[s] = seen ? 0 : k + cnt;
   }
-}
-
-// flags[p] = 1 while the slot at list position p may still rank below k: certain count < its limit.  A slot whose
-// certain count reaches k + c_R has at least k eligible items ahead of it (at most c_R of the certainly larger
-// ones are train items).
-__global__ void rm_keep_flags_kernel(const int32_t* __restrict__ list, const int32_t* __restrict__ n_list, int n_max,
-                                     const int32_t* __restrict__ cnt_hi, const int32_t* __restrict__ lim, uint8_t* __restrict__ flags) {
-  const int p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= n_max) return;
-  const int n = n_list ? *n_list : n_max;
-  uint8_t f = 0;
-  if (p < n) {
-    const int s = list ? list[p] : p;
-    f = cnt_hi[s] < lim[s];
-  }
-  flags[p] = f;
 }
 
 // One thread per candidate pair of the MODE 2 emission (every item with acc >= g^ - E, so every item that is not

@@ -392,6 +392,27 @@ int select_flagged(eals_model* m, const int32_t* in, int n, int32_t* out, int32_
   return in ? run(in) : run(thrust::counting_iterator<int32_t>(0));
 }
 
+// The working list of a filter pass: `cur` (nullptr: the slots 0 .. n-1) and the two buffers it alternates between.
+struct WorkList {
+  const int32_t* cur = nullptr;
+  int32_t *next, *spare;
+  explicit WorkList(eals_eval_ws& ws) : next(ws.list_a.p), spare(ws.list_b.p) {}
+};
+
+// Compaction of the working list: its first n entries whose ws.flags are set (the caller's flag kernel) -> wl.next,
+// their number -> d_n, their fp16 rows ws.Uh -> ws.W; wl.next becomes the list.  Only enqueues work: the count stays
+// on the device for the next filter launch.
+int compact_list(eals_model* m, WorkList& wl, int n, int32_t* d_n) {
+  eals_eval_ws& ws = eval_ws(m);
+  const int KP = (m->K + eals::tc::kKC - 1) / eals::tc::kKC * eals::tc::kKC;
+  OK(select_flagged(m, wl.cur, n, wl.next, d_n));
+  eals::tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, m->stream>>>(ws.Uh.p, KP, wl.next, d_n, ws.W.p);
+  OK(check_launch(m));
+  wl.cur = wl.next;
+  std::swap(wl.next, wl.spare);
+  return EALS_OK;
+}
+
 // Preparation of the tcgen05 filter for the rows X[d_rows[0 .. n)] (d_rows nullable: X[0 .. n); evaluate and
 // recommend): fp16 copies of V in decreasing-norm order (ws.perm: rank -> item) and of the query rows, their norms,
 // the per-tile item norms and the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).
@@ -456,85 +477,118 @@ int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, con
   return tc_prepare_rows(m, n, X, d_rows, d_thr);
 }
 
-// Fills `out` and m->eval_stats (engine 1), or returns with neither touched when the pair list overflows.
-int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, int topk, bool want_triples, ScanResult& out) {
+// What a count pass hands back: the survivors of the certain count (a device list of n_cand slots) and their `pairs`
+// emitted pairs in ws.pairs (that count also at d_pairs on the device); or `overflow` when the pairs would exceed the
+// hard cap: the filter is not filtering, and the caller's exact engine answers instead.
+struct CountPass {
+  const int32_t* surv = nullptr;
+  int n_cand = 0;
+  unsigned long long pairs = 0;
+  unsigned long long* d_pairs = nullptr;
+  bool overflow = false;
+};
+
+// Count-and-emit pass of the tcgen05 filter over n slots that tc_prepare_rows has prepared (evaluate, ranking
+// metrics).  MODE 0 walks the item blocks and counts, per slot, the items certainly ahead of its threshold into
+// ws.cnt; between blocks the working set keeps the slots whose count is below their limit, lim[s] (lim nullable:
+// lim_all for every slot), compacted on the device.  compact_first also compacts once before the first block, for
+// slots that start at their limit; `timed` times the first block into ws.blk0.  The survivors then go through the
+// filter in emission mode EMIT over the whole catalogue: a first buffer of pairs_per_cand pairs per survivor
+// (2^20 .. 2^27), then one more attempt at the exact size; beyond the hard cap (2^30 pairs, 16 GB) it overflows.
+// Both caps as read_pair_caps gives them, the first never above the hard one.
+// ws.cnt_exact is zeroed for the caller's re-score of the pairs.
+template <int EMIT>
+int count_pass(eals_model* m, int n, const int32_t* lim, int lim_all, bool compact_first, bool timed, unsigned long long pairs_per_cand,
+               StageTimer& tm, CountPass& out) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
-  StageTimer tm;
-  const int K = m->K, LD = m->LD, N = m->N;
+  const int K = m->K, N = m->N;
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
   cudaStream_t st = m->stream;
-  OK(tc_prepare(m, n, m->U, d_users, d_gts));
+  out = CountPass{};
   CU(cudaMemsetAsync(ws.cnt.p, 0, sizeof(int32_t) * n, st));
   CU(cudaMemsetAsync(ws.cnt_exact.p, 0, sizeof(int32_t) * n, st));
   CUtensorMap mapV, mapU0, mapW;
   OK(make_half_map(&mapV, ws.Vh.p, (size_t)N, KP));
   OK(make_half_map(&mapU0, ws.Uh.p, (size_t)n, KP));
   OK(make_half_map(&mapW, ws.W.p, (size_t)n + 2 * tc::kTM, KP));
-  int32_t* d_n = ws.scalars.p;          // [0]: size of the current working list, [1]: next
+  int32_t* d_n = ws.scalars.p;          // size of the working list
   set_i32_kernel<<<1, 1, 0, st>>>(d_n, n);
   OK(check_launch(m));
-  tm.lap("eval: fp16 copies, norms, item order");
 
   // ---- MODE 0 over L2-sized item blocks, working set compacted on the device between them ----
   tc::TcArgs a{};
   a.sp0 = ws.sp0.p; a.sp1 = ws.sp1.p; a.tile_norm = ws.tile_norm.p; a.n_items = N; a.cnt_hi = ws.cnt.p; a.perm = ws.perm.p;
-  const int32_t* list = nullptr;        // identity
-  int32_t *list_next = ws.list_a.p, *list_other = ws.list_b.p;
-  auto compact = [&](void) -> int {     // undecided users of the current list -> list_next, their rows -> W
-    tc::undecided_flags_kernel<<<(n + 255) / 256, 256, 0, st>>>(list, d_n, n, ws.cnt.p, topk, ws.flags.p);
+  WorkList wl(ws);
+  auto compact = [&](void) -> int {     // slots of the list still below their limit
+    tc::below_limit_flags_kernel<<<(n + 255) / 256, 256, 0, st>>>(wl.cur, d_n, n, ws.cnt.p, lim, lim_all, ws.flags.p);
     OK(check_launch(m));
-    OK(select_flagged(m, list, n, list_next, d_n + 1));
-    CU(cudaMemcpyAsync(d_n, d_n + 1, sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
-    tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, st>>>(ws.Uh.p, KP, list_next, d_n, ws.W.p);
-    OK(check_launch(m));
-    list = list_next;
-    std::swap(list_next, list_other);
-    return EALS_OK;
+    return compact_list(m, wl, n, d_n);
   };
+  if (compact_first) OK(compact());
   for (ItemBlocks blk(N, 0); blk.i0 < N; blk.next()) {
-    a.act = list; a.n_act = d_n; a.it0 = blk.it0; a.it1 = blk.it1;
-    const bool first_block = blk.i0 == 0;
+    a.act = wl.cur; a.n_act = d_n; a.it0 = blk.it0; a.it1 = blk.it1;
+    const bool first_block = timed && blk.i0 == 0;
     if (first_block) OK(ws.blk0.start(st));
-    OK(launch_filter_k<0>(m, nkc, list ? mapW : mapU0, mapV, a));
+    OK(launch_filter_k<0>(m, nkc, wl.cur ? mapW : mapU0, mapV, a));
     if (first_block) OK(ws.blk0.stop(st, n, std::min<int64_t>(N, (int64_t)a.it1 * tc::kTN)));
     OK(compact());
     if (tm.on) {
       int left = 0;
       cudaMemcpy(&left, d_n, sizeof(int), cudaMemcpyDeviceToHost);
       char what[96];
-      snprintf(what, sizeof(what), "eval: items [%lld, %lld) -> %d undecided", (long long)blk.i0, (long long)blk.i1, left);
+      snprintf(what, sizeof(what), "filter: items [%lld, %lld) -> %d left", (long long)blk.i0, (long long)blk.i1, left);
       tm.lap(what);
     }
   }
-  // ---- MODE 1 for the candidates (certain count <= topK): emit, re-score exactly ----
-  int n_cand = 0;
-  CU(cudaMemcpyAsync(&n_cand, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  // ---- emission for the survivors ----
+  out.surv = wl.cur;
+  out.d_pairs = ws.counters.p + 1;
+  CU(cudaMemcpyAsync(&out.n_cand, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
-  unsigned long long got = 0;
-  unsigned long long* d_np = ws.counters.p + 1;
-  if (n_cand > 0) {
-    unsigned long long cap = std::min<unsigned long long>(1ull << 27, std::max<unsigned long long>(1ull << 20, 1024ull * (unsigned long long)n_cand));
-    unsigned long long hard_cap = 1ull << 30;           // 16 GB of pairs: beyond this the filter is not filtering
-    read_pair_caps(cap, hard_cap, ~0ull);
-    for (int attempt = 0; attempt < 2; attempt++) {
-      OK(ws.pairs.reserve((size_t)cap));
-      CU(cudaMemsetAsync(d_np, 0, sizeof(unsigned long long), st));
-      a.act = list; a.n_act = d_n; a.it0 = 0; a.it1 = n_tiles;
-      a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
-      OK(launch_filter_k<1>(m, nkc, mapW, mapV, a));
-      CU(cudaMemcpyAsync(&got, d_np, sizeof(got), cudaMemcpyDeviceToHost, st));
-      CU(cudaStreamSynchronize(st));
-      if (got <= cap) break;
-      if (attempt == 1 || got > hard_cap) return EALS_OK;   // degenerate scores: exact engine instead
-      cap = got;
-    }
-    tm.lap("eval: candidate emission (MODE 1)");
-    if (got) {
-      tc::eval_rescore_kernel<<<16 * m->sm_count, 128, 0, st>>>(m->U, m->V, K, LD, d_users, 0, d_gts, ws.pairs.p, d_np, got, ws.cnt_exact.p);
-      OK(check_launch(m));
-    }
+  if (out.n_cand == 0) return EALS_OK;
+  unsigned long long cap = std::min<unsigned long long>(1ull << 27, std::max<unsigned long long>(1ull << 20, pairs_per_cand * (unsigned long long)out.n_cand));
+  unsigned long long hard_cap = 1ull << 30;
+  read_pair_caps(cap, hard_cap, ~0ull);
+  cap = std::min(cap, hard_cap);
+  unsigned long long& got = out.pairs;
+  for (int attempt = 0; attempt < 2; attempt++) {
+    OK(ws.pairs.reserve((size_t)cap));
+    CU(cudaMemsetAsync(out.d_pairs, 0, sizeof(unsigned long long), st));
+    a.act = wl.cur; a.n_act = d_n; a.it0 = 0; a.it1 = n_tiles;
+    a.pairs = ws.pairs.p; a.n_pairs = out.d_pairs; a.cap_pairs = cap;
+    OK(launch_filter_k<EMIT>(m, nkc, mapW, mapV, a));
+    CU(cudaMemcpyAsync(&got, out.d_pairs, sizeof(got), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    if (got <= cap) break;
+    if (attempt == 1 || got > hard_cap) { out.overflow = true; return EALS_OK; }
+    cap = got;
+  }
+  tm.lap("filter: candidate emission");
+  return EALS_OK;
+}
+
+// Fills `out` and m->eval_stats (engine 1), or returns with neither touched when the pair list overflows.
+int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, int topk, bool want_triples, ScanResult& out) {
+  namespace tc = eals::tc;
+  eals_eval_ws& ws = eval_ws(m);
+  StageTimer tm;
+  const int K = m->K, LD = m->LD;
+  cudaStream_t st = m->stream;
+  OK(tc_prepare(m, n, m->U, d_users, d_gts));
+  tm.lap("eval: fp16 copies, norms, item order");
+  // a user is decided once its certain count exceeds topK (limit topK + 1, kept from overflowing); the candidates
+  // go through MODE 1, which also emits the pairs whose truncated key may be non-zero
+  CountPass cp;
+  OK(count_pass<1>(m, n, nullptr, (int)std::min<int64_t>((int64_t)topk + 1, INT32_MAX), false, true, 1024, tm, cp));
+  if (cp.overflow) return EALS_OK;
+  const int n_cand = cp.n_cand;
+  const unsigned long long got = cp.pairs;
+  if (got) {
+    tc::eval_rescore_kernel<<<16 * m->sm_count, 128, 0, st>>>(m->U, m->V, K, LD, d_users, 0, d_gts, ws.pairs.p, cp.d_pairs, got,
+                                                              ws.cnt_exact.p);
+    OK(check_launch(m));
   }
   tm.lap("eval: exact re-score");
   // candidates and their exact counts (a few per cent of the users at most); everybody else is decided
@@ -542,15 +596,15 @@ int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, i
   unsigned long long n_tr = 0;
   if (n_cand > 0) {
     OK(ws.active.reserve((size_t)n_cand));
-    eals::gather_i32_kernel<<<(n_cand + 255) / 256, 256, 0, st>>>(ws.cnt_exact.p, list, n_cand, ws.active.p);
+    eals::gather_i32_kernel<<<(n_cand + 255) / 256, 256, 0, st>>>(ws.cnt_exact.p, cp.surv, n_cand, ws.active.p);
     OK(check_launch(m));
-    CU(cudaMemcpyAsync(cand.data(), list, sizeof(int32_t) * n_cand, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(cand.data(), cp.surv, sizeof(int32_t) * n_cand, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(cand_cnt.data(), ws.active.p, sizeof(int32_t) * n_cand, cudaMemcpyDeviceToHost, st));
   }
   if (want_triples && got) {
     OK(ws.tkey.reserve((size_t)got)); OK(ws.tval.reserve((size_t)got));
     unsigned long long* d_nt = ws.counters.p + 2;
-    pairs_to_triples_kernel<<<8 * m->sm_count, 256, 0, st>>>(ws.pairs.p, d_np, ws.cnt.p, ws.cnt_exact.p, topk, ws.tkey.p, ws.tval.p, d_nt);
+    pairs_to_triples_kernel<<<8 * m->sm_count, 256, 0, st>>>(ws.pairs.p, cp.d_pairs, ws.cnt.p, ws.cnt_exact.p, topk, ws.tkey.p, ws.tval.p, d_nt);
     OK(check_launch(m));
     CU(cudaMemcpyAsync(&n_tr, d_nt, sizeof(n_tr), cudaMemcpyDeviceToHost, st));
   }
@@ -728,12 +782,6 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
   for (int t = n_tiles - 1; t >= 0; t--)
     rem[(size_t)t] = std::max(rem[(size_t)t + 1], std::nextafter(tn[(size_t)t].x + tn[(size_t)t].y, std::numeric_limits<float>::infinity()));
   int32_t* d_n = ws.scalars.p;          // [0]: working-list size, [1]: scratch, [2]: size of a chunk of the list
-  auto select = [&](const int32_t* in, int n_in, int32_t* out, int* n_out) -> int {   // select_flagged, count to the host
-    OK(select_flagged(m, in, n_in, out, d_n));
-    CU(cudaMemcpyAsync(n_out, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-    CU(cudaStreamSynchronize(st));
-    return EALS_OK;
-  };
   const rec::MergeArgs base = rec_args(m, q, k);
 
   // ---- seed ----
@@ -746,7 +794,9 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
     for (int b = 0; nl > 0 && r_end < N; b ^= 1) {
       rec::rec_unfilled_flags_kernel<<<(nl + 255) / 256, 256, 0, st>>>(lst, nullptr, nl, ws.thr.p, ws.flags.p);
       OK(check_launch(m));
-      OK(select(lst, nl, bufs[b], &nl));
+      OK(select_flagged(m, lst, nl, bufs[b], d_n));
+      CU(cudaMemcpyAsync(&nl, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+      CU(cudaStreamSynchronize(st));
       lst = bufs[b];
       const int r1 = (int)std::min<int64_t>(N, (int64_t)r_end + step);
       OK(rec_merge_exact(m, base, lst, nl, ws.perm.p, r_end, r1));
@@ -757,19 +807,16 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
   tm.lap("recommend: prep + exact seed");
 
   // ---- item blocks ----
-  const int32_t* list = nullptr;
+  WorkList wl(ws);
   int n_act = n;
-  int32_t *list_next = ws.list_a.p, *list_other = ws.list_b.p;
   auto compact = [&](int it_next) -> int {   // users that may still gain an item from tile it_next on
     OK(params());
-    rec::rec_keep_flags_kernel<<<(n_act + 255) / 256, 256, 0, st>>>(list, nullptr, n_act, ws.un_hat.p, ws.sp0.p, ws.thr.p,
+    rec::rec_keep_flags_kernel<<<(n_act + 255) / 256, 256, 0, st>>>(wl.cur, nullptr, n_act, ws.un_hat.p, ws.sp0.p, ws.thr.p,
                                                                     rem[(size_t)it_next], ws.flags.p);
     OK(check_launch(m));
-    OK(select(list, n_act, list_next, &n_act));
-    tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, st>>>(ws.Uh.p, KP, list_next, d_n, ws.W.p);
-    OK(check_launch(m));
-    list = list_next;
-    std::swap(list_next, list_other);
+    OK(compact_list(m, wl, n_act, d_n));
+    CU(cudaMemcpyAsync(&n_act, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     return EALS_OK;
   };
   OK(compact(seed / tc::kTN));
@@ -795,7 +842,7 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
       CUtensorMap mapW;
       OK(make_half_map(&mapW, ws.W.p + (size_t)p0 * KP, (size_t)(n + 2 * tc::kTM - p0), KP));
       OK(ws.pairs.reserve((size_t)cap));
-      a.act = list + p0; a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
+      a.act = wl.cur + p0; a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
       CU(cudaMemsetAsync(d_np, 0, sizeof(unsigned long long), st));
       const bool timed = first && p0 == 0 && nc == n_act;
       if (timed) OK(ws.blk0.start(st));
@@ -853,14 +900,23 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
   return EALS_OK;
 }
 
+// The device bytes of the per-slot lists of a top-k call, and of a chunk of ranking_metrics' test entries:
+// EALS_REC_LIST_BYTES, default 4 GiB.
+size_t list_budget() {
+  size_t bytes = (size_t)4 << 30;
+  if (const char* e = getenv("EALS_REC_LIST_BYTES")) bytes = std::max<size_t>(1, strtoull(e, nullptr, 10));
+  return bytes;
+}
+
+// The number of slots whose lists of k entries (12 bytes each) fit the budget, at least 1.
+size_t list_slots(int k) { return std::max<size_t>(1, list_budget() / (12 * (size_t)k)); }
+
 // Answers the slots 0 .. n-1 of q into items / scores (host or device memory as `space` says) and m->rec_stats.
 int rec_answer(eals_model* m, int space, int n, const RecQuery& q, int k, int32_t* items, double* scores) {
   eals_eval_ws& ws = eval_ws(m);
-  // Per-slot lists for at most `per` slots at a time (12 bytes per entry; EALS_REC_LIST_BYTES, default 4 GiB): the
-  // slots are answered in balanced chunks, each a complete call of an engine.
-  size_t list_bytes = (size_t)4 << 30;
-  if (const char* e = getenv("EALS_REC_LIST_BYTES")) list_bytes = std::max<size_t>(12 * (size_t)k, strtoull(e, nullptr, 10));
-  const int max_per = (int)std::min<size_t>((size_t)n, std::max<size_t>(1, list_bytes / (12 * (size_t)k)));
+  // Per-slot lists for at most `per` slots at a time: the slots are answered in balanced chunks, each a complete call
+  // of an engine.
+  const int max_per = (int)std::min<size_t>((size_t)n, list_slots(k));
   const int n_chunks = (n + max_per - 1) / max_per, per = (n + n_chunks - 1) / n_chunks;
   const size_t pk = (size_t)per * k;
   OK(ws.top_s.reserve(pk)); OK(ws.top_i.reserve(pk)); OK(ws.thr.reserve((size_t)per));
@@ -887,11 +943,18 @@ int rec_answer(eals_model* m, int space, int n, const RecQuery& q, int k, int32_
   return EALS_OK;
 }
 
-// The argument checks every top-k call shares.
-int rec_check_args(eals_model* m, int space, int n, int k) {
+// The argument checks of every top-k call (recommend, recommend_vectors, ranking_metrics with n = 0), on a model or a
+// group alike.
+int check_topk_args(int space, int n, int k) {
   if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
   if (k < 1 || k > rec::kMaxK) return fail(EALS_ERR_ARG, "k must be in [1, %d], got %d", rec::kMaxK, k);
   if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  return EALS_OK;
+}
+
+// ... and what a model must have for them.
+int rec_check_args(eals_model* m, int space, int n, int k) {
+  OK(check_topk_args(space, n, k));
   if (!m->factors_set) return fail(EALS_ERR_STATE, "factors not initialised");
   if (m->K > rec::kMaxFactors) return fail(EALS_ERR_UNSUPPORTED, "recommend supports up to %d factors", rec::kMaxFactors);
   return EALS_OK;
@@ -945,15 +1008,21 @@ int build_query_side(eals_model* m, Side& s, WsBuf<int>& check, int n, int space
   return rc;
 }
 
+// The argument checks of fold-in, on a model or a group alike.
+int check_fold_in_args(int space, int n, int n_iter) {
+  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
+  if (n_iter < 1) return fail(EALS_ERR_ARG, "n_iter must be >= 1, got %d", n_iter);
+  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  return EALS_OK;
+}
+
 // n_iter passes of update_user_thread (MF_fastALS.cpp:243-322) over each history row, from `init` (NULL: zeros),
 // with the model's V, SV, Wi and reg: the user CD kernels on a CdSide whose X is the workspace, no peers, no
 // prediction cache (every pass recomputes the predictions), untimed.  Nothing of the model changes.
 int fold_in_impl(eals_model* m, int space, int n, const int64_t* row_ptr, const int32_t* col_idx, const double* val,
                  const double* init, int n_iter, double* out) {
   if (!m || (n > 0 && (!row_ptr || !col_idx || !out))) return fail(EALS_ERR_ARG, "null argument");
-  if (n < 0) return fail(EALS_ERR_ARG, "n must be >= 0");
-  if (n_iter < 1) return fail(EALS_ERR_ARG, "n_iter must be >= 1, got %d", n_iter);
-  if (space != EALS_HOST && space != EALS_DEVICE) return fail(EALS_ERR_ARG, "space must be EALS_HOST or EALS_DEVICE");
+  OK(check_fold_in_args(space, n, n_iter));
   if (!m->factors_set) return fail(EALS_ERR_STATE, "factors not initialised");
   CU(cudaSetDevice(m->p.device));
   if (n == 0) return EALS_OK;
@@ -1001,24 +1070,13 @@ int recommend_vectors_impl(eals_model* m, int space, int n, const double* Q, con
 // ---- ranking metrics on a held-out test matrix (ranking.cuh, DESIGN.md §3.7) ------------------------------------
 namespace rk = eals::rk;
 
-// The device bytes a chunk of test entries may use (the entries' fp16 rows and working lists, the train scores):
-// recommend's list budget, EALS_REC_LIST_BYTES (default 4 GiB).
-size_t rm_chunk_bytes() {
-  size_t bytes = (size_t)4 << 30;
-  if (const char* e = getenv("EALS_REC_LIST_BYTES")) bytes = std::max<size_t>(1, strtoull(e, nullptr, 10));
-  return bytes;
-}
-
 // Engine 2 for the test entries of the owned rows [r0, r1) (n entries from e0 on, slot s = entry e0 + s): ranks of the
 // slots into d_ranks[0 .. n).  Fills `st` and sets `done` when it answers; leaves both as they are when the
 // candidate list overflows (the filter is not filtering: the exact engine answers instead).
 int rm_chunk_tc(eals_model* m, int r0, int r1, int k, bool exclude, bool timed, int32_t* d_ranks, EvalStats& st, bool& done) {
-  namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
   const Side &T = ws.test, &R = m->users;
-  const int K = m->K, LD = m->LD, N = m->N;
-  const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
-  const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
+  const int K = m->K, LD = m->LD;
   const int64_t e0 = T.h_ptr[(size_t)r0];
   const int n = (int)(T.h_ptr[(size_t)r1] - e0);
   cudaStream_t st_ = m->stream;
@@ -1041,77 +1099,23 @@ int rm_chunk_tc(eals_model* m, int r0, int r1, int k, bool exclude, bool timed, 
                                                                                        ws.c_r.p, ws.lim.p);
   OK(check_launch(m));
   OK(tc_prepare_rows(m, n, m->U, ws.users.p, ws.gts.p));
-  CU(cudaMemsetAsync(ws.cnt.p, 0, sizeof(int32_t) * n, st_));
-  CU(cudaMemsetAsync(ws.cnt_exact.p, 0, sizeof(int32_t) * n, st_));
-  CUtensorMap mapV, mapU0, mapW;
-  OK(make_half_map(&mapV, ws.Vh.p, (size_t)N, KP));
-  OK(make_half_map(&mapU0, ws.Uh.p, (size_t)n, KP));
-  OK(make_half_map(&mapW, ws.W.p, (size_t)n + 2 * tc::kTM, KP));
-  int32_t* d_n = ws.scalars.p;          // [0]: size of the current working list, [1]: next
-  set_i32_kernel<<<1, 1, 0, st_>>>(d_n, n);
-  OK(check_launch(m));
   tm.lap("ranking: slots, train correction, fp16 rows");
-
-  // ---- MODE 0 over the item blocks; a slot leaves once its certain count reaches k + c_R ----
-  tc::TcArgs a{};
-  a.sp0 = ws.sp0.p; a.sp1 = ws.sp1.p; a.tile_norm = ws.tile_norm.p; a.n_items = N; a.cnt_hi = ws.cnt.p; a.perm = ws.perm.p;
-  const int32_t* list = nullptr;        // identity
-  int32_t *list_next = ws.list_a.p, *list_other = ws.list_b.p;
-  auto compact = [&](void) -> int {     // slots of the current list still below their limit -> list_next, rows -> W
-    rk::rm_keep_flags_kernel<<<(n + 255) / 256, 256, 0, st_>>>(list, d_n, n, ws.cnt.p, ws.lim.p, ws.flags.p);
+  // a slot leaves once its certain count reaches k + c_R; the survivors go through MODE 2 (every item not certainly
+  // below s_g) for the exact tie-aware count.  Test items that are in the train row (limit 0) never enter the filter.
+  CountPass cp;
+  OK(count_pass<2>(m, n, ws.lim.p, 0, exclude, timed, 2048, tm, cp));
+  if (cp.overflow) return EALS_OK;
+  if (cp.pairs) {
+    rk::rm_rescore_kernel<<<16 * m->sm_count, 128, 0, st_>>>(m->U, m->V, K, LD, ws.users.p, ws.gt.p, ws.gts.p, ws.pairs.p, cp.pairs,
+                                                             ws.cnt_exact.p);
     OK(check_launch(m));
-    OK(select_flagged(m, list, n, list_next, d_n + 1));
-    CU(cudaMemcpyAsync(d_n, d_n + 1, sizeof(int32_t), cudaMemcpyDeviceToDevice, st_));
-    tc::gather_rows_kernel<<<8 * m->sm_count, 256, 0, st_>>>(ws.Uh.p, KP, list_next, d_n, ws.W.p);
-    OK(check_launch(m));
-    list = list_next;
-    std::swap(list_next, list_other);
-    return EALS_OK;
-  };
-  if (exclude) OK(compact());           // test items that are in the train row (limit 0) never enter the filter
-  for (ItemBlocks blk(N, 0); blk.i0 < N; blk.next()) {
-    a.act = list; a.n_act = d_n; a.it0 = blk.it0; a.it1 = blk.it1;
-    const bool first_block = timed && blk.i0 == 0;
-    if (first_block) OK(ws.blk0.start(st_));
-    OK(launch_filter_k<0>(m, nkc, list ? mapW : mapU0, mapV, a));
-    if (first_block) OK(ws.blk0.stop(st_, n, std::min<int64_t>(N, (int64_t)a.it1 * tc::kTN)));
-    OK(compact());
-  }
-  tm.lap("ranking: certain count (MODE 0)");
-  // ---- MODE 2 for the survivors (every item not certainly below s_g), exact tie-aware count ----
-  int n_cand = 0;
-  CU(cudaMemcpyAsync(&n_cand, d_n, sizeof(int32_t), cudaMemcpyDeviceToHost, st_));
-  CU(cudaStreamSynchronize(st_));
-  unsigned long long got = 0;
-  unsigned long long* d_np = ws.counters.p + 1;
-  if (n_cand > 0) {
-    unsigned long long cap = std::min<unsigned long long>(1ull << 27, std::max<unsigned long long>(1ull << 20, 2048ull * (unsigned long long)n_cand));
-    unsigned long long hard_cap = 1ull << 30;
-    read_pair_caps(cap, hard_cap, ~0ull);
-    cap = std::min(cap, hard_cap);
-    for (int attempt = 0; attempt < 2; attempt++) {
-      OK(ws.pairs.reserve((size_t)cap));
-      CU(cudaMemsetAsync(d_np, 0, sizeof(unsigned long long), st_));
-      a.act = list; a.n_act = d_n; a.it0 = 0; a.it1 = n_tiles;
-      a.pairs = ws.pairs.p; a.n_pairs = d_np; a.cap_pairs = cap;
-      OK(launch_filter_k<2>(m, nkc, mapW, mapV, a));
-      CU(cudaMemcpyAsync(&got, d_np, sizeof(got), cudaMemcpyDeviceToHost, st_));
-      CU(cudaStreamSynchronize(st_));
-      if (got <= cap) break;
-      if (attempt == 1 || got > hard_cap) return EALS_OK;   // degenerate scores: exact engine instead
-      cap = got;
-    }
-    if (got) {
-      rk::rm_rescore_kernel<<<16 * m->sm_count, 128, 0, st_>>>(m->U, m->V, K, LD, ws.users.p, ws.gt.p, ws.gts.p, ws.pairs.p, got, ws.cnt_exact.p);
-      OK(check_launch(m));
-    }
   }
   rk::rm_rank_kernel<<<(n + 255) / 256, 256, 0, st_>>>(n, ws.cnt.p, ws.lim.p, ws.cnt_exact.p, ws.c_r.p, k, d_ranks);
   OK(check_launch(m));
   CU(cudaStreamSynchronize(st_));
-  tm.lap("ranking: candidates (MODE 2) + exact re-score");
+  tm.lap("ranking: exact re-score + ranks");
   if (timed) OK(ws.blk0.read(st.blk0));
-  st.engine = 1; st.candidates += n_cand; st.pairs += (long long)got;
+  st.engine = 1; st.candidates += cp.n_cand; st.pairs += (long long)cp.pairs;
   done = true;
   return EALS_OK;
 }
@@ -1126,7 +1130,7 @@ int rm_chunk_exact(eals_model* m, int r0, int r1, int k, bool exclude, int32_t* 
   for (int r = r0; r < r1; r++)
     if (T.h_ptr[(size_t)r + 1] > T.h_ptr[(size_t)r]) users.push_back(m->ub + r);
   const int n = (int)users.size();
-  const int per = (int)std::min<size_t>((size_t)std::max(n, 1), std::max<size_t>(1, rm_chunk_bytes() / (12 * (size_t)k)));
+  const int per = (int)std::min<size_t>((size_t)std::max(n, 1), list_slots(k));
   for (int d0 = 0; d0 < n; d0 += per) {
     const int nd = std::min(per, n - d0);
     OK(ws.users.reserve((size_t)nd));
@@ -1160,7 +1164,7 @@ int ranking_metrics_impl(eals_model* m, int space, const int64_t* test_ptr, cons
   m->eval_stats = EvalStats{};
   // ---- ranks, chunk by chunk of whole rows within the device budget ----
   const int KP = (m->K + eals::tc::kKC - 1) / eals::tc::kKC * eals::tc::kKC;
-  const size_t budget = rm_chunk_bytes();
+  const size_t budget = list_budget();   // the entries' fp16 rows and working lists, the train scores
   const size_t per_entry = 4 * (size_t)KP + 128, per_nz = exclude ? 8 : 0;
   EvalStats total;
   bool any = false, all_tc = true, items_ready = false;
