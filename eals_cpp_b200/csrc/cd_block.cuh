@@ -272,7 +272,7 @@ cd_warp_block_kernel(CdSide a, const int32_t* __restrict__ order, int first, int
         if (j < n_n) {
           id_n[m] = a.idx[p0_n + j];
           if (a.use_cache) pc_n[m] = a.pc_in[p0_n + j];
-          if (a.pc_out.n) g_n[m] = a.pc_map[p0_n + j];
+          if (a.pc_out) g_n[m] = a.pc_map[p0_n + j];
         }
       }
     } else if (USER) {
@@ -481,17 +481,16 @@ cd_warp_block_kernel(CdSide a, const int32_t* __restrict__ order, int first, int
       }
     }
     for (int k = lane; k < K; k += 32) store_row_value(a, (size_t)grow * LD + k, x_s[k]);
-    if (a.pc_out.n) {
+    if (a.pc_out) {
 #pragma unroll
       for (int m = 0; m < MAXM; m++) {
         const int j = m * 32 + lane;
-        if (j < n) pc_emit(a, p0 + j, gpos[m], pr[m]);
+        if (j < n) pc_emit(a, gpos[m], pr[m]);
       }
     }
     for (int st = stages_in_loop; st < 4; st++) fetch_next(st, slot + stride);   // K < 64: finish the chain here
     __syncwarp();
   }
-  peers_release(a);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -716,14 +715,13 @@ cd_row_block_kernel(CdSide a, const int32_t* __restrict__ order, int first) {
     }
   }
   for (int k = tid; k < K; k += kT) store_row_value(a, (size_t)grow * LD + k, x_s[k]);
-  if (a.pc_out.n) {
+  if (a.pc_out) {
 #pragma unroll
     for (int m = 0; m < MW; m++) {
       const int j = m * kT + tid;
       if (j < n) pc_store(a, p0 + j, pr[m]);
     }
   }
-  peers_release(a);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -868,7 +866,7 @@ heavy_step_kernel(CdSide a, HeavyUnits hu, int u0, int fb, int nblocks, double* 
       }
       pr = (a0 + a1) + (a2 + a3);
       if (fb < nblocks) pred[poff + tid] = pr;
-      else if (a.pc_out.n) { pc_store(a, off + tid, pr); peers_release(a); }   // final value -> symmetric cache
+      else if (a.pc_out) pc_store(a, off + tid, pr);   // final value -> symmetric cache
     }
   } else if (a.use_cache && tid < n) {
     pred[poff + tid] = pr;   // the pipeline's compact cache starts from the symmetric one
@@ -1007,7 +1005,6 @@ heavy_solve_kernel(CdSide a, HeavyUnits hu, int h0, int g0, int fb, const double
       delta[(size_t)h * 16 + ff] = livef ? xnew - xf : 0.0;
       if (livef) store_row_value(a, (size_t)grow * LD + f0 + ff, xnew);
     }
-    peers_release(a);
   }
 }
 

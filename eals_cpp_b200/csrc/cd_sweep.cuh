@@ -35,13 +35,6 @@ struct PeerSet {
   int n;
 };
 
-// The other orientation's prediction caches: rank r holds global positions [bound[r], bound[r+1]).
-struct PcOut {
-  double* base[8];
-  uint32_t bound[9];
-  int n;                   // ranks (0: no cache)
-};
-
 struct CdSide {
   const int64_t* ptr;   // [rows+1] offsets of the owned rows (first owned row at 0)
   const int32_t* idx;   // neighbour ids, ascending inside a row
@@ -56,72 +49,31 @@ struct CdSide {
   // Symmetric prediction cache.  The prediction <u, v> a user sweep leaves behind for a nonzero is
   // exactly the value the item sweep starts from (and vice versa), so the gather pass that rebuilds
   // it (MF_fastALS.cpp:261-270 / 352-363) is skipped: each side READS its own cache sequentially
-  // (pc_in, this side's nonzero order) and WRITES the other side's cache at the position of the
-  // same nonzero in the other orientation (pc_map), on whichever rank owns that row (pc_out).
+  // (pc_in, this side's nonzero order) and WRITES local nonzero q's final prediction to pc_out[pc_map[q]].
+  // One rank: pc_out is the other orientation's cache and pc_map the position of the same nonzero in it.
+  // Several ranks: pc_out is a LOCAL staging array in destination order (pc_map: the slot in that order), and
+  // the host copies each destination's segment to its owner afterwards.  Scattered 8-byte stores straight into
+  // peer memory were far slower than the gather they replace (r01f).
   const double* pc_in;     // nullptr: no cache
-  const uint32_t* pc_map;  // per local nonzero: its global position in the other orientation
-  PcOut pc_out;
-  // Multi-rank: final predictions are first written to a LOCAL staging array, already in destination order
-  // (pc_map then holds, per local nonzero, its slot in that order), and copied to their owners afterwards by
-  // pc_route_kernel — a pure streaming copy.  Scattered 8-byte stores straight into peer memory were far
-  // slower than the gather they replace (r01f); staging in source order and gathering in the copy kernel cost
-  // 5 ms per half-epoch at 2 GPUs (r02i).
-  double* pc_stage;        // nullptr: store directly through pc_map / pc_out
+  const uint32_t* pc_map;
+  double* pc_out;          // nullptr: no cache output
   int use_cache;           // 1: pc_in is valid on entry, read it instead of recomputing
   PeerSet peers;        // other ranks' replicas of X (n = 0: none)
-  int fence;            // 1: every thread ends with a system-scope fence when it may have stored to a peer (peers_release)
 };
 
+// No fence after the peer stores: grid completion already performs the kernel's stores at system scope before
+// anything ordered after it in the stream (the event the other ranks wait on, or the NCCL all-reduce) can start.
+// A per-thread __threadfence_system() cost 7 % at 4 GPUs (DESIGN.md §6).
 __device__ __forceinline__ void store_row_value(const CdSide& a, size_t off, double v) {
   a.X[off] = v;
   for (int p = 0; p < a.peers.n; p++) a.peers.x[p][off] = v;
 }
 
-// Optional (EALS_PEER_FENCE=1): every thread of a sweep kernel ends with a system-scope fence after its last
-// peer store.  Off by default: grid completion already performs the kernel's stores at system scope before
-// anything ordered after it in the stream (the event the other ranks wait on, or the NCCL all-reduce) can
-// start, and the fence is expensive — a CTA-per-row kernel cannot retire its CTA until the NVLink stores are
-// acknowledged: 129.0 -> 120.5 ms per epoch at 4 GPUs without it (profiles/r2/r02w_*), same loss bits, replicas
-// identical.  It was added in round 1 when one 8-GPU run ended 0.19 % off; that turned out to be the start-up
-// race (no barrier between init and the first peer store, fixed in round 2), not visibility.
-__device__ __forceinline__ void peers_release(const CdSide& a) {
-  if (a.fence && (a.peers.n > 0 || (a.pc_out.n > 1 && !a.pc_stage))) __threadfence_system();
-}
-
-// Store a prediction at global position g of the other orientation's cache (on whichever rank holds it).
-__device__ __forceinline__ void pc_store_at(const CdSide& a, uint32_t g, double v) {
-  int r = 0;
-#pragma unroll
-  for (int t = 1; t < 8; t++) r += (t < a.pc_out.n && g >= a.pc_out.bound[t]) ? 1 : 0;
-  a.pc_out.base[r][g - a.pc_out.bound[r]] = v;
-}
-
-// The final prediction of local nonzero local_pos (its position g in the other orientation already
-// looked up, or not needed when the values are staged).
-__device__ __forceinline__ void pc_emit(const CdSide& a, int64_t local_pos, uint32_t g, double v) {
-  (void)local_pos;
-  if (a.pc_stage) a.pc_stage[g] = v;      // g = slot in destination order
-  else pc_store_at(a, g, v);              // g = global position in the other orientation
-}
+// The final prediction of a local nonzero, whose slot g = pc_map[local position] is already looked up.
+__device__ __forceinline__ void pc_emit(const CdSide& a, uint32_t g, double v) { a.pc_out[g] = v; }
 
 __device__ __forceinline__ void pc_store(const CdSide& a, int64_t local_pos, double v) {
-  pc_emit(a, local_pos, a.pc_map[local_pos], v);
-}
-
-// Second phase of the staged scheme: slot k of the staging array (DESTINATION order: route_dst ascending, so
-// neighbouring threads read neighbouring values and write neighbouring addresses of the same peer) goes to its
-// owner.  A small persistent grid, launched on a side stream right behind the Gram's main kernel.
-__global__ void __launch_bounds__(256)
-pc_route_kernel(const double* __restrict__ stage, const uint32_t* __restrict__ route_dst, int64_t n, PcOut out) {
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride) {
-    const uint32_t g = route_dst[k];
-    int r = 0;
-#pragma unroll
-    for (int t = 1; t < 8; t++) r += (t < out.n && g >= out.bound[t]) ? 1 : 0;
-    out.base[r][g - out.bound[r]] = stage[k];
-  }
-  if (out.n > 1) __threadfence_system();   // see peers_release
+  a.pc_out[a.pc_map[local_pos]] = v;
 }
 
 // inv[perm[k]] = k

@@ -187,6 +187,13 @@ struct BlockTiming { long long users = 0, items = 0; double ms = 0; };
 struct EvalStats { int engine = 0; long long candidates = 0, pairs = 0; BlockTiming blk0; };
 struct RecStats { int engine = 0; long long seed = 0, pairs = 0, left1 = 0; BlockTiming blk0; };   // left1: users left after block 1
 
+// One orientation's prediction caches on all ranks: rank r holds global positions [bound[r], bound[r+1]) at base[r].
+struct PcOut {
+  double* base[8];
+  uint32_t bound[9];
+  int n;                   // ranks (0: no cache)
+};
+
 }  // namespace
 
 struct eals_model {
@@ -223,10 +230,11 @@ struct eals_model {
   uint32_t* map_u = nullptr;     // owned CSR nonzero -> global CSC position of the same nonzero
   uint32_t* map_i = nullptr;     // owned CSC nonzero -> global CSR position
   size_t cap_pc_u = 0, cap_pc_i = 0, cap_map_u = 0, cap_map_i = 0;
-  // multi-rank: staged routing of the final predictions (see CdSide::pc_stage)
+  // multi-rank: the sweeps stage their final predictions in destination order (see CdSide::pc_out); route_src
+  // holds, per local nonzero, its slot in that order
   double *pc_stage_u = nullptr, *pc_stage_i = nullptr;
-  uint32_t *route_src_u = nullptr, *route_dst_u = nullptr, *route_src_i = nullptr, *route_dst_i = nullptr;
-  size_t cap_stage_u = 0, cap_stage_i = 0, cap_rsrc_u = 0, cap_rdst_u = 0, cap_rsrc_i = 0, cap_rdst_i = 0;
+  uint32_t *route_src_u = nullptr, *route_src_i = nullptr;
+  size_t cap_stage_u = 0, cap_stage_i = 0, cap_rsrc_u = 0, cap_rsrc_i = 0;
   bool routed = false;
   // Copy-engine exchange of the staged predictions (multi-rank): pair_cnt[su][ri] = nonzeros whose user belongs to
   // rank su and whose item to rank ri (every rank computes the whole table from the full index arrays).  A sender's
@@ -238,7 +246,6 @@ struct eals_model {
   long long pair_cnt[8][8] = {{0}};
   uint32_t *recv_idx_u = nullptr, *recv_idx_i = nullptr;
   size_t cap_recv_idx_u = 0, cap_recv_idx_i = 0;
-  bool copy_route = false;
   bool unpack_u_pending = false, unpack_i_pending = false;
   // multi-rank: a prediction cache that had to grow is not freed while peers may still map it (CUDA IPC):
   // the old buffer waits here until eals_ipc_gc; ipc_gen counts such reallocations
@@ -250,7 +257,7 @@ struct eals_model {
   int32_t *full_ci = nullptr, *full_ri = nullptr;
   unsigned char* route_tmp = nullptr;
   size_t cap_full_rp = 0, cap_full_cp = 0, cap_full_ci = 0, cap_full_ri = 0, cap_route_tmp = 0;
-  eals::PcOut out_to_items = {}, out_to_users = {};   // where the other side's caches live (all ranks)
+  PcOut out_to_items = {}, out_to_users = {};   // where the other side's caches live (all ranks)
   int n_ranks = 1, rank = 0;
   cudaStream_t side_stream = nullptr;   // routing of the final predictions runs here, under the Gram
   cudaEvent_t ev_swept = nullptr, ev_routed = nullptr;
@@ -433,26 +440,27 @@ __global__ void iota_kernel(uint32_t* __restrict__ v, int64_t n) {
   if (t < n) v[t] = (uint32_t)t;
 }
 
-// Destination order of one side's nonzeros (cub radix sort, once per matrix): route_dst = the map values
-// ascending; rsrc ends up holding, per LOCAL nonzero, its slot in that order — the index the sweep kernels
-// scatter their final predictions through (CdSide::pc_map in staged mode).
+// Destination order of one side's nonzeros (cub radix sort of the map values, once per matrix); rsrc ends up
+// holding, per LOCAL nonzero, its slot in that order — the index the sweep kernels scatter their final
+// predictions through (CdSide::pc_map with several ranks).
 int build_routes(eals_model* m, const uint32_t* map, int64_t n, double** stage, size_t* cap_stage,
-                 uint32_t** rsrc, size_t* cap_rsrc, uint32_t** rdst, size_t* cap_rdst) {
+                 uint32_t** rsrc, size_t* cap_rsrc) {
   OK(dev_reserve(stage, cap_stage, (size_t)n));
   OK(dev_reserve(rsrc, cap_rsrc, (size_t)n));
-  OK(dev_reserve(rdst, cap_rdst, (size_t)n));
   if (n == 0) return EALS_OK;
   if (n >= 0x7fffffffLL) return fail(EALS_ERR_UNSUPPORTED, "too many nonzeros per rank for the routed prediction cache");
-  uint32_t* iota = reinterpret_cast<uint32_t*>(*stage);   // scratch: the staging buffer is not live yet
+  // scratch: the staging buffer is not live yet and its 8 n bytes hold the iota and the sorted keys
+  uint32_t* iota = reinterpret_cast<uint32_t*>(*stage);
+  uint32_t* keys_out = iota + n;
   iota_kernel<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(iota, n);
   OK(check_launch(m));
   size_t tmp_bytes = 0;
-  cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, map, *rdst, iota, *rsrc, (int)n, 0, 32, m->stream);
+  cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, map, keys_out, iota, *rsrc, (int)n, 0, 32, m->stream);
   OK(dev_reserve(&m->route_tmp, &m->cap_route_tmp, std::max<size_t>(tmp_bytes, 16)));
-  const cudaError_t e = cub::DeviceRadixSort::SortPairs(m->route_tmp, tmp_bytes, map, *rdst, iota, *rsrc, (int)n, 0, 32, m->stream);
+  const cudaError_t e = cub::DeviceRadixSort::SortPairs(m->route_tmp, tmp_bytes, map, keys_out, iota, *rsrc, (int)n, 0, 32, m->stream);
   if (e != cudaSuccess) return fail(EALS_ERR_CUDA, "route sort -> %s", cudaGetErrorString(e));
   // the kernels scatter into the staging array through the INVERSE permutation (local nonzero -> slot in
-  // destination order); rsrc is replaced by it (the staging buffer, not live yet, is the scratch)
+  // destination order); rsrc is replaced by it (the staging buffer is the scratch again)
   eals::invert_perm_kernel<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(*rsrc, n, iota);
   OK(check_launch(m));
   CU(cudaMemcpyAsync(*rsrc, iota, sizeof(uint32_t) * (size_t)n, cudaMemcpyDeviceToDevice, m->stream));
@@ -461,7 +469,7 @@ int build_routes(eals_model* m, const uint32_t* map, int64_t n, double** stage, 
 }
 
 // Unmap the other ranks' prediction caches (multi-rank models).
-void close_pc_peers(eals_model* m, eals::PcOut& out, bool& attached_flag) {
+void close_pc_peers(eals_model* m, PcOut& out, bool& attached_flag) {
   for (int r = 0; r < out.n; r++)
     if (r != m->rank && out.base[r]) {
       if (!m->local_peers) cudaIpcCloseMemHandle(out.base[r]);
@@ -565,8 +573,8 @@ int build_pred_cache(eals_model* m, int space, const int64_t* row_ptr, const int
   // destination tables; the own rank's entries are filled now, the peers' by eals_ipc_attach
   const int nr = single ? 1 : m->n_ranks, me = single ? 0 : m->rank;
   {   // the peers' mappings stay (their buffers only move when THEY report a new ipc generation)
-    const eals::PcOut old_items = m->out_to_items, old_users = m->out_to_users;
-    m->out_to_items = eals::PcOut{}; m->out_to_users = eals::PcOut{};
+    const PcOut old_items = m->out_to_items, old_users = m->out_to_users;
+    m->out_to_items = PcOut{}; m->out_to_users = PcOut{};
     if (multi && was_attached)
       for (int r = 0; r < nr; r++) { m->out_to_items.base[r] = old_items.base[r]; m->out_to_users.base[r] = old_users.base[r]; }
   }
@@ -579,38 +587,34 @@ int build_pred_cache(eals_model* m, int space, const int64_t* row_ptr, const int
   m->out_to_users.base[me] = m->pc_u;
   m->pc_attached = single || (multi && was_attached);
   tm.lap("pred cache: position maps");
-  m->routed = false;
-  if (multi && !(getenv("EALS_PC_ROUTE") && getenv("EALS_PC_ROUTE")[0] == '0')) {
-    OK(build_routes(m, m->map_u, nu, &m->pc_stage_u, &m->cap_stage_u, &m->route_src_u, &m->cap_rsrc_u, &m->route_dst_u, &m->cap_rdst_u));
-    OK(build_routes(m, m->map_i, ni, &m->pc_stage_i, &m->cap_stage_i, &m->route_src_i, &m->cap_rsrc_i, &m->route_dst_i, &m->cap_rdst_i));
-    m->routed = true;
+  m->routed = multi;
+  if (multi) {
+    OK(build_routes(m, m->map_u, nu, &m->pc_stage_u, &m->cap_stage_u, &m->route_src_u, &m->cap_rsrc_u));
+    OK(build_routes(m, m->map_i, ni, &m->pc_stage_i, &m->cap_stage_i, &m->route_src_i, &m->cap_rsrc_i));
     // receiver side of the copy-engine exchange: the order the senders' segments arrive in = this rank's nonzeros
     // stably partitioned by the rank that owns the OTHER index (users of an item column ascend and a rank's
     // users are one contiguous range, so every sender's values arrive in ascending position)
-    m->copy_route = !(getenv("EALS_ROUTE_COPY") && getenv("EALS_ROUTE_COPY")[0] == '0');
     m->unpack_u_pending = m->unpack_i_pending = false;
-    if (m->copy_route) {
-      auto build_recv = [&](const Side& sd, bool by_user, uint32_t** out, size_t* cap, double* scratch_a, double* scratch_b) -> int {
-        const int64_t n = sd.nnz;
-        OK(dev_reserve(out, cap, (size_t)std::max<int64_t>(n, 1)));
-        if (n == 0) return EALS_OK;
-        uint32_t* key = reinterpret_cast<uint32_t*>(scratch_a);            // staging arrays are not live yet:
-        uint32_t* key_out = key + n;                                         // 8 n bytes each
-        uint32_t* val = reinterpret_cast<uint32_t*>(scratch_b);
-        source_rank_kernel<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(sd.idx, n, rb, by_user, key, val);
-        OK(check_launch(m));
-        size_t tmp = 0;
-        cub::DeviceRadixSort::SortPairs(nullptr, tmp, key, key_out, val, *out, (int)n, 0, 3, m->stream);
-        OK(dev_reserve(&m->route_tmp, &m->cap_route_tmp, std::max<size_t>(tmp, 16)));
-        if (cub::DeviceRadixSort::SortPairs(m->route_tmp, tmp, key, key_out, val, *out, (int)n, 0, 3, m->stream) != cudaSuccess)
-          return fail(EALS_ERR_CUDA, "receive-order sort");
-        CU(cudaStreamSynchronize(m->stream));
-        return EALS_OK;
-      };
-      // item columns hold USER ids (source = owner of the user); user rows hold ITEM ids
-      OK(build_recv(m->items, true, &m->recv_idx_i, &m->cap_recv_idx_i, m->pc_stage_i, m->pc_i + recv_offset(ni)));
-      OK(build_recv(m->users, false, &m->recv_idx_u, &m->cap_recv_idx_u, m->pc_stage_u, m->pc_u + recv_offset(nu)));
-    }
+    auto build_recv = [&](const Side& sd, bool by_user, uint32_t** out, size_t* cap, double* scratch_a, double* scratch_b) -> int {
+      const int64_t n = sd.nnz;
+      OK(dev_reserve(out, cap, (size_t)std::max<int64_t>(n, 1)));
+      if (n == 0) return EALS_OK;
+      uint32_t* key = reinterpret_cast<uint32_t*>(scratch_a);            // staging arrays are not live yet:
+      uint32_t* key_out = key + n;                                         // 8 n bytes each
+      uint32_t* val = reinterpret_cast<uint32_t*>(scratch_b);
+      source_rank_kernel<<<(unsigned)((n + 255) / 256), 256, 0, m->stream>>>(sd.idx, n, rb, by_user, key, val);
+      OK(check_launch(m));
+      size_t tmp = 0;
+      cub::DeviceRadixSort::SortPairs(nullptr, tmp, key, key_out, val, *out, (int)n, 0, 3, m->stream);
+      OK(dev_reserve(&m->route_tmp, &m->cap_route_tmp, std::max<size_t>(tmp, 16)));
+      if (cub::DeviceRadixSort::SortPairs(m->route_tmp, tmp, key, key_out, val, *out, (int)n, 0, 3, m->stream) != cudaSuccess)
+        return fail(EALS_ERR_CUDA, "receive-order sort");
+      CU(cudaStreamSynchronize(m->stream));
+      return EALS_OK;
+    };
+    // item columns hold USER ids (source = owner of the user); user rows hold ITEM ids
+    OK(build_recv(m->items, true, &m->recv_idx_i, &m->cap_recv_idx_i, m->pc_stage_i, m->pc_i + recv_offset(ni)));
+    OK(build_recv(m->users, false, &m->recv_idx_u, &m->cap_recv_idx_u, m->pc_stage_u, m->pc_u + recv_offset(nu)));
     tm.lap("pred cache: routes");
   }
   m->pcache_on = true;
@@ -1116,7 +1120,7 @@ int run_heavy_batch(eals_model* m, Side& s, const CdSide& a, const HeavyBatch& b
     OK(check_launch(m));
   }
   for (int fb = 0; fb <= nblocks; fb++) {
-    if (fb == nblocks && !a.pc_out.n) break;   // last cache update: only when the symmetric cache keeps the result
+    if (fb == nblocks && !a.pc_out) break;   // last cache update: only when the symmetric cache keeps the result
     step<<<nu, s.slab, step_smem, m->stream>>>(a, hu, b.u0, fb, nblocks, s.pred, s.delta, part);
     OK(check_launch(m));
     if (fb == nblocks) break;
@@ -1168,64 +1172,56 @@ int launch_cd(eals_model* m, Side& s, const CdSide& a, int only_row, bool timed)
   return EALS_OK;
 }
 
-// Launch the routing copy the last sweep left behind: on the side stream (after the sweep's kernels), or on the
-// model's own stream.
+// Launch the copies of the predictions the last sweep staged: on the side stream (after the sweep's kernels),
+// or on the model's own stream.
 int launch_route(eals_model* m, bool on_side_stream) {
   if (!m->route_todo) return EALS_OK;
   const bool user = m->route_todo == 1;
   m->route_todo = 0;
-  static const bool inline_route = getenv("EALS_ROUTE_INLINE") && getenv("EALS_ROUTE_INLINE")[0] == '1';
   const Side& s = user ? m->users : m->items;
-  const eals::PcOut& out = user ? m->out_to_items : m->out_to_users;
+  const PcOut& out = user ? m->out_to_items : m->out_to_users;
   cudaStream_t rs = m->stream;
-  if (on_side_stream && !inline_route) {
+  if (on_side_stream) {
     CU(cudaStreamWaitEvent(m->side_stream, m->ev_swept, 0));
     rs = m->side_stream;
   }
-  if (m->copy_route) {
-    // One peer-to-peer copy per destination rank (copy engines: no SM, runs under the Gram kernel): my segment of
-    // the destination-ordered staging array -> my slot of the destination's receive area.
-    const int me = m->rank, nr = m->n_ranks;
-    const double* stage = user ? m->pc_stage_u : m->pc_stage_i;
-    // side stream + two helpers (round-robin over the destinations) when the copies run beside the Gram
-    cudaStream_t lanes[3] = {rs, rs, rs};
-    static const bool no_fan = getenv("EALS_COPY_FAN") && getenv("EALS_COPY_FAN")[0] == '0';
-    const bool fan = rs != m->stream && nr > 2 && !no_fan;
-    if (fan) {
-      for (int c = 0; c < 2; c++) {
-        if (!m->copy_stream[c]) {
-          CU(cudaStreamCreateWithFlags(&m->copy_stream[c], cudaStreamNonBlocking));
-          CU(cudaEventCreateWithFlags(&m->ev_copied[c], cudaEventDisableTiming));
-        }
-        CU(cudaStreamWaitEvent(m->copy_stream[c], m->ev_swept, 0));
-        lanes[c + 1] = m->copy_stream[c];
+  // One peer-to-peer copy per destination rank (copy engines: no SM, runs under the Gram kernel): my segment of
+  // the destination-ordered staging array -> my slot of the destination's receive area.
+  const int me = m->rank, nr = m->n_ranks;
+  const double* stage = user ? m->pc_stage_u : m->pc_stage_i;
+  // side stream + two helpers (round-robin over the destinations) when the copies run beside the Gram
+  cudaStream_t lanes[3] = {rs, rs, rs};
+  const bool fan = rs != m->stream && nr > 2;
+  if (fan) {
+    for (int c = 0; c < 2; c++) {
+      if (!m->copy_stream[c]) {
+        CU(cudaStreamCreateWithFlags(&m->copy_stream[c], cudaStreamNonBlocking));
+        CU(cudaEventCreateWithFlags(&m->ev_copied[c], cudaEventDisableTiming));
       }
+      CU(cudaStreamWaitEvent(m->copy_stream[c], m->ev_swept, 0));
+      lanes[c + 1] = m->copy_stream[c];
     }
-    int n_copy = 0;
-    long long seg = 0;
-    for (int r = 0; r < nr; r++) {
-      // user sweep: I am the user-owner `me`, destination = item-owner r; item sweep: I am the item-owner, dest = user-owner r
-      const long long cnt = user ? m->pair_cnt[me][r] : m->pair_cnt[r][me];
-      long long off = 0;                                       // senders before me in r's receive area
-      for (int q = 0; q < me; q++) off += user ? m->pair_cnt[q][r] : m->pair_cnt[r][q];
-      const long long dst_n = (long long)out.bound[r + 1] - (long long)out.bound[r];   // values in r's cache
-      if (cnt > 0 && r != me)      // my own segment stays where it is: pc_unpack_kernel reads it from the staging array
-        CU(cudaMemcpyAsync(out.base[r] + recv_offset(dst_n) + off, stage + seg, sizeof(double) * (size_t)cnt, cudaMemcpyDefault,
-                           lanes[n_copy++ % 3]));
-      seg += cnt;
-    }
-    if (fan)                       // the helpers rejoin the side stream: ev_routed below covers all copies
-      for (int c = 0; c < 2; c++) {
-        CU(cudaEventRecord(m->ev_copied[c], m->copy_stream[c]));
-        CU(cudaStreamWaitEvent(m->side_stream, m->ev_copied[c], 0));
-      }
-    if (seg != s.nnz) return fail(EALS_ERR_STATE, "routing table does not cover the staged predictions (%lld of %lld)", seg, (long long)s.nnz);
-    (user ? m->unpack_i_pending : m->unpack_u_pending) = true;      // SPMD: every rank sweeps the same side now
-  } else {
-    const int grid = (int)std::min<int64_t>((s.nnz + 255) / 256, 4 * m->sm_count);
-    eals::pc_route_kernel<<<grid, 256, 0, rs>>>(user ? m->pc_stage_u : m->pc_stage_i, user ? m->route_dst_u : m->route_dst_i, s.nnz, out);
-    OK(check_launch(m));
   }
+  int n_copy = 0;
+  long long seg = 0;
+  for (int r = 0; r < nr; r++) {
+    // user sweep: I am the user-owner `me`, destination = item-owner r; item sweep: I am the item-owner, dest = user-owner r
+    const long long cnt = user ? m->pair_cnt[me][r] : m->pair_cnt[r][me];
+    long long off = 0;                                       // senders before me in r's receive area
+    for (int q = 0; q < me; q++) off += user ? m->pair_cnt[q][r] : m->pair_cnt[r][q];
+    const long long dst_n = (long long)out.bound[r + 1] - (long long)out.bound[r];   // values in r's cache
+    if (cnt > 0 && r != me)      // my own segment stays where it is: pc_unpack_kernel reads it from the staging array
+      CU(cudaMemcpyAsync(out.base[r] + recv_offset(dst_n) + off, stage + seg, sizeof(double) * (size_t)cnt, cudaMemcpyDefault,
+                         lanes[n_copy++ % 3]));
+    seg += cnt;
+  }
+  if (fan)                       // the helpers rejoin the side stream: ev_routed below covers all copies
+    for (int c = 0; c < 2; c++) {
+      CU(cudaEventRecord(m->ev_copied[c], m->copy_stream[c]));
+      CU(cudaStreamWaitEvent(m->side_stream, m->ev_copied[c], 0));
+    }
+  if (seg != s.nnz) return fail(EALS_ERR_STATE, "routing table does not cover the staged predictions (%lld of %lld)", seg, (long long)s.nnz);
+  (user ? m->unpack_i_pending : m->unpack_u_pending) = true;      // SPMD: every rank sweeps the same side now
   if (rs != m->stream) {
     CU(cudaEventRecord(m->ev_routed, m->side_stream));
     m->route_pending = true;
@@ -1286,10 +1282,8 @@ int sweep(eals_model* m, bool user, int only_row) {
   a.row_base = s.row_base;
   a.K = m->K;
   a.reg = m->p.reg;
-  a.pc_in = nullptr; a.pc_map = nullptr; a.pc_out = eals::PcOut{}; a.use_cache = 0; a.pc_stage = nullptr;
+  a.pc_in = nullptr; a.pc_map = nullptr; a.pc_out = nullptr; a.use_cache = 0;
   a.peers = user ? m->peersU : m->peersV;
-  static const bool fence = getenv("EALS_PEER_FENCE") && getenv("EALS_PEER_FENCE")[0] == '1';
-  a.fence = fence ? 1 : 0;   // off by default: grid completion already orders the peer stores (cd_sweep.cuh, peers_release)
   if (only_row >= 0) {
     m->pc_u_valid = m->pc_i_valid = false;   // a single-row update changes factors behind the cache's back
     if (user) m->su_fresh = false;           // ... and U behind SU's back (MF_fastALS.cpp:243-322 never touches SU)
@@ -1298,11 +1292,12 @@ int sweep(eals_model* m, bool user, int only_row) {
     bool& out_valid = user ? m->pc_i_valid : m->pc_u_valid;
     if (m->pred_refresh_every > 0 && m->sweeps_since_fresh >= m->pred_refresh_every) in_valid = false;
     a.pc_in = user ? m->pc_u : m->pc_i;
-    a.pc_map = user ? m->map_u : m->map_i;
-    a.pc_out = user ? m->out_to_items : m->out_to_users;
     if (m->routed) {     // staged: the map is the slot in destination order (build_routes)
-      a.pc_stage = user ? m->pc_stage_u : m->pc_stage_i;
+      a.pc_out = user ? m->pc_stage_u : m->pc_stage_i;
       a.pc_map = user ? m->route_src_u : m->route_src_i;
+    } else {             // one rank: straight into the other orientation's cache
+      a.pc_out = user ? m->pc_i : m->pc_u;
+      a.pc_map = user ? m->map_u : m->map_i;
     }
     a.use_cache = in_valid ? 1 : 0;
     m->sweeps_since_fresh = in_valid ? m->sweeps_since_fresh + 1 : 0;
@@ -1311,12 +1306,12 @@ int sweep(eals_model* m, bool user, int only_row) {
   }
   if (user) { DISPATCH_LD(m->LD, OK((launch_cd<LD, true>(m, s, a, only_row, true)))); }
   else      { DISPATCH_LD(m->LD, OK((launch_cd<LD, false>(m, s, a, only_row, true)))); }
-  if (a.pc_stage && s.nnz > 0) {
+  if (m->routed && a.pc_out && s.nnz > 0) {
     // Second phase: staged predictions to their owners, in destination order.  Nobody needs them before the
-    // NEXT half-epoch's sweep, so the copy is launched by gram() on a side stream right behind the Gram's main
-    // kernel (a small persistent grid that shares the SMs with it) and joined before gram() returns — i.e.
-    // before the all-reduce that orders the ranks.  Round 1 had it on the sweep's stream: 7 % of the step at
-    // 2 GPUs.  A caller that never calls gram() gets it inline at the next sweep / sync (join_route).
+    // NEXT half-epoch's sweep, so the copies are issued by gram() on a side stream right behind the Gram's main
+    // kernel and joined before gram() returns — i.e. before the all-reduce that orders the ranks.  Round 1
+    // routed on the sweep's stream: 7 % of the step at 2 GPUs.  A caller that never calls gram() gets the copies
+    // on the model's stream at the next sweep / sync (join_route).
     if (!m->side_stream) {
       CU(cudaStreamCreateWithFlags(&m->side_stream, cudaStreamNonBlocking));
       CU(cudaEventCreateWithFlags(&m->ev_swept, cudaEventDisableTiming));
@@ -1542,7 +1537,7 @@ int eals_destroy(eals_model* m) {
   cudaFree(m->terms); cudaFree(m->partials); cudaFree(m->flags); cudaFree(m->S_tmp);
   cudaFree(m->pc_u); cudaFree(m->pc_i); cudaFree(m->map_u); cudaFree(m->map_i);
   cudaFree(m->pc_stage_u); cudaFree(m->pc_stage_i);
-  cudaFree(m->route_src_u); cudaFree(m->route_dst_u); cudaFree(m->route_src_i); cudaFree(m->route_dst_i);
+  cudaFree(m->route_src_u); cudaFree(m->route_src_i);
   cudaFree(m->recv_idx_u); cudaFree(m->recv_idx_i);
   for (void* p : m->graveyard) cudaFree(p);
   delete m->eval;
@@ -2148,7 +2143,7 @@ int eals_ipc_attach(eals_model* m, int32_t which, int32_t n_peers, const void* h
     if (!m->pcache_on) return fail(EALS_ERR_STATE, "prediction cache is off on this model");
     if (m->n_ranks < 2 || n_peers != m->n_ranks - 1)
       return fail(EALS_ERR_ARG, "prediction caches need eals_params.n_ranks - 1 = %d peer handles, got %d", m->n_ranks - 1, n_peers);
-    eals::PcOut& out = which == EALS_BUF_PC_USER ? m->out_to_users : m->out_to_items;
+    PcOut& out = which == EALS_BUF_PC_USER ? m->out_to_users : m->out_to_items;
     bool& flag = which == EALS_BUF_PC_USER ? m->pc_users_attached : m->pc_items_attached;
     close_pc_peers(m, out, flag);
     int p = 0;

@@ -422,9 +422,8 @@ class MF_fastALS:
             return
         dev = f"cuda:{self.device}"
         shared = [_lib.BUF_U, _lib.BUF_V] if factors else []
-        # The prediction caches are shared across ranks too: a sweep stages its final predictions locally
-        # and a second kernel routes them to their owners in destination order (EALS_PC_ROUTE=0: scattered
-        # 8-byte peer stores straight from the sweep kernels, measured 4x slower on the item side, r01f).
+        # The prediction caches are shared across ranks too: a sweep stages its final predictions locally in
+        # destination order and peer-to-peer copies move each destination's segment into that rank's receive area.
         pc = os.environ.get("EALS_PEER_PRED_CACHE", "1") == "1" and self._pred_cache_everywhere()
         if pc:
             shared += [_lib.BUF_PC_USER, _lib.BUF_PC_ITEM]
