@@ -81,6 +81,7 @@ SIGNATURES = {
     "eals_recommend_stats": (C.c_int, [_P, _P]),
     "eals_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "eals_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    "eals_similar": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int32, _P, _P]),
     "eals_ranking_metrics": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "eals_leading_dim": (C.c_int, [_P]),
     "eals_device_buffer": (C.c_int, [_P, C.c_int32, C.POINTER(_P), C.POINTER(C.c_int64)]),
@@ -125,6 +126,7 @@ SIGNATURES = {
     "eals_group_recommend": (C.c_int, [_P, C.c_int32, C.c_int32, _P, C.c_int32, C.c_int32, _P, _P]),
     "eals_group_fold_in": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, _P, C.c_int32, _P]),
     "eals_group_recommend_vectors": (C.c_int, [_P, C.c_int32, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    "eals_group_similar": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_int32, _P, C.c_int32, _P, _P]),
     "eals_group_ranking_metrics": (C.c_int, [_P, C.c_int32, _P, _P, C.c_int32, C.c_int32, _P, _P, _P, _P]),
     "eals_group_sync": (C.c_int, [_P]),
     "eals_group_replicas_consistent": (C.c_int, [_P, C.POINTER(C.c_int32)]),

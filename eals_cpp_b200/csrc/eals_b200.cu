@@ -2033,6 +2033,11 @@ int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double
   return recommend_vectors_impl(m, space, n, Q, ex_ptr, ex_idx, k, items, scores);
 }
 
+int eals_similar(eals_model* m, int32_t which, int32_t space, int32_t n, const int32_t* ids, int32_t k, int32_t* out_ids,
+                 double* scores) {
+  return similar_impl(m, which, space, n, ids, k, out_ids, scores);
+}
+
 int eals_ranking_metrics(eals_model* m, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
                          int32_t exclude_seen, double sums[6], int64_t* n_users, double* per_user, int32_t* ranks) {
   return ranking_metrics_impl(m, space, test_ptr, test_idx, k, exclude_seen, sums, n_users, per_user, ranks);

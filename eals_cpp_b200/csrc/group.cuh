@@ -583,6 +583,25 @@ int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const 
   return EALS_OK;
 }
 
+int eals_group_similar(eals_group* g, int32_t which, int32_t space, int32_t n, const int32_t* ids, int32_t k, int32_t* out_ids,
+                       double* scores) {
+  if (!g || (n > 0 && (!ids || !out_ids))) return fail(EALS_ERR_ARG, "null argument");
+  if (which != EALS_BUF_U && which != EALS_BUF_V) return fail(EALS_ERR_ARG, "which must be EALS_BUF_U or EALS_BUF_V");
+  OK(check_topk_args(space, n, k));
+  OK(group_barrier(g));
+  if (n == 0) return EALS_OK;
+  std::vector<int32_t> id_buf, out_i((size_t)n * k);
+  std::vector<double> out_s((size_t)n * k);
+  const int32_t* hid = nullptr;
+  OK(host_view(space, ids, (size_t)n, id_buf, &hid));
+  OK(group_slices(g, n, [&](int q, int lo, int hi) {
+    return eals_similar(g->r[q], which, EALS_HOST, hi - lo, hid + lo, k, out_i.data() + (size_t)lo * k, out_s.data() + (size_t)lo * k);
+  }));
+  OK(host_result(space, out_ids, out_i));
+  if (scores) OK(host_result(space, scores, out_s));
+  return EALS_OK;
+}
+
 // Every rank ranks the test entries of the rows it owns (its train rows are the ones to exclude), the ranks at once;
 // the sums are added in rank order.
 int eals_group_ranking_metrics(eals_group* g, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,

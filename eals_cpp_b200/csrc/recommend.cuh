@@ -255,6 +255,51 @@ __global__ void rec_keep_flags_kernel(const int32_t* __restrict__ list, const in
   flags[p] = f;
 }
 
+// Cosine catalogue of similar(): out[r] = Y[r] / |Y[r]| for the rows [0, rows) of Y [rows][LD], with
+// |y| = __dsqrt_rn(seq_dot(y, y)) and one __ddiv_rn per factor, so the normalised rows are defined bit for bit.  A row
+// of norm 0 stays zero; the padding columns [K, LD) are written as zeros.  One warp per row: the row is read as
+// coalesced 256-byte pieces (LD <= kMaxFactors, so at most 8 per lane stay in registers) and its squares are added
+// in factor order through shuffles, every lane holding the same sum.
+__global__ void sim_normalize_kernel(const double* __restrict__ Y, int rows, int K, int LD, double* __restrict__ out) {
+  const int lane = threadIdx.x & 31;
+  const long long warps = ((long long)gridDim.x * blockDim.x) >> 5;
+  for (long long r = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; r < rows; r += warps) {
+    const double* y = Y + (size_t)r * LD;
+    double v[kMaxFactors / 32];
+    double acc = 0.0;
+#pragma unroll
+    for (int c = 0; c < kMaxFactors / 32; c++) {
+      const int k0 = c * 32;
+      v[c] = 0.0;
+      if (k0 < K) {
+        if (k0 + lane < K) v[c] = y[k0 + lane];
+        const double p = __dmul_rn(v[c], v[c]);
+        const int kend = min(32, K - k0);
+        for (int j = 0; j < kend; j++) acc = __dadd_rn(acc, __shfl_sync(kFullMask, p, j));
+      }
+    }
+    const double norm = __dsqrt_rn(acc);
+    double* o = out + (size_t)r * LD;
+#pragma unroll
+    for (int c = 0; c < kMaxFactors / 32; c++) {
+      const int k = c * 32 + lane;
+      if (k < LD) o[k] = k < K && norm != 0.0 ? __ddiv_rn(v[c], norm) : 0.0;
+    }
+  }
+}
+
+// The query rows of similar() and their self-exclusion CSR: qx[s] = Yhat[ids[s]] ([n][LD]) and ex_ptr[s] = s for
+// s <= n, so that row s of the CSR over the index array `ids` is the query's own id and nothing else.
+__global__ void sim_queries_kernel(const double* __restrict__ Yhat, int LD, const int32_t* __restrict__ ids, int n,
+                                   double* __restrict__ qx, int64_t* __restrict__ ex_ptr) {
+  const size_t total = (size_t)n * LD;   // >= n + 1 (LD >= 16, n >= 1)
+  for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+    const size_t s = t / LD;
+    qx[t] = Yhat[(size_t)ids[s] * LD + t % LD];
+    if (t <= (size_t)n) ex_ptr[t] = (int64_t)t;
+  }
+}
+
 // flags[p] = 1 when slot p's list is not full yet (the seed has to be extended for it)
 __global__ void rec_unfilled_flags_kernel(const int32_t* __restrict__ list, const int32_t* __restrict__ n_list, int n_max,
                                           const double* __restrict__ thr, uint8_t* __restrict__ flags) {

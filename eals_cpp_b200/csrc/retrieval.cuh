@@ -141,6 +141,9 @@ struct eals_eval_ws {
   Side hist, excl;
   WsBuf<int> hist_check, excl_check;
   WsBuf<double> qx;
+  // similar: the normalised catalogue [n_Y][LD] and the offsets of the self-exclusion CSR (its index array is ws.users)
+  WsBuf<double> yhat;
+  WsBuf<int64_t> self_ptr;
   // ranking metrics: the owned rows of the test matrix (validated by build_side, row_base = the first owned user),
   // per entry its rank, per slot c_R and the certain-count limit, the chunk's train scores, the per-user metrics
   // and the gain / ideal-DCG tables
@@ -414,13 +417,15 @@ int compact_list(eals_model* m, WorkList& wl, int n, int32_t* d_n) {
 }
 
 // Preparation of the tcgen05 filter for the rows X[d_rows[0 .. n)] (d_rows nullable: X[0 .. n); evaluate and
-// recommend): fp16 copies of V in decreasing-norm order (ws.perm: rank -> item) and of the query rows, their norms,
-// the per-tile item norms and the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).
-// The item half (once per call of ranking_metrics, which prepares several chunks of rows against it) ...
-int tc_prepare_items(eals_model* m) {
+// recommend) against the catalogue Y [N][LD] (V, or a normalised U / V for similar): fp16 copies of Y in
+// decreasing-norm order (ws.perm: rank -> row of Y) and of the query rows, their norms, the per-tile catalogue norms
+// and the per-slot thresholds from `d_thr` (the exact gt score, or a user's k-th score).  Every call prepares its
+// catalogue again, so nothing of one catalogue carries over to a call on another.
+// The catalogue half (once per call of ranking_metrics, which prepares several chunks of rows against it) ...
+int tc_prepare_items(eals_model* m, const double* Y, int N) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
-  const int K = m->K, LD = m->LD, N = m->N;
+  const int K = m->K, LD = m->LD;
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
   cudaStream_t st = m->stream;
@@ -431,15 +436,15 @@ int tc_prepare_items(eals_model* m) {
   OK(ws.tile_norm.reserve((size_t)n_tiles));
   unsigned long long* d_vmax = ws.counters.p;
   CU(cudaMemsetAsync(ws.counters.p, 0, 4 * sizeof(unsigned long long), st));
-  tc::absmax_kernel<<<4 * m->sm_count, 256, 0, st>>>(m->V, (size_t)N, K, LD, d_vmax);
+  tc::absmax_kernel<<<4 * m->sm_count, 256, 0, st>>>(Y, (size_t)N, K, LD, d_vmax);
   OK(check_launch(m));
-  tc::item_sort_keys_kernel<<<(unsigned)(((size_t)N * 32 + 255) / 256), 256, 0, st>>>(m->V, K, LD, N, ws.keys.p, ws.ids.p);
+  tc::item_sort_keys_kernel<<<(unsigned)(((size_t)N * 32 + 255) / 256), 256, 0, st>>>(Y, K, LD, N, ws.keys.p, ws.ids.p);
   OK(check_launch(m));
   OK(cub_call(m, "item norm sort", [&](void* tmp, size_t& bytes) {
     return cub::DeviceRadixSort::SortPairs(tmp, bytes, ws.keys.p, ws.keys_out.p, ws.ids.p, ws.perm.p, N, 0, 32, st); }));
   {
     tc::PrepOut o{ws.Vh.p, ws.vn_hat.p, ws.vn_del.p, ws.vn_h.p, nullptr};
-    tc::prep_rows_kernel<false><<<(unsigned)(((size_t)N * 32 + 255) / 256), 256, 0, st>>>(m->V, K, LD, KP, N, ws.perm.p, 0, d_vmax, o);
+    tc::prep_rows_kernel<false><<<(unsigned)(((size_t)N * 32 + 255) / 256), 256, 0, st>>>(Y, K, LD, KP, N, ws.perm.p, 0, d_vmax, o);
     OK(check_launch(m));
     tc::tile_norm_kernel<<<n_tiles, 32, 0, st>>>(ws.vn_h.p, ws.vn_del.p, N, n_tiles, ws.tile_norm.p);
     OK(check_launch(m));
@@ -472,8 +477,8 @@ int tc_prepare_rows(eals_model* m, int n, const double* X, const int32_t* d_rows
   return EALS_OK;
 }
 
-int tc_prepare(eals_model* m, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
-  OK(tc_prepare_items(m));
+int tc_prepare(eals_model* m, const double* Y, int N, int n, const double* X, const int32_t* d_rows, const double* d_thr) {
+  OK(tc_prepare_items(m, Y, N));
   return tc_prepare_rows(m, n, X, d_rows, d_thr);
 }
 
@@ -576,7 +581,7 @@ int scan_tc(eals_model* m, int n, const int32_t* d_users, const double* d_gts, i
   StageTimer tm;
   const int K = m->K, LD = m->LD;
   cudaStream_t st = m->stream;
-  OK(tc_prepare(m, n, m->U, d_users, d_gts));
+  OK(tc_prepare(m, m->V, m->N, n, m->U, d_users, d_gts));
   tm.lap("eval: fp16 copies, norms, item order");
   // a user is decided once its certain count exceeds topK (limit topK + 1, kept from overflowing); the candidates
   // go through MODE 1, which also emits the pairs whose truncated key may be non-zero
@@ -704,16 +709,19 @@ int evaluate_slots(eals_model* m, const std::vector<int32_t>& users_h, const int
 // ---- top-k retrieval (recommend.cuh) --------------------------------------------------------------------
 namespace rec = eals::rec;
 
-// What the engines answer: slot s asks for the top-k of row rows[s] of X (rows nullable: row s), its excluded items
-// being row (that row - ex_base) of the CSR ex_ptr / ex_idx (ex_ptr nullable: none).  recommend: the model's U, the
-// users, the owned train rows; recommend_vectors: the query vectors copied to [n][LD], the identity, the caller's
-// exclusion lists.
+// What the engines answer: slot s asks for the top-k rows of the catalogue Y [nY][LD] for row rows[s] of X (rows
+// nullable: row s), its excluded catalogue rows being row (that row - ex_base) of the CSR ex_ptr / ex_idx (ex_ptr
+// nullable: none).  recommend: the model's U, the users, the owned train rows, catalogue V; recommend_vectors: the
+// query vectors copied to [n][LD], the identity, the caller's exclusion lists, catalogue V; similar: the normalised
+// query rows copied to [n][LD], the identity, each query's own id, the normalised U or V.
 struct RecQuery {
   const double* X;
   const int32_t* rows;
   const int64_t* ex_ptr;
   const int32_t* ex_idx;
   int ex_base;
+  const double* Y;
+  int nY;
   RecQuery from(int s0, int LD) const {   // the same query for the slots s0 ..
     RecQuery q = *this;
     if (rows) q.rows += s0;
@@ -725,7 +733,7 @@ struct RecQuery {
 rec::MergeArgs rec_args(eals_model* m, const RecQuery& q, int k) {
   eals_eval_ws& ws = eval_ws(m);
   rec::MergeArgs a{};
-  a.U = q.X; a.V = m->V; a.K = m->K; a.LD = m->LD; a.users = q.rows; a.k = k;
+  a.U = q.X; a.V = q.Y; a.K = m->K; a.LD = m->LD; a.users = q.rows; a.k = k;
   a.top_s = ws.top_s.p; a.top_i = ws.top_i.p; a.thr = ws.thr.p;
   a.ptr = q.ex_ptr; a.idx = q.ex_idx; a.row_base = q.ex_base;
   return a;
@@ -749,7 +757,7 @@ int rec_merge_exact(eals_model* m, rec::MergeArgs a, const int32_t* list, int n_
 // (EALS_EVAL_SCALAR=1) and its fall-back.
 int rec_exact(eals_model* m, int n, const RecQuery& q, int k) {
   OK(rec_reset(m, n, k));
-  return rec_merge_exact(m, rec_args(m, q, k), nullptr, n, nullptr, 0, m->N);
+  return rec_merge_exact(m, rec_args(m, q, k), nullptr, n, nullptr, 0, q.nY);
 }
 
 // Engine 2: tcgen05 filter.  Seed: the highest-norm items scored exactly (extended tile by tile for users whose
@@ -761,13 +769,13 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
   namespace tc = eals::tc;
   eals_eval_ws& ws = eval_ws(m);
   StageTimer tm;
-  const int K = m->K, N = m->N;
+  const int K = m->K, N = q.nY;
   const int nkc = (K + tc::kKC - 1) / tc::kKC, KP = nkc * tc::kKC;
   const int n_tiles = (N + tc::kTN - 1) / tc::kTN;
   const int ut = nkc <= 2 ? 2 : 1;
   cudaStream_t st = m->stream;
   OK(rec_reset(m, n, k));
-  OK(tc_prepare(m, n, q.X, q.rows, ws.thr.p));
+  OK(tc_prepare(m, q.Y, N, n, q.X, q.rows, ws.thr.p));
   const double gamma = (double)KP * (1.0 / 2097152.0);
   auto params = [&]() -> int {   // per-slot filter thresholds from the current k-th scores
     tc::slot_params_kernel<<<(n + 255) / 256, 256, 0, st>>>(ws.thr.p, ws.exps.p, ws.counters.p, ws.un_hat.p, ws.un_del.p, ws.un_h.p, n,
@@ -864,7 +872,7 @@ int rec_tc(eals_model* m, int n, const RecQuery& q, int k, RecStats& stats) {
         OK(ws.pscore.reserve((size_t)got)); OK(ws.pkey.reserve((size_t)got)); OK(ws.pkey_out.reserve((size_t)got));
         OK(ws.pval.reserve((size_t)got)); OK(ws.pval_out.reserve((size_t)got));
         OK(ws.run_slot.reserve((size_t)got)); OK(ws.run_cnt.reserve((size_t)got)); OK(ws.run_off.reserve((size_t)got));
-        rec::rec_rescore_kernel<tc::EvalPair><<<16 * m->sm_count, 128, 0, st>>>(q.X, m->V, K, m->LD, q.rows, ws.pairs.p, got,
+        rec::rec_rescore_kernel<tc::EvalPair><<<16 * m->sm_count, 128, 0, st>>>(q.X, q.Y, K, m->LD, q.rows, ws.pairs.p, got,
                                                                                ws.pscore.p, ws.pkey.p, ws.pval.p);
         OK(check_launch(m));
         const int ng = (int)got, end_bit = slot_bits(n);
@@ -960,6 +968,24 @@ int rec_check_args(eals_model* m, int space, int n, int k) {
   return EALS_OK;
 }
 
+// The first position of the device ids d_ids[0 .. n) outside [lo, hi) -> *pos and its id -> *id; *pos = -1 when every
+// id is inside.  Synchronises.
+int find_outside(eals_model* m, const int32_t* d_ids, int n, int lo, int hi, int* pos, int* id) {
+  const int none = 0x7fffffff;
+  int bad = none;
+  CU(cudaMemcpyAsync(m->flags, &none, sizeof(int), cudaMemcpyHostToDevice, m->stream));
+  rec::rec_check_users_kernel<<<(n + 255) / 256, 256, 0, m->stream>>>(d_ids, n, lo, hi, m->flags);
+  OK(check_launch(m));
+  CU(cudaMemcpyAsync(&bad, m->flags, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
+  CU(cudaStreamSynchronize(m->stream));
+  *pos = -1;
+  if (bad != none) {
+    *pos = bad - 1;
+    CU(cudaMemcpy(id, d_ids + (bad - 1), sizeof(int), cudaMemcpyDeviceToHost));
+  }
+  return EALS_OK;
+}
+
 int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k, int exclude, int32_t* items, double* scores) {
   if (!m || (n > 0 && (!users || !items))) return fail(EALS_ERR_ARG, "null argument");
   OK(rec_check_args(m, space, n, k));
@@ -975,21 +1001,14 @@ int recommend_impl(eals_model* m, int space, int n, const int32_t* users, int k,
   OK(ws.users.reserve((size_t)n));
   OK(copy_in(ws.users.p, users, (size_t)n, space, m->stream));
   if (space == EALS_DEVICE) {
-    const int none = 0x7fffffff;
-    int bad = none;
-    CU(cudaMemcpyAsync(m->flags, &none, sizeof(int), cudaMemcpyHostToDevice, m->stream));
-    rec::rec_check_users_kernel<<<(n + 255) / 256, 256, 0, m->stream>>>(ws.users.p, n, m->ub, m->ue, m->flags);
-    OK(check_launch(m));
-    CU(cudaMemcpyAsync(&bad, m->flags, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
-    CU(cudaStreamSynchronize(m->stream));
-    if (bad != none) {
-      int u = 0;
-      CU(cudaMemcpy(&u, ws.users.p + (bad - 1), sizeof(int), cudaMemcpyDeviceToHost));
-      if (u < 0 || u >= m->M) return fail(EALS_ERR_ARG, "user %d (position %d) outside [0, %d)", u, bad - 1, m->M);
-      return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", u, bad - 1, m->ub, m->ue);
+    int pos = -1, u = 0;
+    OK(find_outside(m, ws.users.p, n, m->ub, m->ue, &pos, &u));
+    if (pos >= 0) {
+      if (u < 0 || u >= m->M) return fail(EALS_ERR_ARG, "user %d (position %d) outside [0, %d)", u, pos, m->M);
+      return fail(EALS_ERR_ARG, "user %d (position %d) outside this model's users [%d, %d)", u, pos, m->ub, m->ue);
     }
   }
-  RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0};
+  RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0, m->V, m->N};
   if (exclude) { q.ex_ptr = m->users.ptr; q.ex_idx = m->users.idx; q.ex_base = m->users.row_base; }
   return rec_answer(m, space, n, q, k, items, scores);
 }
@@ -1061,11 +1080,51 @@ int recommend_vectors_impl(eals_model* m, int space, int n, const double* Q, con
   CU(cudaMemcpyAsync(&bad, m->flags, sizeof(int), cudaMemcpyDeviceToHost, m->stream));
   CU(cudaStreamSynchronize(m->stream));
   if (bad != none) return fail(EALS_ERR_ARG, "query row %d has a non-finite entry", bad - 1);
-  RecQuery q{ws.qx.p, nullptr, nullptr, nullptr, 0};
+  RecQuery q{ws.qx.p, nullptr, nullptr, nullptr, 0, m->V, m->N};
   if (ex_ptr) { q.ex_ptr = ws.excl.ptr; q.ex_idx = ws.excl.idx; }
   return rec_answer(m, space, n, q, k, items, scores);
 }
 
+// ---- similar items and similar users (DESIGN.md §3.8) ------------------------------------------------------------
+
+// For each id q of the catalogue Y (which = EALS_BUF_V: V, the items; EALS_BUF_U: U, the users) the k rows r != q of
+// highest cosine score seq_dot(Yhat[q], Yhat[r]), Yhat = Y with every row normalised (sim_normalize_kernel).  That is
+// recommend_vectors on the normalised catalogue with the normalised query rows and each query's own row as its one
+// excluded entry: the same engines, order, padding, limits, chunking and fall-backs.  U and V are replicated, so any
+// id in [0, n_Y) may be asked for on any rank.
+int similar_impl(eals_model* m, int which, int space, int n, const int32_t* ids, int k, int32_t* out_ids, double* scores) {
+  if (!m || (n > 0 && (!ids || !out_ids))) return fail(EALS_ERR_ARG, "null argument");
+  if (which != EALS_BUF_U && which != EALS_BUF_V) return fail(EALS_ERR_ARG, "which must be EALS_BUF_U or EALS_BUF_V");
+  OK(rec_check_args(m, space, n, k));
+  CU(cudaSetDevice(m->p.device));
+  if (n == 0) return EALS_OK;
+  const bool users = which == EALS_BUF_U;
+  const double* Y = users ? m->U : m->V;
+  const int nY = users ? m->M : m->N, LD = m->LD;
+  const char* what = users ? "user" : "item";
+  if (space == EALS_HOST)
+    for (int s = 0; s < n; s++)
+      if (ids[s] < 0 || ids[s] >= nY) return fail(EALS_ERR_ARG, "%s %d (position %d) outside [0, %d)", what, ids[s], s, nY);
+  eals_eval_ws& ws = eval_ws(m);
+  OK(ws.users.reserve((size_t)n));
+  OK(copy_in(ws.users.p, ids, (size_t)n, space, m->stream));
+  if (space == EALS_DEVICE) {
+    int pos = -1, id = 0;
+    OK(find_outside(m, ws.users.p, n, 0, nY, &pos, &id));
+    if (pos >= 0) return fail(EALS_ERR_ARG, "%s %d (position %d) outside [0, %d)", what, id, pos, nY);
+  }
+  OK(ws.yhat.reserve((size_t)nY * LD));
+  OK(ws.qx.reserve((size_t)n * LD));
+  OK(ws.self_ptr.reserve((size_t)n + 1));
+  rec::sim_normalize_kernel<<<(unsigned)std::min<size_t>(((size_t)nY * 32 + 255) / 256, 64 * (size_t)m->sm_count), 256, 0, m->stream>>>(
+      Y, nY, m->K, LD, ws.yhat.p);
+  OK(check_launch(m));
+  rec::sim_queries_kernel<<<(unsigned)std::min<size_t>(((size_t)n * LD + 255) / 256, 8 * (size_t)m->sm_count), 256, 0, m->stream>>>(
+      ws.yhat.p, LD, ws.users.p, n, ws.qx.p, ws.self_ptr.p);
+  OK(check_launch(m));
+  const RecQuery q{ws.qx.p, nullptr, ws.self_ptr.p, ws.users.p, 0, ws.yhat.p, nY};
+  return rec_answer(m, space, n, q, k, out_ids, scores);
+}
 
 // ---- ranking metrics on a held-out test matrix (ranking.cuh, DESIGN.md §3.7) ------------------------------------
 namespace rk = eals::rk;
@@ -1136,7 +1195,7 @@ int rm_chunk_exact(eals_model* m, int r0, int r1, int k, bool exclude, int32_t* 
     OK(ws.users.reserve((size_t)nd));
     OK(ws.top_s.reserve((size_t)nd * k)); OK(ws.top_i.reserve((size_t)nd * k)); OK(ws.thr.reserve((size_t)nd));
     CU(cudaMemcpyAsync(ws.users.p, users.data() + d0, sizeof(int32_t) * nd, cudaMemcpyHostToDevice, m->stream));
-    RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0};
+    RecQuery q{m->U, ws.users.p, nullptr, nullptr, 0, m->V, m->N};
     if (exclude) { q.ex_ptr = m->users.ptr; q.ex_idx = m->users.idx; q.ex_base = m->users.row_base; }
     OK(rec_exact(m, nd, q, k));
     rk::rm_lookup_kernel<<<(unsigned)(((size_t)nd * k + 255) / 256), 256, 0, m->stream>>>(ws.top_i.p, k, nd, ws.users.p, m->ub, T.ptr,
@@ -1184,7 +1243,7 @@ int ranking_metrics_impl(eals_model* m, int space, const int64_t* test_ptr, cons
       EvalStats c;
       bool done = false;
       if (use_tc_engine(m, (int)n)) {   // n <= max(2^28, one row of at most N items)
-        if (!items_ready) OK(tc_prepare_items(m));
+        if (!items_ready) OK(tc_prepare_items(m, m->V, m->N));
         items_ready = true;
         OK(rm_chunk_tc(m, r0, r1, k, exclude, !any, ws.ranks.p + e0, c, done));
       }

@@ -13,6 +13,7 @@
 //   eals_main [--data yelp.rating] [--factors 64] [--iters 20] [--w0 10] [--alpha 0.75] [--reg 0.01]
 //             [--topk 10] [--no-loss] [--exact-eval] [--device 0] [--gpus N | --devices 0,1,..] [--online U,I]
 //             [--save FILE] [--load FILE] [--recommend K [--recommend-out FILE]]
+//             [--similar-items K [--similar-out FILE]]
 // --gpus N: shard users and items over GPUs device .. device+N-1 (eals_group: the exchange runs inside the
 // library); --devices lists them explicitly — a repeated id puts several ranks on one GPU.
 // --save / --load: factor checkpoint after training / instead of the random initialisation.
@@ -20,6 +21,8 @@
 // the model is built — needs no GPU; the loader is checked against the reference's own binary this way.
 // --recommend K: after training and evaluation, every user's top-K unseen items, one line "user item score" per
 // recommended item (score with %.17g), to --recommend-out FILE (default: stdout).
+// --similar-items K: after training and evaluation, every item's K most similar items (cosine), one line
+// "item similar score" per listed item (score with %.17g), to --similar-out FILE (default: stdout).
 // --online U,I: after training and evaluation, add the interaction (U, I) with the online update
 // (updateModel, MF_fastALS.cpp:223-242) and print the prediction before and after.
 #include <algorithm>
@@ -49,8 +52,8 @@ int main(int argc, char** argv) {
   bool showProgress = false, showLoss = true, exact = false;
   int online_u = -1, online_i = -1, n_gpus = 1;
   std::vector<int> devices;
-  std::string save_path, load_path, dump_split, recommend_out;
-  int recommend_k = 0;
+  std::string save_path, load_path, dump_split, recommend_out, similar_out;
+  int recommend_k = 0, similar_k = 0;
   for (int a = 1; a < argc; a++) {
     auto is = [&](const char* f) { return std::strcmp(argv[a], f) == 0; };
     auto next = [&]() -> const char* { if (a + 1 >= argc) { std::fprintf(stderr, "missing value after %s\n", argv[a]); std::exit(2); } return argv[++a]; };
@@ -69,6 +72,8 @@ int main(int argc, char** argv) {
     else if (is("--dump-split")) dump_split = next();
     else if (is("--recommend")) recommend_k = std::atoi(next());
     else if (is("--recommend-out")) recommend_out = next();
+    else if (is("--similar-items")) similar_k = std::atoi(next());
+    else if (is("--similar-out")) similar_out = next();
     else if (is("--no-loss")) showLoss = false;
     else if (is("--exact-eval")) exact = true;
     else if (is("--online")) { if (std::sscanf(next(), "%d,%d", &online_u, &online_i) != 2) { std::fprintf(stderr, "--online wants U,I\n"); return 2; } }
@@ -155,6 +160,19 @@ int main(int argc, char** argv) {
           if (rec.items[q] >= 0) std::fprintf(f, "%d %d %.17g\n", u, rec.items[q], rec.scores[q]);
         }
       if (f != stdout && std::fclose(f) != 0) { std::fprintf(stderr, "Error: writing %s failed\n", recommend_out.c_str()); return EXIT_FAILURE; }
+    }
+    if (similar_k > 0) {
+      std::vector<int> all((size_t)itemCount);
+      for (int i = 0; i < itemCount; i++) all[(size_t)i] = i;
+      const auto sim = fals.similar_items(all, similar_k);
+      FILE* f = similar_out.empty() ? stdout : std::fopen(similar_out.c_str(), "w");
+      if (!f) { std::fprintf(stderr, "Error: cannot write %s\n", similar_out.c_str()); return EXIT_FAILURE; }
+      for (int i = 0; i < itemCount; i++)
+        for (int j = 0; j < similar_k; j++) {
+          const size_t q = (size_t)i * similar_k + j;
+          if (sim.items[q] >= 0) std::fprintf(f, "%d %d %.17g\n", i, sim.items[q], sim.scores[q]);
+        }
+      if (f != stdout && std::fclose(f) != 0) { std::fprintf(stderr, "Error: writing %s failed\n", similar_out.c_str()); return EXIT_FAILURE; }
     }
     if (online_u >= 0) {
       const double before = fals.predict(online_u, online_i);

@@ -287,6 +287,28 @@ def _recommend_vectors_call(fn, handle, factors, device, Q, k, exclude):
     return (items, scores) if isinstance(items, np.ndarray) else (items.cpu().numpy(), scores.cpu().numpy())
 
 
+def _similar_call(fn, handle, which, device, ids, k):
+    """One eals_similar / eals_group_similar call over the catalogue ``which`` (_lib.BUF_V items, _lib.BUF_U users);
+    ``ids``: a sequence, a numpy array or a torch tensor (a CUDA tensor is read on the device).  Returns (ids, scores)
+    on the host."""
+    k = int(k)
+    if not hasattr(ids, "shape"):
+        ids = np.asarray(ids, np.int32)
+    ids = ids.reshape(-1)
+    n = _rows(ids)
+    space, (q,) = _same_space([(ids, np.int32)], device)
+    shape = (max(n, 1), max(k, 1))
+    if space == _lib.EALS_DEVICE:
+        import torch
+        out_i = torch.empty(shape, dtype=torch.int32, device=device)
+        out_s = torch.empty(shape, dtype=torch.float64, device=device)
+    else:
+        out_i, out_s = np.empty(shape, np.int32), np.empty(shape, np.float64)
+    check(fn(handle, which, space, n, _ptr(q), k, _ptr(out_i), _ptr(out_s)))
+    out_i, out_s = out_i[:n], out_s[:n]
+    return (out_i, out_s) if isinstance(out_i, np.ndarray) else (out_i.cpu().numpy(), out_s.cpu().numpy())
+
+
 RANKING_METRICS = ("hit_rate", "precision", "recall", "ndcg", "map", "mrr")
 
 
@@ -976,6 +998,29 @@ class MF_fastALS:
         return tuple(self._collective_slices(len(q), run, [((max(k, 1),), np.int32, -1),
                                                            ((max(k, 1),), np.float64, float("-inf"))]))
 
+    def similar_items(self, items, k):
+        """The k items most similar to each of ``items`` by cosine similarity: ``(ids int32[n, k], scores float64[n, k])``.
+        With ``v^ = v / sqrt(seq_dot(v, v))`` per row (a zero row stays zero) the score is ``seq_dot(v^_q, v^_r)`` bit for
+        bit; the order is score descending, then item id ascending; only the query item itself is left out (other
+        items with the same vector tie); slots that cannot be filled hold -1 and -inf.  1 <= k <= 1024.  ``items`` may
+        be a torch CUDA tensor.  The model is not touched.  With several ranks the call is collective, like
+        ``recommend_vectors``."""
+        return self._similar(_lib.BUF_V, items, k)
+
+    def similar_users(self, users, k):
+        """``similar_items`` over the user factors: the k users most similar to each of ``users``."""
+        return self._similar(_lib.BUF_U, users, k)
+
+    def _similar(self, which, ids, k):
+        dev = f"cuda:{self.device}"
+        if self.world == 1:
+            return _similar_call(self.lib.eals_similar, self.h, which, dev, ids, k)
+        q = (ids.cpu().numpy() if hasattr(ids, "cpu") else np.asarray(ids)).reshape(-1)
+        k = int(k)
+        run = lambda lo, hi: _similar_call(self.lib.eals_similar, self.h, which, dev, q[lo:hi], k)
+        return tuple(self._collective_slices(len(q), run, [((max(k, 1),), np.int32, -1),
+                                                           ((max(k, 1),), np.float64, float("-inf"))]))
+
     def ranking_metrics(self, test: SparseMat, k, exclude_seen=True, per_user=False, ranks=False):
         """Ranking metrics at k on a held-out test matrix ``test`` (a SparseMat with one row per user over this model's
         items; only its CSR is read).  For a test entry (u, g) the rank is g's 0-based position in
@@ -1284,6 +1329,14 @@ class GroupMF_fastALS:
         """``MF_fastALS.recommend_vectors`` over all ranks: balanced contiguous slices of the queries, one per rank."""
         return _recommend_vectors_call(self.lib.eals_group_recommend_vectors, self.g, self.factors, f"cuda:{self.devices[0]}",
                                        Q, k, exclude)
+
+    def similar_items(self, items, k):
+        """``MF_fastALS.similar_items`` over all ranks: balanced contiguous slices of the queries, one per rank."""
+        return _similar_call(self.lib.eals_group_similar, self.g, _lib.BUF_V, f"cuda:{self.devices[0]}", items, k)
+
+    def similar_users(self, users, k):
+        """``MF_fastALS.similar_users`` over all ranks: balanced contiguous slices of the queries, one per rank."""
+        return _similar_call(self.lib.eals_group_similar, self.g, _lib.BUF_U, f"cuda:{self.devices[0]}", users, k)
 
     def ranking_metrics(self, test: SparseMat, k, exclude_seen=True, per_user=False, ranks=False):
         """``MF_fastALS.ranking_metrics`` over all ranks: each rank ranks the test rows it owns, sums in rank order."""

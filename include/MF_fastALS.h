@@ -221,6 +221,11 @@ class MF_fastALS_T {
                                        r.scores.data()), "eals_group_recommend_vectors");
     return r;
   }
+  // Similar items / similar users: for each id the k other items (users) of highest cosine score, seq_dot of the rows
+  // normalised by their norm sqrt(seq_dot(y, y)), ties by id ascending; only the query itself is left out.
+  // Row-major [ids.size()][k]; slots that cannot be filled hold -1 and -inf.  1 <= k <= 1024.  The model is not touched.
+  Recommendations similar_items(const std::vector<int>& items, int k) { return similar(EALS_BUF_V, items, k); }
+  Recommendations similar_users(const std::vector<int>& users, int k) { return similar(EALS_BUF_U, users, k); }
   // Ranking metrics at k on a held-out test matrix (CSR over all users: row_ptr of userCount + 1 offsets, ascending
   // col_idx).  A test item's rank is its position in recommend({u}, k, exclude_seen), or -1; the means are over the
   // users with test items.  per_user: [userCount][6] (hit rate, precision, recall, NDCG, MAP, MRR), ranks: one per
@@ -275,6 +280,15 @@ class MF_fastALS_T {
   eals_model* handle(int rank = 0) { eals_model* m = nullptr; check(eals_group_model(g_, rank, &m), "eals_group_model"); return m; }
 
  private:
+  Recommendations similar(int32_t which, const std::vector<int>& ids, int k) {
+    Recommendations r;
+    std::vector<int32_t> q(ids.begin(), ids.end());
+    r.items.resize(q.size() * (size_t)std::max(k, 0));
+    r.scores.resize(r.items.size());
+    check(eals_group_similar(g_, which, EALS_HOST, (int32_t)q.size(), q.data(), k, r.items.data(), r.scores.data()),
+          "eals_group_similar");
+    return r;
+  }
   struct Flat {
     std::vector<int64_t> row_ptr, col_ptr;
     std::vector<int32_t> col_idx, row_idx;

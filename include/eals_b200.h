@@ -250,6 +250,18 @@ int eals_fold_in(eals_model* m, int32_t space, int32_t n, const int64_t* row_ptr
 int eals_recommend_vectors(eals_model* m, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr, const int32_t* ex_idx,
                            int32_t k, int32_t* items, double* scores);
 
+/* Similar items (which = EALS_BUF_V, catalogue V of n_items rows) or similar users (which = EALS_BUF_U, catalogue U
+ * of n_users rows): for each of the n ids, the k other rows of the catalogue of highest cosine score, ordered by
+ * score descending and id ascending.  With |y| = sqrt(seq_dot(y, y)) (predict's sequential fp64 sum of separately
+ * rounded products, correctly rounded square root) and y^ = y / |y| per factor (a zero row stays zero), the score of
+ * (q, r) is seq_dot(y^_q, y^_r) bit for bit.  Only the query's own row is left out: other rows with the same vector
+ * stay and tie.  Slots that cannot be filled hold id -1 and score -inf.  ids may be any row in [0, n_Y) on any rank
+ * (U and V are replicated).  out_ids: [n][k] int32, scores: [n][k] double or NULL; ids, out_ids and scores are host or
+ * device memory as `space` says.  1 <= k <= 1024, factors <= 256, the engines of eals_recommend.  The model stays
+ * exactly as it was; eals_recommend_stats reports the last call. */
+int eals_similar(eals_model* m, int32_t which, int32_t space, int32_t n, const int32_t* ids, int32_t k, int32_t* out_ids,
+                 double* scores);
+
 /* Ranking metrics at k on a held-out test matrix.  test_ptr / test_idx: a CSR with one row per user (n_users + 1
  * offsets, the rules of eals_set_train; this model reads the rows of its own users).  For a test entry (u, g) the
  * rank is g's 0-based position in the list eals_recommend(u, k, exclude_seen) returns, or -1 when g is not in it (a
@@ -362,6 +374,10 @@ int eals_group_fold_in(eals_group* g, int32_t space, int32_t n, const int64_t* r
                        const double* val, const double* init, int32_t n_iter, double* out);
 int eals_group_recommend_vectors(eals_group* g, int32_t space, int32_t n, const double* Q, const int64_t* ex_ptr,
                                  const int32_t* ex_idx, int32_t k, int32_t* items, double* scores);
+/* eals_similar over the group: the queries go to the ranks in balanced contiguous slices (U and V are replicated),
+ * results in input order. */
+int eals_group_similar(eals_group* g, int32_t which, int32_t space, int32_t n, const int32_t* ids, int32_t k, int32_t* out_ids,
+                       double* scores);
 /* eals_ranking_metrics over the whole matrix: each rank on the rows it owns, sums added in rank order.  means[6] are
  * divided by *n_users (0 when no user has test items); per_user is [n_users][6], ranks in test-entry order. */
 int eals_group_ranking_metrics(eals_group* g, int32_t space, const int64_t* test_ptr, const int32_t* test_idx, int32_t k,
